@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 gravitational force engine.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload direct|tree]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload direct|tree] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1]: DirectForceComputer, 2^20 particles,
 softened gravity (eps = 0.01), one force evaluation per step.  Metric: pairwise
@@ -385,6 +385,36 @@ class Sharded:
             got = self._checksum(self.posm[r * self.n // D.world:(r + 1) * self.n // D.world])
             ok = ok and bool((got == owners[r][0]).item())
         return D.all_ok(ok)
+
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(D, out_dir, n, rows, scalars=None):
+    """--dump-outputs: write what the timed path returned in its last step as <out_dir>/<name>.npy (float32 /
+    float64) on rank 0, so that two builds can be compared output for output.  `rows` maps a name to this rank's
+    [nl, k] device rows of an n-row result (target order); they are gathered over the ranks.  Above
+    DUMP_LIMIT_BYTES in all, the same fixed, seeded sample of rows (sorted row indices) is kept from every array."""
+    torch = D.torch
+    full = {}
+    for name, t in rows.items():
+        t = t.contiguous()
+        if D.world > 1:
+            parts = [torch.empty(((r + 1) * n // D.world - r * n // D.world, t.shape[1]), dtype=t.dtype, device=D.dev)
+                     for r in range(D.world)]
+            D.dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        full[name] = t.cpu().numpy()
+    if D.rank != 0:
+        return
+    row_bytes = sum(a.itemsize * a.shape[1] for a in full.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES - 4096:
+        keep = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT_BYTES - 4096) // row_bytes, replace=False))
+        full = {k: a[keep] for k, a in full.items()}
+    full.update({k: np.asarray(v, np.float64) for k, v in (scalars or {}).items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in full.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def sample_block(lo, nl, want=1024):
@@ -999,6 +1029,12 @@ def bench_gpu(args):
     launches = eng.launches - launches0
     eng.set_timing(False)
     sampler.stop()
+    if args.dump_outputs:           # before anything below runs the step again
+        rows, scalars = {"acc": acc}, None
+        if args.kdk:
+            rows.update(pos=shard[:, :3], vel=vel)
+            scalars = {"scale_factor": kdk["a"]}
+        dump_outputs(D, args.dump_outputs, n, rows, scalars)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_s = D.max(sum(step_ms)) * 1e-3
     kern_s = D.max(float(np.mean(kernel_ms))) * 1e-3
@@ -1195,7 +1231,15 @@ def main():
     ap.add_argument("--kdk", action="store_true",
                     help="each step is a full Lambda-CDM KDK leapfrog step (fused kick-kick-drift pass, scale-factor "
                          "update, source all-gather, force evaluation) instead of a bare force evaluation")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the last timed step computed (forces; with --kdk "
+                         "also positions, velocities and the scale factor) as DIR/<name>.npy, at most 64 MB in all "
+                         "(a fixed, seeded sample of rows beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
     if args.impl == "reference":
         bench_reference(args)
     else:

@@ -221,15 +221,17 @@ def test_tree_c4_size_16m(engine, oracle):
 
 
 def test_tree_zeldovich_c3(engine, oracle):
-    """BASELINE config 3 inputs: the reference's own "Zel'dovich" generator (grid 128 -> 2^20 particles,
-    seed 12345, z = 49, box 100), shifted to the centred convention; run live from the prebuilt
-    oracle/_ref (no /root/reference needed at run time)."""
+    """BASELINE config 3 scale: Zel'dovich initial conditions (grid 128 -> 2^20 particles, seed 12345, z = 49,
+    box 100) from the engine's own generator (b200_zeldovich_ics_dev, held to oracle/ics_np.py by
+    test_gpu_ics.py), shifted to the centred convention."""
     import torch
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref not built")
     n = 1 << 20
-    zp, zv, zm = Ref().zeldovich(n, grid=128, box=100.0, z_init=49.0, seed=12345)
+    ics = torch.empty((n, 4), dtype=torch.float32, device="cuda")
+    engine.zeldovich_ics_dev(ics, torch.empty((n, 3), dtype=torch.float32, device="cuda"), n_particles=n, grid=128,
+                             box=100.0, z_initial=49.0, seed=12345)
+    torch.cuda.synchronize()
+    zp, zm = np.ascontiguousarray(ics[:, :3].cpu().numpy()), np.ascontiguousarray(ics[:, 3].cpu().numpy())
+    del ics
     p = (zp - np.float32(50.0)).astype(np.float32)
     posm, t = _build_export(engine, p, zm, box=100.0, leaf_cap=8, max_depth=20)
     o = oracle.tree_build(p, zm)
