@@ -142,6 +142,45 @@ int b200_power_spectrum_dev(b200_ctx* ctx, const void* posm4, size_t n, int grid
                             int mass_weighted, int shot_noise_correction, float* k_out, float* p_out,
                             int* count_out, void* stream);
 
+/* ---- periodic particle mesh ----------------------------------------------------
+ * The solver the reference reserves the factory name "PMForceComputer" for (src/forces/
+ * force_computer_factory.cpp:40-63) and never implements: the true periodic force of the box with a uniform
+ * neutralising background, O(N + grid^3 log grid), where every other force path keeps only the nearest image.
+ * Definition (G = 1; box L, mesh grid^3, h = L / grid, r_s = r_split):
+ *   positions are wrapped, x - L floor(x / L) (the [0, L) and origin-centred frames give the same mesh); mesh point
+ *   i sits at i h; cloud-in-cell (CIC) assignment of the sources posm4[0 .. n_sources) with masses .w;
+ *   rho = sum m W / h^3 minus its mean (the k = 0 mode is zero);
+ *   phi_k = -4 pi rho_k exp(-k^2 r_s^2) / (k^2 W(k)^2), W(k) = prod_a sinc^2(k_a h / 2)  (one W for the
+ *   assignment, one for the interpolation, as GADGET-2);
+ *   a_k = -i k_a phi_k (zero on the Nyquist plane of axis a), inverse FFT, CIC interpolation at the targets
+ *   posm4[i0 .. i0+n_targets) with the deposit's weights.
+ * acc3: float[3*n_targets] ACCELERATION, overwritten, in the sign convention of the direct sum.  phi (float
+ * [n_targets], NULL = skip): the NEGATED mesh potential, interpolated the same way -- positive, as
+ * b200_direct_potential_dev (potential energy = -1/2 sum m phi); long range only, and it includes the particle's
+ * own smoothed self term (about m / (sqrt(pi) r_s)).
+ * r_split > 0 is the Gaussian split radius of TreePM (Springel 2005); there is no "off" value, because without the
+ * filter the W^-2 deconvolution makes the pair force noisy (100-200 % r.m.s. at 2-8 cells).  Recommended:
+ * r_split = 1.25 h.  The PM force plus the short-range remainder sum m d / r^3 [erfc(r / 2 r_s) + r / (r_s sqrt(pi))
+ * exp(-r^2 / 4 r_s^2)] (minimum image) then matches an Ewald sum to 0.02 / 0.2 / 0.8 / 1.0 / 0.6 / 0.3 % r.m.s. at
+ * r = 0.5 / 1 / 2 / 4 / 8 / 12 h; used alone, the PM force is smooth below a few cells, the mesh's resolution.
+ * The mass deposit accumulates in int64 fixed point: the meshes, and so the result for a target, are bitwise the
+ * same whatever the storage order of the sources and whichever target range is asked for.  Sharded use: every rank
+ * passes the full all-gathered array (b200_allgather_sources_dev) and its own target range (b200_shard_range); the
+ * deposit is replicated, so the meshes are bitwise identical on every rank and the concatenated result is that of
+ * one call.  FFTs are cuFFT, bound at run time: B200_ERR_UNSUPPORTED if libcufft is absent.  Meshes and plans are
+ * kept on the context per grid (about 40 grid^3 bytes).
+ * B200_ERR_INVALID: grid odd or outside 8..1024, box <= 0, r_split <= 0, i0 + n_targets > n_sources, acc3 NULL. */
+int b200_pm_forces_dev(b200_ctx* ctx, const void* posm4, size_t n_sources, size_t i0, size_t n_targets,
+                       int grid, float box, float r_split, void* acc3, void* phi /* NULL = skip */, void* stream);
+/* Host-array form for "PMForceComputer" (IForceComputer::compute_forces): pos3 float[3n], mass float[n] or NULL
+ * (= 1), acc3 float[3n]; all n particles are sources and targets.  Blocking. */
+int b200_pm_forces_host(b200_ctx* ctx, const float* pos3, const float* mass /* NULL = 1 */, float* acc3,
+                        size_t n, int grid, float box, float r_split);
+/* With b200_set_timing on: CUDA-event times (ms) of the phases of the last b200_pm_forces_dev on this context --
+ * [0] deposit (mesh clear, mass bound, deposit), [1] convert, [2] R2C, [3] k-space, [4] the C2R transforms,
+ * [5] interpolation, [6] the whole call.  Synchronises; B200_ERR_STATE without a timed call. */
+int b200_pm_phase_ms(b200_ctx* ctx, float ms[7]);
+
 /* ---- Barnes-Hut (rows T1-T6) ----------------------------------------------
  * Morton keys: replaces compute_morton_codes_kernel + morton3D
  * (src/forces/barnes_hut_tree.cu:33-55, include/forces/barnes_hut_tree.hpp:11-27);

@@ -8,6 +8,7 @@
 #include "direct.cuh"
 #include "ics.cuh"
 #include "leapfrog.cuh"
+#include "pm.cuh"
 #include "probe.cuh"
 #include "shard.cuh"
 #include "sort.cuh"
@@ -74,6 +75,7 @@ int b200_ctx_destroy(b200_ctx* ctx) {
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     tree_destroy(ctx);
     shard_finalize(ctx);
+    pm_destroy(ctx);
     ctx->src_tiles.release(); ctx->partials.release(); ctx->mass_flag.release(); ctx->zero_flag.release();
     ctx->energy_part.release(); ctx->energy_phi.release(); ctx->energy_out.release();
     ctx->ic_wk.release(); ctx->ic_tmp.release(); ctx->ic_psi.release(); ctx->ic_stats.release();
@@ -248,6 +250,45 @@ int b200_direct_forces_host(b200_ctx* ctx, const float* pos3, const float* mass,
     return B200_OK;
 }
 
+// ---- periodic particle mesh -------------------------------------------------
+int b200_pm_forces_dev(b200_ctx* ctx, const void* posm4, size_t n_sources, size_t i0, size_t n_targets,
+                       int grid, float box, float r_split, void* acc3, void* phi, void* stream) {
+    if (!ctx || !acc3 || i0 + n_targets > n_sources || (n_sources && !posm4)) return B200_ERR_INVALID;
+    if (grid < 8 || grid > 1024 || (grid & 1) || !(box > 0.f) || !(r_split > 0.f)) return B200_ERR_INVALID;
+    if (n_targets == 0) return B200_OK;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return pm_forces(ctx, posm4, n_sources, i0, n_targets, grid, box, r_split, acc3, phi, pick_stream(ctx, stream));
+}
+
+int b200_pm_forces_host(b200_ctx* ctx, const float* pos3, const float* mass, float* acc3, size_t n, int grid,
+                        float box, float r_split) {
+    if (!ctx || !acc3 || (n && !pos3)) return B200_ERR_INVALID;
+    if (grid < 8 || grid > 1024 || (grid & 1) || !(box > 0.f) || !(r_split > 0.f)) return B200_ERR_INVALID;
+    if (n == 0) return B200_OK;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    B200_TRY(ctx->h_pos3.reserve(n * 3 * sizeof(float)));
+    B200_TRY(ctx->h_posm4.reserve(n * 4 * sizeof(float)));
+    B200_TRY(ctx->h_acc3.reserve(n * 3 * sizeof(float)));
+    B200_CUDA(cudaMemcpyAsync(ctx->h_pos3.p, pos3, n * 3 * sizeof(float), cudaMemcpyHostToDevice, st));
+    const float* d_mass = nullptr;
+    if (mass) {
+        B200_TRY(ctx->h_mass.reserve(n * sizeof(float)));
+        B200_CUDA(cudaMemcpyAsync(ctx->h_mass.p, mass, n * sizeof(float), cudaMemcpyHostToDevice, st));
+        d_mass = ctx->h_mass.as<float>();
+    }
+    B200_TRY(pack_posm(ctx, ctx->h_pos3.p, d_mass, n, ctx->h_posm4.p, st));
+    B200_TRY(pm_forces(ctx, ctx->h_posm4.p, n, 0, n, grid, box, r_split, ctx->h_acc3.p, nullptr, st));
+    B200_CUDA(cudaMemcpyAsync(acc3, ctx->h_acc3.p, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    B200_CUDA(cudaStreamSynchronize(st));
+    return B200_OK;
+}
+
+int b200_pm_phase_ms(b200_ctx* ctx, float ms[7]) {
+    if (!ctx || !ms) return B200_ERR_INVALID;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return pm_phase_ms(ctx, ms);
+}
 
 // ---- Barnes-Hut -------------------------------------------------------------
 int b200_morton_keys_dev(b200_ctx* ctx, const void* posm4, size_t n, float box, void* keys_u32,

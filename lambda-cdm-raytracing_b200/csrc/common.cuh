@@ -46,7 +46,7 @@ struct DevBuf {
     template <class T> T* as() const { return (T*)p; }
 };
 
-namespace b200 { struct TreeState; struct ShardState; }   // tree.cu, shard.cu
+namespace b200 { struct TreeState; struct ShardState; struct PmState; }   // tree.cu, shard.cu, pm.cu
 
 constexpr int B200_MAX_KERNEL_CFG = 64;
 struct KernelCfg { const void* fn; int blocks_per_sm; };   // per-device launch configuration of a kernel instance
@@ -77,6 +77,7 @@ struct b200_ctx {
 
     b200::TreeState* tree = nullptr;
     b200::ShardState* shard = nullptr;    // NCCL communicator (b200_shard_init)
+    b200::PmState* pm = nullptr;          // particle-mesh meshes and cuFFT plans, per grid (b200_pm_forces_dev)
 };
 
 static inline int ceil_div_i(long long a, long long b) { return (int)((a + b - 1) / b); }

@@ -30,6 +30,7 @@ EXPORTS = [
     "b200_allgather_sources_dev", "b200_allreduce_sum_f64", "b200_direct_potential_dev", "b200_energy_dev",
     "b200_ic_params_default", "b200_zeldovich_ics_dev", "b200_force_error_dev", "b200_power_spectrum_dev", "b200_tree_build_fixed_dev", "b200_tree_forces_fixed_host", "b200_tree_set_periodic", "b200_spatial_order_dev", "b200_tree_build_host", "b200_tree_walk_host", "b200_tree_potential_dev", "b200_tree_energy_dev",
     "b200_fp32_peak_probe", "b200_last_kernel_ms", "b200_set_timing", "b200_launch_count",
+    "b200_pm_forces_dev", "b200_pm_forces_host", "b200_pm_phase_ms",
 ]
 
 
@@ -124,6 +125,9 @@ def load_library(path=None):
     L.b200_zeldovich_ics_dev.argtypes = [vp, C.POINTER(ICParams), sz, vp, vp, C.POINTER(f64), vp]
     L.b200_force_error_dev.argtypes = [vp, vp, vp, sz, C.POINTER(f64), C.POINTER(f64), vp]
     L.b200_power_spectrum_dev.argtypes = [vp, vp, sz, i32, f32, i32, i32, vp, vp, vp, vp]
+    L.b200_pm_forces_dev.argtypes = [vp, vp, sz, sz, sz, i32, f32, f32, vp, vp, vp]
+    L.b200_pm_forces_host.argtypes = [vp, vp, vp, vp, sz, i32, f32, f32]
+    L.b200_pm_phase_ms.argtypes = [vp, vp]
     L.b200_fp32_peak_probe.argtypes = [vp, i32, i32, C.POINTER(f64), C.POINTER(f32)]
     L.b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
     L.b200_set_timing.argtypes = [vp, i32]
@@ -427,6 +431,35 @@ class Engine:
                                                    int(shot_noise_correction), _ptr(k), _ptr(p), _ptr(c), _stream(stream)))
         return k, p, c
 
+    # ---- periodic particle mesh ----
+    def pm_forces_dev(self, posm, acc, i0=0, n_targets=None, grid=128, box=100.0, r_split=None, phi=None,
+                      stream=None):
+        """Periodic long-range PM acceleration of targets posm[i0 : i0+n_targets) from all of posm (device);
+        phi (device float[n_targets] or None): the positive long-range potential.  r_split=None: 1.25 box / grid."""
+        n = posm.shape[0]
+        nt = n - i0 if n_targets is None else n_targets
+        rs = 1.25 * box / grid if r_split is None else r_split
+        self._check(self.L.b200_pm_forces_dev(self._h, _ptr(posm), n, i0, nt, grid, box, rs, _ptr(acc), _ptr(phi),
+                                              _stream(stream)))
+        return acc
+
+    def pm_forces_host(self, pos, mass, grid, box, r_split=None, out=None):
+        pos = np.ascontiguousarray(pos, np.float32)
+        n = pos.shape[0]
+        m = None if mass is None else np.ascontiguousarray(mass, np.float32)
+        if out is None:
+            out = np.empty((n, 3), np.float32)
+        rs = 1.25 * box / grid if r_split is None else r_split
+        self._check(self.L.b200_pm_forces_host(self._h, _ptr(pos), _ptr(m), _ptr(out), n, grid, box, rs))
+        return out
+
+    def pm_phase_ms(self):
+        """Phase times (ms) of the last timed pm_forces_dev: deposit, convert, R2C, k-space, C2R, interpolation,
+        whole call."""
+        ms = np.zeros(7, np.float32)
+        self._check(self.L.b200_pm_phase_ms(self._h, _ptr(ms)))
+        return ms
+
     # ---- energy diagnostic ----
     def direct_potential_dev(self, posm, phi, i0=0, n_targets=None, eps=0.01, box=0.0, stream=None):
         n = posm.shape[0]
@@ -487,13 +520,14 @@ class LambdaCDMSimulation:
     physics::LambdaCDMSimulation (include/physics/lambda_cdm.hpp:22-75;
     step order src/physics/lambda_cdm_impl.cu:167-213), driving the C ABI.
 
-    force: "direct" or "tree".  The first half-kick of the first step uses the
+    force: "direct", "tree" or "pm" (periodic particle mesh on a pm_grid^3 mesh, Gaussian split radius r_split,
+    None = 1.25 box / pm_grid).  The first half-kick of the first step uses the
     forces at the initial positions (the reference reads uninitialised memory
     there; SURVEY 8c)."""
 
     def __init__(self, engine, pos, vel, mass, box=100.0, force="direct", eps=0.01, theta=0.5,
                  leaf_cap=8, max_depth=20, wrap=True, a0=1.0, cosmo=(0.31, 0.0, 0.69, 0.67),
-                 i0=0, n_local=None, gather=None):
+                 i0=0, n_local=None, gather=None, pm_grid=128, r_split=None):
         import torch
         self.torch = torch
         self.e = engine
@@ -507,6 +541,8 @@ class LambdaCDMSimulation:
         self.a = float(a0)
         self.cosmo = cosmo
         self.gather = gather              # callable(posm_full) -> refreshes non-local rows (multi-GPU)
+        self.pm_grid = int(pm_grid)
+        self.r_split = 1.25 * self.box / self.pm_grid if r_split is None else float(r_split)
         pm = np.concatenate([np.asarray(pos, np.float32), np.asarray(mass, np.float32)[:, None]], axis=1)
         self.posm = torch.from_numpy(np.ascontiguousarray(pm)).to(dev)
         self.vel = torch.from_numpy(np.ascontiguousarray(vel, np.float32)[i0:i0 + self.nl].copy()).to(dev)
@@ -517,6 +553,8 @@ class LambdaCDMSimulation:
     def compute_forces(self):
         if self.force == "direct":
             self.e.direct_forces_dev(self.posm, self.acc, self.i0, self.nl, self.eps, 0.0)
+        elif self.force == "pm":
+            self.e.pm_forces_dev(self.posm, self.acc, self.i0, self.nl, self.pm_grid, self.box, self.r_split)
         else:
             self.e.tree_build_dev(self.posm, self.n, self.box, self.leaf_cap, self.max_depth)
             self.e.tree_walk_dev(self.acc, self.i0, self.nl, self.theta)
