@@ -58,6 +58,11 @@ cic_kernel(const float4* __restrict__ posm, long long n, int G, float inv_spacin
         float x = fmodf(p.x * inv_spacing + Gf, Gf);                                          // :93-101
         float y = fmodf(p.y * inv_spacing + Gf, Gf);
         float z = fmodf(p.z * inv_spacing + Gf, Gf);
+        // fmodf keeps the dividend's sign: below -box the reference's formula leaves x negative, and a negative
+        // index would write before the grid.  x + G may round to G; (ix + dx) % G folds that back to cell 0.
+        if (x < 0.f) x += Gf;
+        if (y < 0.f) y += Gf;
+        if (z < 0.f) z += Gf;
         const int ix = (int)x, iy = (int)y, iz = (int)z;
         const float fx = x - ix, fy = y - iy, fz = z - iz;
         const float m = mass_weighted ? p.w : 1.0f;

@@ -16,6 +16,7 @@ def cic_grid(pos, mass, grid, box, mass_weighted=True):
     G = grid
     g = np.zeros((G, G, G), np.float64)
     x = np.fmod(pos.astype(np.float32) * np.float32(G / box) + np.float32(G), np.float32(G)).astype(np.float32)  # :93-101
+    x = np.where(x < 0, x + np.float32(G), x).astype(np.float32)     # below -box fmod stays negative (not in :93-101)
     i = x.astype(np.int64)
     f = (x - i.astype(np.float32)).astype(np.float32)
     m = mass.astype(np.float32) if mass_weighted else np.ones(len(pos), np.float32)

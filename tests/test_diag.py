@@ -36,6 +36,21 @@ def test_white_noise_is_shot_noise():
     assert np.allclose(pk - pk2, box ** 3 / G ** 3)              # the reference subtracts V / G^3 (:271)
 
 
+def test_cic_grid_is_periodic_in_whole_boxes():
+    """The CIC mesh of positions moved by whole periods, -3L .. +3L, is the mesh of the originals.  Below -L the
+    reference's fmod(x G / L + G, G) is negative; unwrapped, that mesh differs by more than its largest value."""
+    rng = np.random.default_rng(17)
+    G, box, n = 32, 100.0, 20000
+    pos = rng.uniform(0, box, (n, 3)).astype(np.float32)
+    mass = rng.uniform(0.5, 2.0, n).astype(np.float32)
+    g0 = pk_np.cic_grid(pos, mass, G, box)
+    for k in (-3, -2, -1, 1, 2, 3):
+        g = pk_np.cic_grid((pos + np.float32(k * box)).astype(np.float32), mass, G, box)
+        # float32 positions near 3L carry ~1e-5 of rounding, i.e. ~4e-6 of a cell
+        assert np.abs(g - g0).max() <= 1e-4 * g0.max(), (k, np.abs(g - g0).max(), g0.max())
+        assert abs(g.sum() - g0.sum()) <= 1e-9 * g0.sum(), k
+
+
 def test_force_error_measure():
     ref = np.array([[3.0, 4.0, 0.0], [0.0, 0.0, 2.0]], np.float32)
     tst = np.array([[3.0, 4.5, 0.0], [0.0, 0.0, 2.0]], np.float32)

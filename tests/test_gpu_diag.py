@@ -53,6 +53,24 @@ def test_power_spectrum_vs_numpy(engine, grid, n, weighted, shot, centred):
     assert np.abs(p - p0).max() < 2e-4 * scale          # float atomics / float FFT vs double
 
 
+def test_power_spectrum_periodic_in_whole_boxes(engine):
+    """Positions moved by -2L, -3L and +5L give the P(k) of the originals, and match pk_np on the moved positions
+    (below -L the deposit must wrap the negative fmod result back into the grid)."""
+    G, box, n = 32, 100.0, 20000
+    rng = np.random.default_rng(23)
+    pos = rng.uniform(0, box, (n, 3)).astype(np.float32)
+    mass = masses_np(n, seed=24)
+    k0, p0, c0 = engine.power_spectrum_dev(torch.from_numpy(np.concatenate([pos, mass[:, None]], 1)).cuda(), G, box)
+    scale = np.abs(p0).max()
+    for shift in (-2, -3, 5):
+        moved = (pos + np.float32(shift * box)).astype(np.float32)
+        k, p, c = engine.power_spectrum_dev(torch.from_numpy(np.concatenate([moved, mass[:, None]], 1)).cuda(), G, box)
+        assert np.array_equal(c, c0) and np.array_equal(k, k0)
+        assert np.abs(p - p0).max() < 2e-4 * scale, (shift, np.abs(p - p0).max() / scale)
+        _, pn, cn = pk_np.power_spectrum(moved, mass, G, box)
+        assert np.array_equal(c, cn) and np.abs(p - pn).max() < 2e-4 * scale, (shift, np.abs(p - pn).max() / scale)
+
+
 def test_zeldovich_particles_carry_the_input_spectrum(engine):
     """ICs -> CIC -> FFT -> P(k): at wavelengths well above the mesh, P_measured = D^2 P_linear."""
     G = 128
