@@ -117,13 +117,29 @@ def test_direct_periodic_vs_oracle(engine, oracle):
     assert rel_l2(a[ok], want[ok]) < TOL
 
 
+def _fixed_path_n(sm, n_min):
+    """The smallest n >= n_min (targets = sources = n) on the fixed-point path: direct_forces takes it when
+    ceil(n / 2048) * ceil(n / 512) >= 4 * SMs (and n >= 8192, eps >= 1e-4 box)."""
+    n = n_min
+    while -(-n // 2048) * -(-n // 512) < 4 * sm:
+        n += 1
+    return n
+
+
 @pytest.mark.parametrize("n,unit,eps,box", [(20000, True, 0.05, 100.0), (20000, False, 0.05, 100.0),
                                             (20000, True, 0.05, 64.0), (9000, True, 0.05, 100.0),
-                                            (20000, False, 1e-3, 100.0)])
+                                            (20000, False, 1e-3, 100.0),
+                                            ("fixed", True, 0.05, 100.0), ("fixed", False, 0.05, 100.0),
+                                            ("fixed", True, 0.05, 64.0), ("fixed", False, 1e-3, 100.0)])
 def test_direct_periodic_both_minimum_image_paths(engine, oracle, n, unit, eps, box):
-    """Above 8192 targets with eps >= 1e-4 box the x and y separations are taken in 32-bit fixed point (the wrap
-    is the integer overflow); below either bound the FP32 minimum image runs.  Same gate for both; n is never a
-    multiple of the 512-source tile, so the padding slots are exercised too (equal and general masses)."""
+    """With eps >= 1e-4 box and at least 4 (2048-target block x 512-source tile) work units per SM (24577 particles
+    on 148 SMs; "fixed" = the smallest such n + 1000) the x and y separations are taken in 32-bit fixed point (the
+    wrap is the integer overflow); below either bound (9000 and 20000 particles: 400 units on 148 SMs; eps = 1e-3)
+    the FP32 minimum image runs.  Same gate for both; n is never a multiple of the 512-source tile, so the padding slots are exercised too
+    (equal and general masses)."""
+    if n == "fixed":
+        n = _fixed_path_n(engine.sm_count, 8192) + 1000
+        assert n % 512
     rng = np.random.default_rng(n + int(box))
     p = rng.uniform(0.0, box, (n, 3)).astype(np.float32)
     m = np.full(n, 1.5, np.float32) if unit else masses_np(n, seed=16)
@@ -138,9 +154,9 @@ def test_direct_periodic_both_minimum_image_paths(engine, oracle, n, unit, eps, 
 
 def test_direct_periodic_nan_propagates(engine):
     """A NaN coordinate poisons every force in both minimum-image paths (the fixed-point conversion of x and y
-    must not swallow it)."""
+    must not swallow it): 3000 and 20000 particles run the FP32 minimum image, the third size the fixed point."""
     rng = np.random.default_rng(3)
-    for n in (3000, 20000):
+    for n in (3000, 20000, _fixed_path_n(engine.sm_count, 8192) + 1000):
         p = rng.uniform(0.0, 100.0, (n, 3)).astype(np.float32)
         p[n // 2, 0] = np.nan
         a = engine.direct_forces_host(p, None, eps=0.05, box=100.0)
