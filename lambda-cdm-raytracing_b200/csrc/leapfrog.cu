@@ -9,16 +9,14 @@
 // 512-byte run): positions as one float4 per particle, velocities and accelerations
 // (3 floats per particle, AoS) as the tile's 768 float4 words staged through shared
 // memory, where thread t reads floats 3p .. 3p+2 of its particles (stride 3: no bank
-// conflicts).  B200_LEAPFROG=v1 selects the round-1 kernel (a thread owns 4 consecutive
-// particles; 128-bit accesses at a 48/64-byte lane stride) for comparison.
+// conflicts).  The n mod 1024 particles behind the last full tile go to the tail kernel
+// (a thread owns 4 consecutive particles; 128-bit accesses at a 48/64-byte lane stride).
 //
 // The arithmetic keeps the reference's operation order with one rounding per
 // operation (no FMA contraction) so trajectories are bit-identical to the CPU
 // restatement given identical accelerations:
 //     v += ((acc*m) * (1/m)) * dt * (1/a^2)        (:307-318; F = acc*m, :217-219)
 //     x  = fmodf((x + v*dt) + box, box)            (:322-329)
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "leapfrog.cuh"
 
@@ -55,9 +53,10 @@ __device__ __forceinline__ void step_particle(float4& p, float& vx, float& vy, f
     }
 }
 
+// The particles behind the last full tile of leapfrog_kernel: 4 per thread, the last group scalar.
 __global__ void __launch_bounds__(256)
-leapfrog_v1_kernel(float4* __restrict__ posm, float4* __restrict__ vel4, const float4* __restrict__ acc4,
-                   long long n, int n_kicks, float dt_kick, float a2inv, float dt_drift, float box) {
+leapfrog_tail_kernel(float4* __restrict__ posm, float4* __restrict__ vel4, const float4* __restrict__ acc4,
+                     long long n, int n_kicks, float dt_kick, float a2inv, float dt_drift, float box) {
     const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // group of 4 particles
     const long long i0 = q * 4;
     if (i0 >= n) return;
@@ -100,7 +99,7 @@ leapfrog_v1_kernel(float4* __restrict__ posm, float4* __restrict__ vel4, const f
     }
 }
 
-// Tile kernel: full tiles of LF_TILE particles only (the host sends the ragged tail to the v1 kernel).
+// Tile kernel: full tiles of LF_TILE particles only (the host sends the ragged tail to leapfrog_tail_kernel).
 constexpr int LF_THREADS = 256;
 constexpr int LF_PER = 4;
 constexpr int LF_TILE = LF_THREADS * LF_PER;          // 1024 particles, 768 float4 words of vel / acc
@@ -211,8 +210,7 @@ int leapfrog(b200_ctx* ctx, void* posm4, void* vel3, const void* acc3, size_t n,
     if (((uintptr_t)vel3 | (uintptr_t)acc3 | (uintptr_t)posm4) & 15) return B200_ERR_INVALID;
     // lambda_cdm_kernels.cu:308: const float a2_inv = 1.0f / (scale_factor * scale_factor);
     const float a2inv = (float)(1.0f / (a * a));
-    static const bool use_v1 = getenv("B200_LEAPFROG") != nullptr && getenv("B200_LEAPFROG")[1] == '1';   // tuning hook
-    const long long full = use_v1 ? 0 : (long long)n / LF_TILE;                // particles [0, full * LF_TILE)
+    const long long full = (long long)n / LF_TILE;                             // particles [0, full * LF_TILE)
     if (full > 0) {
         const long long cap = (long long)ctx->sm_count * 8;                    // 8 CTAs (24 KB of shared memory each) per SM
         leapfrog_kernel<<<(unsigned)(full < cap ? full : cap), LF_THREADS, 0, st>>>(
@@ -222,7 +220,7 @@ int leapfrog(b200_ctx* ctx, void* posm4, void* vel3, const void* acc3, size_t n,
     const long long done = full * LF_TILE, rest = (long long)n - done;          // tail: a multiple-of-4 offset keeps vel/acc 16-byte aligned
     if (rest > 0) {
         const long long groups = (rest + 3) / 4;
-        leapfrog_v1_kernel<<<(unsigned)((groups + 255) / 256), 256, 0, st>>>(
+        leapfrog_tail_kernel<<<(unsigned)((groups + 255) / 256), 256, 0, st>>>(
             (float4*)posm4 + done, (float4*)((float*)vel3 + 3 * done), (const float4*)((const float*)acc3 + 3 * done),
             rest, n_kicks, dt_kick, a2inv, dt_drift, box);
         ctx->launches += 1;

@@ -73,7 +73,7 @@ struct TreeState {
     float periodic_box = 0.f;    // fixed mode only: > 0 = minimum-image separations in the walk
     DevBuf center, com, meta, nstart, ncount, nsplit_rank;
     DevBuf ent_idx[2], ent_node[2], digit;
-    DevBuf part_idx, part_pos;
+    DevBuf part_idx;
     DevBuf nodes;                 // walk records, 32 B each, depth-first order: {centre of mass, M} {skip, first leaf pair, edge, leaf count}
     DevBuf leaf_pos, lscan, pscan, leaf_tile_sum;   // leaf sources grouped by parent, pair-interleaved (walk-only)
     DevBuf sub;                   // walk records in the subtree of a node (0: leaf or massless)
@@ -124,7 +124,7 @@ struct TreeState {
         memcpy(&bb, &box, 4); memcpy(&eb, &eps, 4);
         mix(bb); mix(eb);
         const DevBuf* all[] = {&center, &com, &meta, &nstart, &ncount, &nsplit_rank, &ent_idx[0], &ent_idx[1],
-                               &ent_node[0], &ent_node[1], &digit, &part_idx, &part_pos, &nodes, &leaf_pos,
+                               &ent_node[0], &ent_node[1], &digit, &part_idx, &nodes, &leaf_pos,
                                &lscan, &pscan, &sub, &leaf_tile_sum, &slot_node, &slot_digit, &globals, &tile_hist,
                                &tile_warp_prefix, &node_tile_sum, &split_node, &split_where, &split_local,
                                &split_cstart};
@@ -147,7 +147,7 @@ struct TreeState {
         if (ev_out) cudaEventDestroy(ev_out);
         ev_in = ev_out = nullptr;
         DevBuf* all[] = {&center, &com, &meta, &nstart, &ncount, &nsplit_rank, &ent_idx[0],
-                         &ent_idx[1], &ent_node[0], &ent_node[1], &digit, &part_idx, &part_pos, &nodes, &leaf_pos, &lscan, &pscan, &sub, &leaf_tile_sum, &slot_node, &slot_digit,
+                         &ent_idx[1], &ent_node[0], &ent_node[1], &digit, &part_idx, &nodes, &leaf_pos, &lscan, &pscan, &sub, &leaf_tile_sum, &slot_node, &slot_digit,
                          &globals, &tile_hist, &tile_warp_prefix, &node_tile_sum, &split_node,
                          &split_where, &split_local, &split_cstart, &keys, &keys_sorted, &perm,
                          &sort_scratch, &order};
@@ -659,23 +659,21 @@ __device__ __forceinline__ int tree_node_count(const TreeGlobals* g, int max_dep
     return nn;
 }
 
-// Stored particles in stored order, (x, y, z, particle index bits) -- or, in the fixed mode, the
-// float4 as it is (x, y, z, mass): that walk uses real masses and needs no self test -- and, for the
-// slots that belong to leaf nodes, a second copy in the walk's layout: the leaf particles of one
-// parent are contiguous and PAIR-INTERLEAVED, pair p = {x0 x1 y0 y1} {z0 z1 w0 w1}, so that one
-// packed-FP32 instruction of the walk handles two sources (lscan: rank of a leaf's first particle
+// The stored particles that belong to leaf nodes, in the walk's layout: (x, y, z, particle index bits) -- or,
+// in the fixed mode, the float4 as it is (x, y, z, mass): that walk uses real masses and needs no self test.
+// The leaf particles of one parent are contiguous and PAIR-INTERLEAVED, pair p = {x0 x1 y0 y1} {z0 z1 w0 w1},
+// so that one packed-FP32 instruction of the walk handles two sources (lscan: rank of a leaf's first particle
 // among all leaf particles; pscan: first pair of a sibling group).
 __global__ void stored_pos_kernel(const TreeGlobals* __restrict__ g, const int* __restrict__ part_idx,
                                   const int* __restrict__ slot_node,
                                   const int4* __restrict__ meta, const int* __restrict__ lscan,
                                   const int* __restrict__ pscan, const float4* __restrict__ posm, int n,
-                                  float4* __restrict__ part_pos, float* __restrict__ leaf_pairs, int fixed) {
+                                  float* __restrict__ leaf_pairs, int fixed) {
     int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n || q >= g->stored_total) return;            // a part build stores only its octants' particles
     const int idx = part_idx[q];
     float4 p = posm[idx];
     if (!fixed) p.w = __int_as_float(idx);
-    part_pos[q] = p;
     const int k = slot_node[q];
     const int4 m = meta[k];
     if (m.x >= 0) return;                                       // an orphan: never a source
@@ -1084,93 +1082,10 @@ __global__ void forest_root_kernel(ForestTables F, const int* __restrict__ hdr, 
 }
 
 // ------------------------------------------------------------------ walk ---
-// Legacy kernel (B200_WALK_PER_THREAD=1; kept as an independent cross-check of the warp walk).
-// One thread per target, targets taken in space-filling-curve order so the 32 lanes of a
-// warp walk nearly the same nodes.  Stackless: every node carries the id of the
-// node that follows its subtree in depth-first order (meta.y), so "skip" is one
-// load and "open" is meta.x.  Accept test: IEEE sqrt/divide, no contraction, so
-// every lane takes exactly the decision the CPU code takes (:302-310).
-__device__ __forceinline__ bool accept_cell(float size, float d2, float theta);
-
-template <bool COUNT>
-__global__ void __launch_bounds__(128)
-walk_kernel(const float4* __restrict__ posm, const int* __restrict__ order, int i0, int n_targets,
-            const float4* __restrict__ com, const float4* __restrict__ center,
-            const int4* __restrict__ meta, const float4* __restrict__ part_pos, float theta,
-            float* __restrict__ acc3, TreeGlobals* __restrict__ g) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    unsigned long long c_vis = 0, c_pc = 0, c_pp = 0;
-    if (t < n_targets) {
-        const int i = order ? order[t] : (i0 + t);
-        const float4 p = posm[i];
-        float ax = 0.f, ay = 0.f, az = 0.f;
-        const float eps2 = __fmul_rn(0.01f, 0.01f);                      // :281-282, :334-335
-        int k = 0;
-        while (k >= 0) {
-            const float4 c = com[k];
-            const int4 m = meta[k];
-            if (COUNT) ++c_vis;
-            if (c.w == 0.0f) { k = m.y; continue; }                      // :260
-            if (m.x < 0) {                                               // leaf :268-270
-                for (int q = m.z; q < m.z + m.w; ++q) {
-                    const float4 s = part_pos[q];
-                    if (__float_as_int(s.w) == i) continue;              // :321
-                    const float dx = s.x - p.x, dy = s.y - p.y, dz = s.z - p.z;
-                    const float r2 = dx * dx + dy * dy + dz * dz + eps2;
-                    const float rinv = rsqrtf(r2);
-                    const float f = rinv * rinv * rinv;                  // unit mass (:253, :340)
-                    ax += f * dx; ay += f * dy; az += f * dz;
-                    if (COUNT) ++c_pp;
-                }
-                k = m.y;
-                continue;
-            }
-            const float dx = __fsub_rn(c.x, p.x), dy = __fsub_rn(c.y, p.y), dz = __fsub_rn(c.z, p.z);
-            const float d2 = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
-            if (accept_cell(center[k].w, d2, theta)) {                   // :309
-                const float r2 = d2 + eps2;
-                const float rinv = rsqrtf(r2);
-                const float f = c.w * rinv * rinv * rinv;                // :280-290
-                ax += f * dx; ay += f * dy; az += f * dz;
-                if (COUNT) ++c_pc;
-                k = m.y;
-            } else {
-                k = m.x;                                                 // :293-297
-            }
-        }
-        const size_t o = (size_t)(i - i0) * 3;
-        acc3[o + 0] = ax; acc3[o + 1] = ay; acc3[o + 2] = az;
-    }
-    if (COUNT) {
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) {
-            c_vis += __shfl_down_sync(FULL, c_vis, s);
-            c_pc += __shfl_down_sync(FULL, c_pc, s);
-            c_pp += __shfl_down_sync(FULL, c_pp, s);
-        }
-        if ((threadIdx.x & 31) == 0) {
-            atomicAdd(&g->counters[0], c_vis);
-            atomicAdd(&g->counters[1], c_pc);
-            atomicAdd(&g->counters[2], c_pp);
-        }
-    }
-}
-
-// The accept decision of satisfies_opening_criterion (:302-310), bit for bit, at a
-// fraction of its cost: size * rsqrt(d2) decides unless it lands within 1e-5 of
-// theta, in which case the exact IEEE sqrt/divide sequence of the CPU code is
-// evaluated (rsqrt.approx is good to ~2^-22, so the fast verdict is certain
-// outside that band).
 __device__ __forceinline__ float rsqrt_fast(float x) {   // one MUFU.RSQ, flush-to-zero
     float r;
     asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
-}
-
-__device__ __forceinline__ bool accept_cell(float size, float d2, float theta) {
-    const float q = size * rsqrt_fast(d2);                 // d2 == 0 -> inf -> open, as size/0
-    if (fabsf(q - theta) > 1.0e-5f * theta) return q < theta;
-    return __fdiv_rn(size, __fsqrt_rn(d2)) < theta;
 }
 
 // Warp-cooperative walk: a warp owns 32 targets that are neighbours on a Hilbert curve and walks the
@@ -1194,8 +1109,6 @@ __device__ __forceinline__ bool accept_cell_d(float size, float dx, float dy, fl
     return __fdiv_rn(size, __fsqrt_rn(d2)) < theta;
 }
 
-// FIXED: the "fixed physics" walk -- leaf sources carry their real mass in .w and there is no
-// self test (with eps > 0 the self pair adds exactly 0; it is counted), softening = eps.
 __device__ __forceinline__ unsigned long long w_pk(float lo, float hi) {
     unsigned long long r;
     asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
@@ -1220,13 +1133,13 @@ __device__ __forceinline__ unsigned long long w_fma2(unsigned long long a, unsig
     return r;
 }
 
-// PERIODIC (fixed mode only): separations are taken to the nearest periodic image, d -= box*round(d/box)
+// PERIODIC (fixed-physics walk only): separations are taken to the nearest periodic image, d -= box*round(d/box)
 // (the minimum image of compute_forces_direct, src/physics/lambda_cdm_kernels.cu:39-41, which is also what
 // the reference's GPU tree kernel applies to its cells, src/forces/barnes_hut_tree.cu:247-254) -- for the
 // accept test and the monopole with roundf, for the pair rows with the packed magic-number rounding.
 // A cell that reaches across the half-box distance from the target (|d| + edge > box/2 on any axis) is
 // always opened: its particles need not share the image of its centre of mass.
-// POT (fixed mode, no counters): the same walk accumulating the potential phi_i = sum m / sqrt(|d|^2 + eps^2)
+// POT (fixed-physics walk, no counters): the same walk accumulating the potential phi_i = sum m / sqrt(|d|^2 + eps^2)
 // -- monopole M / r for an accepted cell -- instead of the acceleration; one float per target comes out.
 // The pair loop has no self test, so the i == i term m_i / eps is subtracted at the end; that is exact as
 // long as a target never accepts a cell that contains itself, i.e. theta <= 1/sqrt(3) (checked by the host).
@@ -1254,26 +1167,20 @@ __device__ __forceinline__ unsigned ends_first(unsigned cta, unsigned n_ctas) {
     return cta < tail ? n_ctas - tail + cta : cta - tail;
 }
 
-// FOREST: the octree arrives as the walk tables of several part builds (octant-sharded build: each part holds
-// the subtrees of its own octants of the root, the other octants are empty leaves there) plus one merged root
-// record.  A target tests the root once, then walks part after part -- octant order, i.e. the depth-first order
-// of the whole tree -- with the same loop; node ids are local to a part's table.
+// One target per lane: the "fixed physics" walk -- leaf sources carry their real mass in .w and there is no
+// self test (with eps > 0 the self pair adds exactly 0; it is counted), softening = eps.  128-thread CTAs, 9
+// resident per SM (56 registers).
 // by_slot: acc3 is indexed by the target's position in `order` (an explicit target list), not by index - i0.
-// MINB: resident 128-thread CTAs per SM the register budget is cut for (10 -> 48 registers, 9 -> 56, 8 -> 64).
-// EARLY: the record of the next visit is requested as soon as the successor is known (after the vote, before the
-// monopole arithmetic and the leaf range) instead of at the end of the visit.  Measured: no gain in either kernel,
-// and speculative requests (the skip target, or id + 1, before the vote) cost time -- every broadcast 256-bit load
-// writes 1 KB into the register file, and in the one-target kernel that return path (l1tex lsu writeback, 128 B per
-// clock and SM) is 76 % busy, as busy as the issue slots: a wrong guess is not free.
-template <bool COUNT, bool FIXED, bool PERIODIC = false, bool POT = false, bool FOREST = false, int MINB = 9,
-          bool EARLY = false>
-__global__ void __launch_bounds__(128, MINB)
+// The record of the next visit is requested at the end of a visit.  Requesting it as soon as the successor is
+// known (after the vote) measured no gain, and speculative requests (the skip target, or id + 1, before the vote)
+// cost time -- every broadcast 256-bit load writes 1 KB into the register file, and in this kernel that return path
+// (l1tex lsu writeback, 128 B per clock and SM) is 76 % busy, as busy as the issue slots: a wrong guess is not free.
+template <bool COUNT, bool PERIODIC, bool POT>
+__global__ void __launch_bounds__(128, 9)
 walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order, int i0, int n_targets,
                  const float4* __restrict__ nodes,
                  const ulonglong2* __restrict__ leaf_pairs, float theta, float theta2, float eps2, float box,
-                 float* __restrict__ acc3, TreeGlobals* __restrict__ g,
-                 const ForestTables* __restrict__ forest = nullptr, const float4* __restrict__ forest_root = nullptr,
-                 int by_slot = 0) {
+                 float* __restrict__ acc3, TreeGlobals* __restrict__ g, int by_slot) {
     typedef unsigned long long u64;
     const int t = ends_first(blockIdx.x, gridDim.x) * blockDim.x + threadIdx.x;
     const bool valid = t < n_targets;
@@ -1282,8 +1189,8 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
     if (valid) p = posm[i];
     float ax = 0.f, ay = 0.f, az = 0.f;                                  // cells
     u64 ax2 = 0ull, ay2 = 0ull, az2 = 0ull;                              // leaf pairs, two sources per lane-op
-    // theta2 = theta^2 (0 when theta <= 0: nothing is ever accepted) and eps2 (0.01f * 0.01f, :281-282, :334-335,
-    // or the fixed mode's eps^2) come from the host as kernel parameters: constant-bank operands, no registers
+    // theta2 = theta^2 (0 when theta <= 0: nothing is ever accepted) and eps2 = eps^2 come from the host as kernel
+    // parameters: constant-bank operands, no registers
     const u64 eps2_2 = w_pk(eps2, eps2);
     const u64 npx = w_pk(-p.x, -p.x), npy = w_pk(-p.y, -p.y), npz = w_pk(-p.z, -p.z);
     [[maybe_unused]] u64 inv_box2, magic2, nmagic2, nbox2;
@@ -1301,12 +1208,12 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                                           // lane is awake iff id >= wake
 
     // `cnt` leaf particles stored as pairs from pair `q` on, against this lane's target; on_lane = the
-    // lane takes part.  Branch-free packed rows: a lane that is out, or is the particle itself (:321), or a
+    // lane takes part.  Branch-free packed rows: a lane that is out, or is the particle itself, or a
     // padding slot, adds f = 0.
     auto leaf_range = [&](const ulonglong2* __restrict__ pairs, int q, int cnt, bool on_lane) {
         // A lane that is out takes eps^2 = +inf: rsqrt gives exactly 0 and every row adds 0 -- no select per row.
-        // The particle itself (:321) needs no test either: d = 0 makes its term exactly 0 (eps > 0); the index in
-        // .w is compared only when the interactions are being counted.  Padding slots are parked far away.
+        // The particle itself needs no test either: d = 0 makes its term exactly 0 (eps > 0).  Padding slots are
+        // parked far away with mass 0.
         const float e2 = on_lane ? eps2 : __int_as_float(0x7f800000);
         const u64 e2_2 = w_pk(e2, e2);
         auto row2 = [&](const ulonglong2& a, const ulonglong2& b) {      // a = {x0 x1 | y0 y1}, b = {z0 z1 | w0 w1}
@@ -1327,17 +1234,10 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                 return;
             }
             if (COUNT) c_slots += 2;                                     // every lane issues the row: two source slots
-            u64 f = w_mul2(w_mul2(rinv, rinv), rinv);                    // unit mass (:253, :340)
-            if (FIXED) f = w_mul2(f, b.y);
+            const u64 f = w_mul2(w_mul2(w_mul2(rinv, rinv), rinv), b.y);  // m / r^3
             ax2 = w_fma2(f, dx, ax2); ay2 = w_fma2(f, dy, ay2); az2 = w_fma2(f, dz, az2);
-            if (COUNT && !FIXED) {
-                float w0, w1;
-                w_unpk(b.y, w0, w1);
-                c_pp += (on_lane && __float_as_int(w0) != i && __float_as_int(w0) >= 0) +
-                        (on_lane && __float_as_int(w1) != i && __float_as_int(w1) >= 0);
-            }
         };
-        if (COUNT && FIXED && on_lane) c_pp += cnt;
+        if (COUNT && on_lane) c_pp += cnt;
         const ulonglong2* src = pairs + 2 * (size_t)q;
         const int np = (cnt + 1) >> 1;
         int k2 = 0;
@@ -1354,7 +1254,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
         }
     };
 
-    // a build that ran out of node slots (possible only in the fixed mode, whose node count has no a-priori
+    // a build that ran out of node slots (possible only in the fixed tree, whose node count has no a-priori
     // bound short of 2.3 N) left an incomplete tree: fail loudly rather than return a plausible force
     if (g->error) {
         if (valid) {
@@ -1411,7 +1311,6 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             };
             int nk = skip;
             if (!__any_sync(FULL, active & !(sure & accept))) {
-                if constexpr (EARLY) { if (nk < kend) ld256(record(nk), cn, mn); }
                 monopole(active);        // the common visit: every awake lane accepts the cell outright
             } else {
                 if (!sure) {             // the reference's own sequence, one rounding per operation
@@ -1421,7 +1320,6 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                 const bool open = active && !accept;
                 const bool descend = __any_sync(FULL, open);                 // :293-297
                 if (descend) nk = k + 1;
-                if constexpr (EARLY) { if (nk < kend) ld256(record(nk), cn, mn); }
                 monopole(active && accept);
                 if (descend) {
                     if (COUNT && open) c_vis += 8;                           // its 8 children, leaves included
@@ -1429,7 +1327,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                 }
             }
             B200_DEV_ASSERT(nk > k && nk <= kend);
-            if (!EARLY && nk < kend) ld256(record(nk), cn, mn);
+            if (nk < kend) ld256(record(nk), cn, mn);
             k = nk;
         };
         float4 c0, m0, c1, m1;
@@ -1440,44 +1338,12 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             visit(c1, m1, c0, m0);
         }
     };
-    if constexpr (!FOREST) {
-        // the root: massless -> nothing to do (:260); a leaf -> one pair loop (:268-270)
-        const float4* nd = nodes;
-        const ulonglong2* pairs = leaf_pairs;
-        const float4 c = nd[0];
-        const float4 mf = nd[1];
-        if (c.w != 0.0f) {
-            if (__float_as_int(mf.x) == ROOT_LEAF) leaf_range(pairs, 0, __float_as_int(mf.w), valid);
-            else walk_table(nd, pairs, 0, __float_as_int(mf.x));             // the root's skip = the record count
-        }
-    } else {
-        // the merged root: one accept test per target (:257-300 at depth 0), then part after part
-        const float4 c = forest_root[0], mf = forest_root[1];
-        if (c.w != 0.0f) {                                                   // :260
-            if (COUNT) { c_nl += 1; c_na += valid; }
-            const float dx = __fsub_rn(c.x, p.x), dy = __fsub_rn(c.y, p.y), dz = __fsub_rn(c.z, p.z);
-            const float d2 = fmaf(dz, dz, fmaf(dy, dy, dx * dx));
-            const bool accept = accept_cell_d(mf.z, dx, dy, dz, d2, theta, theta2);
-            const bool take = valid && accept, open = valid && !accept;
-            const float rinv = take ? rsqrt_fast(d2 + eps2) : 0.0f;
-            const float f = c.w * rinv * rinv * rinv;
-            ax = fmaf(f, dx, ax); ay = fmaf(f, dy, ay); az = fmaf(f, dz, az);
-            if (COUNT) c_pc += take;
-            if (take) wake = NEVER;                                          // the whole tree is one monopole for this target
-            if (__any_sync(FULL, open)) {
-                if (COUNT && open) c_vis += 8;
-                const int n_parts = forest->n_parts;
-                for (int q = 0; q < n_parts; ++q) {
-                    const float4* nd = forest->nodes[q];
-                    const ulonglong2* pairs = forest->leaf_pairs[q];
-                    const float4 r1 = nd[1];                                 // this part's root record: its own octants
-                    if (wake != NEVER) wake = 0;                             // a lane sleeping to the end of a part wakes here
-                    const int lcnt = __float_as_int(r1.w);
-                    if (lcnt > 0) leaf_range(pairs, __float_as_int(r1.y), lcnt, open);    // root children that are leaves
-                    walk_table(nd, pairs, 1, __float_as_int(r1.x));
-                }
-            }
-        }
+    // the root: massless -> nothing to do (:260); a leaf -> one pair loop (:268-270)
+    const float4 c = nodes[0];
+    const float4 mf = nodes[1];
+    if (c.w != 0.0f) {
+        if (__float_as_int(mf.x) == ROOT_LEAF) leaf_range(leaf_pairs, 0, __float_as_int(mf.w), valid);
+        else walk_table(nodes, leaf_pairs, 0, __float_as_int(mf.x));         // the root's skip = the record count
     }
     if (valid) {
         float lo, hi;
@@ -1517,10 +1383,16 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
 // unit the L1 return path counts) and one visit now serve 64 accept tests, and the whole visit runs in packed FP32:
 // a lane's A and B separations, |d|^2, screening test and monopole are the two halves of FADD2 / FFMA2 / FMUL2
 // operands.  A leaf range is summed for group A and for group B separately, each only if one of its own 32 targets
-// opened the cell, so the pair rows serve the same compact 32-target groups as in the one-target kernel and the
-// row loads are shared.  Decisions, interaction sets and counters are those of the one-target walk.
+// opened the cell, so the pair rows serve compact 32-target groups and the row loads are shared.  Decisions,
+// interaction sets and counters are those of a walk of one target at a time.
 // The reference's faithful tree only (unit-mass leaf pairs, eps = 0.01 literal from the host).
-template <bool COUNT, bool FOREST, int MINB, bool EARLY, int THREADS>
+// FOREST: the octree arrives as the walk tables of several part builds (octant-sharded build: each part holds
+// the subtrees of its own octants of the root, the other octants are empty leaves there) plus one merged root
+// record.  A target tests the root once, then walks part after part -- octant order, i.e. the depth-first order
+// of the whole tree -- with the same loop; node ids are local to a part's table.
+// MINB: resident CTAs per SM the register budget is cut for, in units of 64 threads (16 -> 64 registers).
+// by_slot: as in walk_warp_kernel.
+template <bool COUNT, bool FOREST, int MINB, int THREADS>
 __global__ void __launch_bounds__(THREADS, MINB * 64 / THREADS)
 walk_warp2_kernel(const float4* __restrict__ posm, const int* __restrict__ order, int i0, int n_targets,
                   const float4* __restrict__ nodes, const ulonglong2* __restrict__ leaf_pairs, float theta,
@@ -1639,7 +1511,6 @@ walk_warp2_kernel(const float4* __restrict__ posm, const int* __restrict__ order
             int nk = skip;
             // (bitwise on purpose: four independent compares and one combine, not a chain of dependent predicates)
             if (!__any_sync(FULL, (actA & !(sureA & accA)) | (actB & !(sureB & accB)))) {
-                if constexpr (EARLY) { if (nk < kend) ld256(record(nk), cn, mn); }
                 monopole(actA, actB);    // the common visit: every awake target accepts the cell outright
             } else {
                 auto exact = [&](float ddx, float ddy, float ddz) {          // :302-310, one rounding per operation
@@ -1655,7 +1526,6 @@ walk_warp2_kernel(const float4* __restrict__ posm, const int* __restrict__ order
                 const bool openA = actA && !accA, openB = actB && !accB;
                 const bool anyA = __any_sync(FULL, openA), anyB = __any_sync(FULL, openB);
                 if (anyA || anyB) nk = k + 1;                                // :293-297
-                if constexpr (EARLY) { if (nk < kend) ld256(record(nk), cn, mn); }
                 monopole(actA && accA, actB && accB);
                 if (anyA || anyB) {
                     if (COUNT) c_vis += (openA ? 8 : 0) + (openB ? 8 : 0);   // its 8 children, leaves included
@@ -1663,7 +1533,7 @@ walk_warp2_kernel(const float4* __restrict__ posm, const int* __restrict__ order
                 }
             }
             B200_DEV_ASSERT(nk > k && nk <= kend);
-            if (!EARLY && nk < kend) ld256(record(nk), cn, mn);
+            if (nk < kend) ld256(record(nk), cn, mn);
             k = nk;
         };
         float4 c0, m0, c1, m1;
@@ -1861,7 +1731,6 @@ static int tree_build_impl(b200_ctx* ctx, const void* posm4, const int* arrival,
     }
     B200_TRY(T->digit.reserve(n));
     B200_TRY(T->part_idx.reserve(n * sizeof(int)));
-    B200_TRY(T->part_pos.reserve(n * sizeof(float4)));
     B200_TRY(T->nodes.reserve((T->max_split + 2) * 2 * sizeof(float4)));     // walk records: internal nodes only
     B200_TRY(T->leaf_pos.reserve((n + T->max_split + 2) * sizeof(float4)));     // pair layout: <= 1 pad slot per parent
     B200_TRY(T->pscan.reserve((T->max_split + 2) * sizeof(int)));
@@ -2089,7 +1958,7 @@ static int tree_enqueue(b200_ctx* ctx, TreeState* T, cudaStream_t st, bool condi
     leaf_apply_kernel<1><<<pgrid, 256, 0, st>>>(g, max_depth, meta, lscan, tsum, pscan);
     stored_pos_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(
         g, T->part_idx.as<int>(), T->slot_node.as<int>(), meta, lscan, pscan, T->posm, (int)n,
-        T->part_pos.as<float4>(), T->leaf_pos.as<float>(), fixed ? 1 : 0);
+        T->leaf_pos.as<float>(), fixed ? 1 : 0);
     pair_pad_kernel<<<pgrid, 256, 0, st>>>(g, max_depth, lscan, pscan, T->leaf_pos.as<float>(), fixed ? 1 : 0);
     ctx->launches += 8;
     ctx->launches += pack_levels(0, deep ? shallow - 1 : max_depth, st);
@@ -2105,13 +1974,8 @@ static int tree_target_order(b200_ctx* ctx, TreeState* T, size_t i0, size_t n_ta
     B200_TRY(T->keys_sorted.reserve(n_targets * sizeof(uint32_t)));
     B200_TRY(T->order.reserve(n_targets * sizeof(int)));
     B200_TRY(T->sort_scratch.reserve(sort_scratch_bytes(n_targets)));
-    // warp grouping of the targets: Hilbert order (B200_WALK_ORDER=morton: the 30-bit Morton keys of row T1)
-    const char* ord = getenv("B200_WALK_ORDER");
-    if (ord && ord[0] == 'm' && !T->fixed)
-        B200_TRY(morton_keys(ctx, T->posm + i0, n_targets, T->box, T->keys.as<uint32_t>(), st));
-    else
-        B200_TRY(hilbert_keys(ctx, T->posm + i0, n_targets, T->box,
-                              T->fixed ? T->globals.as<TreeGlobals>()->root : nullptr, T->keys.as<uint32_t>(), st));
+    B200_TRY(hilbert_keys(ctx, T->posm + i0, n_targets, T->box,
+                          T->fixed ? T->globals.as<TreeGlobals>()->root : nullptr, T->keys.as<uint32_t>(), st));
     B200_TRY(sort_pairs(ctx, T->keys.as<uint32_t>(), n_targets, T->keys_sorted.as<uint32_t>(),
                         T->order.as<int>(), 30, T->sort_scratch.p, st));
     if (i0) {
@@ -2122,6 +1986,32 @@ static int tree_target_order(b200_ctx* ctx, TreeState* T, size_t i0, size_t n_ta
     B200_CUDA(cudaGetLastError());
     T->order_valid = true; T->order_i0 = i0; T->order_n = n_targets; T->order_age = 0;
     return B200_OK;
+}
+
+// The fixed-physics walk (one target per lane, 128-thread CTAs) of the targets order[0 .. n_targets), or of
+// [i0, i0 + n_targets) when order is null: accelerations, or with POT the potentials.
+template <bool COUNT, bool POT>
+static void launch_fixed_walk(const TreeState* T, const int* order, size_t i0, size_t n_targets, float theta,
+                              float* out, int by_slot, cudaStream_t st) {
+    const unsigned grid = (unsigned)((n_targets + 127) / 128);
+    const float theta2 = theta > 0.f ? theta * theta : 0.f;
+    auto kernel = T->periodic_box > 0.f ? walk_warp_kernel<COUNT, true, POT> : walk_warp_kernel<COUNT, false, POT>;
+    kernel<<<grid, 128, 0, st>>>(T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(),
+                                 T->leaf_pos.as<ulonglong2>(), theta, theta2, T->eps * T->eps, T->periodic_box, out,
+                                 T->globals.as<TreeGlobals>(), by_slot);
+}
+
+// The faithful tree's walk (two targets per lane), of this context's tree or (FOREST) of the published forest.
+template <bool COUNT, bool FOREST, int MINB, int THREADS>
+static void launch_walk2(const TreeState* T, const int* order, size_t i0, size_t n_targets, float theta,
+                         float* acc3, int by_slot, cudaStream_t st) {
+    const unsigned groups = (unsigned)((n_targets + 63) / 64);           // 64 targets per warp
+    const float theta2 = theta > 0.f ? theta * theta : 0.f;
+    const float eps2 = 0.01f * 0.01f;                                   // :281-282, :334-335
+    const ForestTables* forest = T->forest_root.p ? (const ForestTables*)(T->forest_root.as<char>() + 64) : nullptr;
+    walk_warp2_kernel<COUNT, FOREST, MINB, THREADS><<<(groups * 32 + THREADS - 1) / THREADS, THREADS, 0, st>>>(
+        T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(), T->leaf_pos.as<ulonglong2>(), theta, theta2,
+        eps2, acc3, T->globals.as<TreeGlobals>(), forest, T->forest_root.as<float4>(), by_slot);
 }
 
 // Targets: the index range [i0, i0 + n_targets) (list == nullptr; warps are formed from a Hilbert order of the
@@ -2145,79 +2035,25 @@ static int tree_walk_impl(b200_ctx* ctx, const int* list, size_t i0, size_t n_ta
         order = T->order.as<int>();
     }
     const int by_slot = list ? 1 : 0;
-    TreeGlobals* g = T->globals.as<TreeGlobals>();
-    const unsigned grid = (unsigned)((n_targets + 127) / 128);
     if (T->counting) {
-        zero_counters_kernel<<<1, 1, 0, st>>>(g);
+        zero_counters_kernel<<<1, 1, 0, st>>>(T->globals.as<TreeGlobals>());
         ctx->launches += 1;
     }
     if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev0, st));
-    const bool per_thread = !T->fixed && !forest && !list && getenv("B200_WALK_PER_THREAD") != nullptr;     // tuning hook
-    const float theta2 = theta > 0.f ? theta * theta : 0.f;
-    const float eps2 = T->fixed ? T->eps * T->eps : 0.01f * 0.01f;
-    // launch macros for the walk's instances.  One-target kernel <COUNT, FIXED, PERIODIC, POT, FOREST, MINB, EARLY>:
-    // the fixed-physics modes, 128-thread CTAs, 9 resident per SM (56 registers).  Two-target kernel
-    // <COUNT, FOREST, MINB, EARLY, THREADS>: the reference-faithful tree (the hot path), MINB = resident CTAs per SM
-    // in units of 64 threads (16 -> 64 registers).
-#define B200_WALK_V(COUNT_, FIXED_, PERIODIC_, FOREST_, MINB_, EARLY_)                                           \
-    walk_warp_kernel<COUNT_, FIXED_, PERIODIC_, false, FOREST_, MINB_, EARLY_><<<grid, 128, 0, st>>>(            \
-        T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(),                                          \
-        T->leaf_pos.as<ulonglong2>(), theta, theta2, eps2, T->periodic_box, (float*)acc3, g,                     \
-        T->forest_root.as<ForestTables>() ? (const ForestTables*)(T->forest_root.as<char>() + 64) : nullptr,     \
-        T->forest_root.as<float4>(), by_slot)
-#define B200_WALK(COUNT_, FIXED_, PERIODIC_, FOREST_) B200_WALK_V(COUNT_, FIXED_, PERIODIC_, FOREST_, 9, false)
-    const unsigned groups = (unsigned)((n_targets + 63) / 64);           // 64 targets per warp
-#define B200_WALK2(COUNT_, FOREST_, MINB_, EARLY_, THREADS_)                                                     \
-    walk_warp2_kernel<COUNT_, FOREST_, MINB_, EARLY_, THREADS_>                                                  \
-        <<<(groups * 32 + THREADS_ - 1) / THREADS_, THREADS_, 0, st>>>(                                          \
-        T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(), T->leaf_pos.as<ulonglong2>(), theta,     \
-        theta2, eps2, (float*)acc3, g,                                                                           \
-        T->forest_root.as<ForestTables>() ? (const ForestTables*)(T->forest_root.as<char>() + 64) : nullptr,     \
-        T->forest_root.as<float4>(), by_slot)
-    // Tuning hook (B200_WALK_VARIANT): 0 = two targets per lane, 256-thread CTAs (adjacent groups share the L1;
-    // 1.79 ms per 2^20 uniform targets), 1 = the same with 64-thread CTAs (1.83 ms), 2 = EARLY (1.88 ms),
-    // 3 = the one-target kernel (2.00 ms), 4 = two targets, 128-thread CTAs, 72 registers (1.83 ms).
-    // Tried and removed: persistent warps fed by an SM-local scheduler (a contiguous range of groups per SM, common
-    // pool for the tail) -- L1 hit rate 63 % against 69 %, 1.90 ms; a 48-register build (40 warps per SM) -- 2.11 ms.
-    static const int variant = getenv("B200_WALK_VARIANT") ? atoi(getenv("B200_WALK_VARIANT")) : 0;
-#define B200_WALK_HOT(FOREST_)                                                                                   \
-    switch (variant) {                                                                                           \
-        case 1:  B200_WALK2(false, FOREST_, 16, false, 64); break;                                               \
-        case 2:  B200_WALK2(false, FOREST_, 16, true, 256); break;                                               \
-        case 3:  B200_WALK_V(false, false, false, FOREST_, 9, false); break;                                     \
-        case 4:  B200_WALK2(false, FOREST_, 14, false, 128); break;                                              \
-        default:                                                                                                 \
-            /* the forest instance keeps 8 more values live (part loop): at 64 registers they spill inside the   \
-               walk loop; 72 registers (7 CTAs of 128 threads) measured 4.5 % faster on 8 GPUs */               \
-            if (FOREST_) B200_WALK2(false, FOREST_, 14, false, 128);                                             \
-            else B200_WALK2(false, FOREST_, 16, false, 256);                                                     \
-            break;                                                                                               \
-    }
-#define B200_WALK_HOT_COUNT(FOREST_)                                                                             \
-    if (variant == 3) B200_WALK(true, false, false, FOREST_); else B200_WALK2(true, FOREST_, 12, false, 256);
+    float* out = (float*)acc3;
+    // The faithful tree's instances: 256-thread CTAs, in which adjacent groups share the L1.  The forest instance
+    // keeps 8 more values live (part loop): at 64 registers they spill inside the walk loop; 72 registers (7 CTAs of
+    // 128 threads) measured 4.5 % faster on 8 GPUs.
     if (forest) {
-        if (T->counting) { B200_WALK_HOT_COUNT(true) }
-        else B200_WALK_HOT(true)
+        if (T->counting) launch_walk2<true, true, 12, 256>(T, order, i0, n_targets, theta, out, by_slot, st);
+        else launch_walk2<false, true, 14, 128>(T, order, i0, n_targets, theta, out, by_slot, st);
     } else if (T->fixed) {
-        const bool periodic = T->periodic_box > 0.f;
-        if (T->counting) { if (periodic) B200_WALK(true, true, true, false); else B200_WALK(true, true, false, false); }
-        else             { if (periodic) B200_WALK(false, true, true, false); else B200_WALK(false, true, false, false); }
-    } else if (!per_thread) {
-        if (T->counting) { B200_WALK_HOT_COUNT(false) }
-        else B200_WALK_HOT(false)
-#undef B200_WALK
-#undef B200_WALK_V
-#undef B200_WALK2
-#undef B200_WALK_HOT
-#undef B200_WALK_HOT_COUNT
-    } else if (T->counting)
-        walk_kernel<true><<<grid, 128, 0, st>>>(T->posm, order, (int)i0, (int)n_targets,
-                                                T->com.as<float4>(), T->center.as<float4>(), T->meta.as<int4>(),
-                                                T->part_pos.as<float4>(), theta, (float*)acc3, g);
-    else
-        walk_kernel<false><<<grid, 128, 0, st>>>(T->posm, order, (int)i0, (int)n_targets,
-                                                 T->com.as<float4>(), T->center.as<float4>(), T->meta.as<int4>(),
-                                                 T->part_pos.as<float4>(), theta, (float*)acc3, g);
+        if (T->counting) launch_fixed_walk<true, false>(T, order, i0, n_targets, theta, out, by_slot, st);
+        else launch_fixed_walk<false, false>(T, order, i0, n_targets, theta, out, by_slot, st);
+    } else {
+        if (T->counting) launch_walk2<true, false, 12, 256>(T, order, i0, n_targets, theta, out, by_slot, st);
+        else launch_walk2<false, false, 16, 256>(T, order, i0, n_targets, theta, out, by_slot, st);
+    }
     if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev1, st));
     B200_CUDA(cudaGetLastError());
     ctx->launches += 1;
@@ -2360,18 +2196,7 @@ int tree_potential(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, void
     if (n_targets == 0) return B200_OK;
     if (!phi || i0 + n_targets > T->n) return B200_ERR_INVALID;
     B200_TRY(tree_target_order(ctx, T, i0, n_targets, st));
-    TreeGlobals* g = T->globals.as<TreeGlobals>();
-    const unsigned grid = (unsigned)((n_targets + 127) / 128);
-    const float theta2 = theta > 0.f ? theta * theta : 0.f;
-    const float eps2 = T->eps * T->eps;
-    if (T->periodic_box > 0.f)
-        walk_warp_kernel<false, true, true, true><<<grid, 128, 0, st>>>(
-            T->posm, T->order.as<int>(), (int)i0, (int)n_targets, T->nodes.as<float4>(),
-            T->leaf_pos.as<ulonglong2>(), theta, theta2, eps2, T->periodic_box, (float*)phi, g);
-    else
-        walk_warp_kernel<false, true, false, true><<<grid, 128, 0, st>>>(
-            T->posm, T->order.as<int>(), (int)i0, (int)n_targets, T->nodes.as<float4>(),
-            T->leaf_pos.as<ulonglong2>(), theta, theta2, eps2, T->periodic_box, (float*)phi, g);
+    launch_fixed_walk<false, true>(T, T->order.as<int>(), i0, n_targets, theta, (float*)phi, 0, st);
     B200_CUDA(cudaGetLastError());
     ctx->launches += 1;
     return B200_OK;

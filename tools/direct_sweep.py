@@ -1,5 +1,5 @@
 """Tuning harness for the direct-sum kernel: times every register-blocking
-variant (B200_DIRECT_VARIANT = "R,MINB") with CUDA events on one problem size and
+variant (B200_DIRECT_VARIANT = "R,THREADS,MINB") with CUDA events on one problem size and
 prints interactions/s and the fraction of the measured FP32 peak."""
 import argparse
 import os
@@ -32,14 +32,11 @@ def main():
     eng.set_timing(True)
     ref = None
     for v in args.variants.split(";"):
-        # periodic only: "float:" / "mixed:" prefix picks the minimum-image flavour (default: fixed point)
+        # periodic only: a "float:" prefix picks the FP32 minimum image (default: fixed point)
         os.environ.pop("B200_DIRECT_PERIODIC_FLOAT", None)
-        os.environ.pop("B200_DIRECT_PERIODIC_MIXED", None)
         label = v
         if v.startswith("float:"):
             os.environ["B200_DIRECT_PERIODIC_FLOAT"] = "1"; v = v[6:]
-        elif v.startswith("mixed:"):
-            os.environ["B200_DIRECT_PERIODIC_MIXED"] = "1"; v = v[6:]
         if v.startswith("default"):
             os.environ.pop("B200_DIRECT_VARIANT", None)
             v = "default"

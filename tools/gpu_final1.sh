@@ -10,9 +10,9 @@ python -c "import __graft_entry__ as g; g.smoke()" > $O/smoke_final.log 2>&1; ec
 ncu --metrics gpu__time_duration.sum --clock-control none -c 900 --csv --log-file $O/r2_bench_launches.csv \
     python bench.py --steps 2 --warmup 3 --no-cpu --no-c5 > $O/ncu_bench_final.log 2>&1; echo "ncu list rc=$?" >> $O/final1.log
 ncu --set full --clock-control none --import-source on -k regex:walk_warp2 -c 1 -f -o $O/r2_walk_final \
-    python tools/tree_bench.py --no-thread > $O/ncu_walk_final.log 2>&1; echo "ncu walk rc=$?" >> $O/final1.log
+    python tools/tree_bench.py > $O/ncu_walk_final.log 2>&1; echo "ncu walk rc=$?" >> $O/final1.log
 python tools/tree_bench.py > $O/tree_bench_final.log 2>&1
 python tools/tree_bench.py --dist clustered >> $O/tree_bench_final.log 2>&1
 python tools/tree_bench.py --dist box >> $O/tree_bench_final.log 2>&1
-python tools/tree_bench.py --no-thread --n 16777216 >> $O/tree_bench_final.log 2>&1
-cat $O/final1.log; tail -3 $O/pytest_gpu_final.log; cat $O/smoke_final.log | tail -2; grep "build\|walk\[" $O/tree_bench_final.log | cut -c1-110
+python tools/tree_bench.py --n 16777216 >> $O/tree_bench_final.log 2>&1
+cat $O/final1.log; tail -3 $O/pytest_gpu_final.log; cat $O/smoke_final.log | tail -2; grep "build\|^walk " $O/tree_bench_final.log | cut -c1-110

@@ -1,5 +1,5 @@
 """Times leapfrog_kernel (fused kick-kick-drift) at n particles with CUDA events: 68 B per particle against the
-measured HBM copy bandwidth.  B200_LEAPFROG=v1 selects the round-1 kernel (strided 128-bit accesses)."""
+measured HBM copy bandwidth."""
 import argparse
 import json
 import os
@@ -23,7 +23,6 @@ def main():
     eng = b200grav.Engine(0)
     D = bench.Dist(torch, dist, 1, 0, torch.device("cuda", 0))
     out = bench.leapfrog_roofline(eng, D, args.n)
-    out["variant"] = os.environ.get("B200_LEAPFROG", "tile (default)")
     print(json.dumps(out))
     eng.close()
 

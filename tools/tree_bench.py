@@ -1,5 +1,4 @@
-"""Times the Barnes-Hut build and the two walk kernels (warp-cooperative default,
-per-thread via B200_WALK_PER_THREAD=1) with CUDA events and cross-checks them."""
+"""Times the Barnes-Hut build and the walk with CUDA events and prints the walk's interaction counters."""
 import argparse
 import os
 import sys
@@ -17,7 +16,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=1 << 20)
     ap.add_argument("--dist", default="uniform", choices=["uniform", "box", "clustered"])
-    ap.add_argument("--no-thread", action="store_true", help="skip the per-thread cross-check kernel")
     args = ap.parse_args()
     n = args.n
     rng = np.random.default_rng(42)
@@ -42,33 +40,23 @@ def main():
     torch.cuda.synchronize()
     print(f"n={n} dist={args.dist}  build {ev0.elapsed_time(ev1) / 5:.3f} ms  stats {eng.tree_stats()}")
     eng.set_timing(True)
-    res = {}
-    for mode in (("warp",) if args.no_thread else ("warp", "thread")):
-        if mode == "thread":
-            os.environ["B200_WALK_PER_THREAD"] = "1"
-        else:
-            os.environ.pop("B200_WALK_PER_THREAD", None)
-        best = 1e30
-        for _ in range(4):
-            eng.tree_walk_dev(acc, 0, n, 0.5)
-            torch.cuda.synchronize()
-            best = min(best, eng.last_kernel_ms())
-        res[mode] = acc.cpu().numpy().copy()
-        eng.tree_set_counting(True)
+    best = 1e30
+    for _ in range(4):
         eng.tree_walk_dev(acc, 0, n, 0.5)
         torch.cuda.synchronize()
-        cnt = eng.tree_counters()
-        st = [int(x) for x in eng.tree_walk_stats()]
-        eng.tree_set_counting(False)
-        inter = float(cnt[1] + cnt[2])
-        print(f"walk[{mode:6s}] {best:8.3f} ms  {inter / best / 1e-3:.3e} interactions/s  counters {list(map(int, cnt))}  "
-              f"per target: {cnt[0] / n:.0f} visits {cnt[1] / n:.0f} cells {cnt[2] / n:.0f} pairs")
-        if mode == "warp" and st[3] and st[4]:
-            print(f"   lane use: pair-row slots issued {st[3]} (useful {st[2] / st[3]:.3f}), node-visit target slots issued "
-                  f"{st[4]} (awake {st[5] / st[4]:.3f}; {st[4] / n:.0f} per target)")
-    if not args.no_thread:
-        d = res["warp"].astype(np.float64) - res["thread"]
-        print("warp vs thread rel-L2:", float(np.sqrt((d * d).sum() / (res["thread"].astype(np.float64) ** 2).sum())))
+        best = min(best, eng.last_kernel_ms())
+    eng.tree_set_counting(True)
+    eng.tree_walk_dev(acc, 0, n, 0.5)
+    torch.cuda.synchronize()
+    cnt = eng.tree_counters()
+    st = [int(x) for x in eng.tree_walk_stats()]
+    eng.tree_set_counting(False)
+    inter = float(cnt[1] + cnt[2])
+    print(f"walk {best:8.3f} ms  {inter / best / 1e-3:.3e} interactions/s  counters {list(map(int, cnt))}  "
+          f"per target: {cnt[0] / n:.0f} visits {cnt[1] / n:.0f} cells {cnt[2] / n:.0f} pairs")
+    if st[3] and st[4]:
+        print(f"   lane use: pair-row slots issued {st[3]} (useful {st[2] / st[3]:.3f}), node-visit target slots issued "
+              f"{st[4]} (awake {st[5] / st[4]:.3f}; {st[4] / n:.0f} per target)")
     eng.close()
 
 
