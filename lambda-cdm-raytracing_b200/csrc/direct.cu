@@ -30,9 +30,6 @@
 //  * per-tile FP32 partial sums are folded into FP64 running sums, so the
 //    round-off does not grow like sqrt(N_sources) (the sequential FP32 CPU
 //    loop is 8.6e-6 from FP64 truth at 64 K sources already).
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "direct.cuh"
 
@@ -573,39 +570,10 @@ int direct_forces(b200_ctx* ctx, const DirectSources& src, const void* targets4,
     // and the last, partly filled target block wastes little; 2 targets/thread below that.
     const long long units8 = (((long long)n_targets + 2047) / 2048) * (long long)src.total_tiles;
     const bool small = n_targets < 4 * 2048 || units8 < 4ll * ctx->sm_count;
-    if (const char* v = getenv("B200_DIRECT_VARIANT")) {      // tuning hook: "R,THREADS,MINB"
-        int r = 0, th = 0, mb = 0;
-        if (sscanf(v, "%d,%d,%d", &r, &th, &mb) == 3 && box > 0.f) {
-            const bool fp = getenv("B200_DIRECT_PERIODIC_FLOAT") != nullptr;
-#define B200_PVARIANT(RR, TH, MB) \
-    if (r == RR && th == TH && mb == MB) \
-        return fp ? launch_direct<RR, TH, MB, PMODE_FLOAT>(ctx, src, tg, n_targets, eps, box, out, mass_diff, st) \
-                  : launch_direct<RR, TH, MB, PMODE_FIXED_XY>(ctx, src, tg, n_targets, eps, box, out, mass_diff, st);
-            B200_PVARIANT(4, 256, 1) B200_PVARIANT(8, 256, 1) B200_PVARIANT(4, 512, 1)
-#undef B200_PVARIANT
-            return B200_ERR_UNSUPPORTED;
-        }
-        if (sscanf(v, "%d,%d,%d", &r, &th, &mb) == 3 && box == 0.f) {
-#define B200_VARIANT(RR, TH, MB) \
-    if (r == RR && th == TH && mb == MB) \
-        return launch_direct<RR, TH, MB, PMODE_OPEN>(ctx, src, tg, n_targets, eps, box, out, mass_diff, st);
-            B200_VARIANT(2, 256, 2) B200_VARIANT(4, 256, 1) B200_VARIANT(4, 256, 2) B200_VARIANT(5, 256, 1)
-            B200_VARIANT(6, 256, 1) B200_VARIANT(8, 256, 1) B200_VARIANT(4, 384, 1) B200_VARIANT(4, 512, 1)
-            B200_VARIANT(3, 512, 1) B200_VARIANT(6, 128, 2) B200_VARIANT(8, 128, 2) B200_VARIANT(7, 256, 1)
-            B200_VARIANT(6, 384, 1) B200_VARIANT(5, 384, 1) B200_VARIANT(8, 192, 1) B200_VARIANT(6, 320, 1)
-            B200_VARIANT(10, 256, 1) B200_VARIANT(5, 128, 3) B200_VARIANT(4, 128, 4)
-            B200_VARIANT(2, 256, 3) B200_VARIANT(2, 256, 4) B200_VARIANT(3, 256, 2) B200_VARIANT(3, 256, 3)
-            B200_VARIANT(2, 512, 2) B200_VARIANT(2, 1024, 1) B200_VARIANT(1, 256, 8) B200_VARIANT(1, 512, 4)
-#undef B200_VARIANT
-            return B200_ERR_UNSUPPORTED;
-        }
-    }
     if (box > 0.f) {
         // fixed-point x, y only while the position quantum (box * 2^-33) is below ~1e-6 eps, and never
-        // for small problems (launch-bound anyway); B200_DIRECT_PERIODIC_FLOAT forces the FP32 minimum image (A/B)
-        const long long units4 = (((long long)n_targets + 2047) / 2048) * (long long)src.total_tiles;
-        const bool fixed_ok = eps >= 1e-4f * box && n_targets >= 4 * 2048 && units4 >= 4ll * ctx->sm_count &&
-                              getenv("B200_DIRECT_PERIODIC_FLOAT") == nullptr;
+        // for small problems (launch-bound anyway)
+        const bool fixed_ok = eps >= 1e-4f * box && !small;
         if (fixed_ok)
             return launch_direct<4, 512, 1, PMODE_FIXED_XY>(ctx, src, tg, n_targets, eps, box, out, mass_diff, st);
         return small ? launch_direct<2, 256, 2, PMODE_FLOAT>(ctx, src, tg, n_targets, eps, box, out, mass_diff, st)

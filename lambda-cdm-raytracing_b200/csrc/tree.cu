@@ -1748,9 +1748,9 @@ static int tree_build_impl(b200_ctx* ctx, const void* posm4, const int* arrival,
     B200_TRY(T->split_local.reserve(T->max_split * 8 * sizeof(unsigned)));
     B200_TRY(T->split_cstart.reserve(T->max_split * 8 * sizeof(unsigned)));
 
-    // graph replay (B200_NO_GRAPH=1: plain launches).  The graph runs on the context's own stream,
-    // ordered after / before the caller's stream by events; a caller that is itself capturing gets
-    // the plain launches on its stream instead (they become part of its graph).
+    // graph replay, the deep levels behind IF nodes (B200_NO_GRAPH=1: plain launches).  The graph runs on the
+    // context's own stream, ordered after / before the caller's stream by events; a caller that is itself
+    // capturing gets the unconditional plain launches on its stream instead (they become part of its graph).
     cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
     if (st != nullptr && cudaStreamIsCapturing(st, &cap_status) != cudaSuccess) { cudaGetLastError(); cap_status = cudaStreamCaptureStatusNone; }
     if (getenv("B200_NO_GRAPH") == nullptr && cap_status == cudaStreamCaptureStatusNone && ctx->stream != nullptr) {
@@ -1760,7 +1760,7 @@ static int tree_build_impl(b200_ctx* ctx, const void* posm4, const int* arrival,
             cudaGraph_t graph = nullptr;
             if (cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
                 const uint64_t before = ctx->launches;
-                const int rc = tree_enqueue(ctx, T, ctx->stream, getenv("B200_NO_COND") == nullptr);
+                const int rc = tree_enqueue(ctx, T, ctx->stream, true);
                 const cudaError_t ce = cudaStreamEndCapture(ctx->stream, &graph);
                 T->graph_launches = (int)(ctx->launches - before);
                 ctx->launches = before;

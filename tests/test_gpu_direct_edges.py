@@ -7,9 +7,12 @@ device's SM count, and test_every_instance_is_reached runs this file's case list
 instance exists in an equal-mass (UNIT, chosen on the device) and a general-mass version.
 
 Gates: forces 1e-5 relative L2 against float64, potential 2e-6 max relative (test_gpu_direct.py, test_gpu_energy.py).
-Also here: the production periodic configuration's route (bitwise), the half-box tie contract of both periodic
-paths, frame and whole-period invariance (bitwise, dyadic input), mass and coordinate edges, non-finite inputs on
-every path, shard sums of the energy and the multi-part (peer-memory) source path."""
+Every path is reached the way a caller reaches it: the periodic fixed-point path at eps >= fl(1e-4f * box) when the
+call is not small, the FP32 minimum image one float below that bound (_fixed_eps_bound / _float_eps).
+
+Also here: the production periodic configuration's route (by how it resolves half-box ties), the half-box tie
+contract of both periodic paths, frame and whole-period invariance (bitwise, dyadic input), mass and coordinate
+edges, non-finite inputs on every path, shard sums of the energy and the multi-part (peer-memory) source path."""
 import numpy as np
 import pytest
 import torch
@@ -23,8 +26,6 @@ TOL = 1e-5
 POT_TOL = 2e-6
 TILE = 512
 SM = torch.cuda.get_device_properties(0).multi_processor_count if torch.cuda.is_available() else 148
-FIXED_ENV = {"B200_DIRECT_VARIANT": "4,512,1"}             # periodic: the fixed-point x/y instance, R4 x 512
-FLOAT_ENV = {"B200_DIRECT_PERIODIC_FLOAT": "1"}            # periodic: the FP32 minimum image only
 
 
 # ---- the dispatch rule, restated -------------------------------------------------------------------------------------
@@ -33,12 +34,22 @@ def _tiles(ns):
     return -(-ns // TILE)
 
 
-def _force_instance(nt, tiles, eps, box, sm=SM, force_float=False):
+def _fixed_eps_bound(box):
+    """fl(1e-4f * box): the smallest eps the fixed-point path takes."""
+    return np.float32(np.float32(1e-4) * np.float32(box))
+
+
+def _float_eps(box):
+    """One float below _fixed_eps_bound: the FP32 minimum image at every size."""
+    return float(np.nextafter(_fixed_eps_bound(box), np.float32(0)))
+
+
+def _force_instance(nt, tiles, eps, box, sm=SM):
     units = -(-nt // 2048) * tiles
     small = nt < 4 * 2048 or units < 4 * sm
     if box == 0:
         return "OPEN_R2" if small else "OPEN_R8"
-    fixed_ok = np.float32(eps) >= np.float32(np.float32(1e-4) * np.float32(box)) and not small and not force_float
+    fixed_ok = np.float32(eps) >= _fixed_eps_bound(box) and not small
     return "FIXED_R4" if fixed_ok else ("FLOAT_R2" if small else "FLOAT_R4")
 
 
@@ -82,13 +93,6 @@ def _potential(engine, posm, i0, nt, eps, box):
     engine.direct_potential_dev(posm, phi, i0, nt, eps=eps, box=box)
     torch.cuda.synchronize()
     return phi.cpu().numpy()
-
-
-def _with_env(monkeypatch, env):
-    for k in ("B200_DIRECT_VARIANT", "B200_DIRECT_PERIODIC_FLOAT"):
-        monkeypatch.delenv(k, raising=False)
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
 
 
 def _sample(i0, nt, k, seed=0):
@@ -163,9 +167,8 @@ FORCE_CASES = [
 
 @pytest.mark.parametrize("unit", [True, False], ids=["unit", "general"])
 @pytest.mark.parametrize("case", FORCE_CASES, ids=[c[0] for c in FORCE_CASES])
-def test_force_instance_vs_float64(engine, oracle, monkeypatch, case, unit):
+def test_force_instance_vs_float64(engine, oracle, case, unit):
     name, ns, i0, nt, eps, box = case
-    _with_env(monkeypatch, {})
     pos, mass = _cloud(ns, box, len(name)), _mass(ns, unit, ns)
     a = _forces(engine, _posm(pos, mass), i0, nt, eps, box)
     idx = _sample(i0, nt, 512 if ns <= 65536 else 384)
@@ -176,9 +179,8 @@ def test_force_instance_vs_float64(engine, oracle, monkeypatch, case, unit):
 
 
 @pytest.mark.parametrize("box", [0.0, 100.0])
-def test_one_target_against_two_to_the_20(engine, oracle, monkeypatch, box):
+def test_one_target_against_two_to_the_20(engine, oracle, box):
     """nt = 1: one target block spread over every CTA, the finalize pass adds one record per CTA."""
-    _with_env(monkeypatch, {})
     n = 1 << 20
     pos, mass = _cloud(n, box, 5), _mass(n, False, 6)
     posm = _posm(pos, mass)
@@ -199,38 +201,39 @@ def production():
     return pos, idx
 
 
-def test_production_periodic_route(engine, monkeypatch, production):
+def test_production_periodic_route_by_tie_images(engine, production):
     """2^20 particles in [0, 100), eps = 0.01: fl(0.01) == fl(1e-4f * 100), so the fixed-point path is taken on the
-    equality; one float below it the FP32 minimum image runs."""
+    equality; one float below it the FP32 minimum image runs.
+
+    The witness of the path: a half-box tie in the origin-centred frame takes the flipped image on the fixed-point
+    path and keeps its raw sign on the FP32 path at box 100 (test_fixed_point_encoding.py).  It runs at N_F, where
+    the rule makes the same choice as at 2^20 (_planted_ties finds no free x slot at 2^20)."""
+    box, eps = 100.0, 0.01
+    below = _float_eps(box)
+    assert np.float32(eps) == _fixed_eps_bound(box)
+    pos, mass, tgt = _planted_ties(N_F, box, 100)
+    p = _centred(pos, box)
+    for e, path, ties in ((eps, "FIXED_R4", "flip"), (below, "FLOAT_R4", "raw")):
+        assert _force_instance(N_F, _tiles(N_F), e, box) == path
+        want = {t: direct_np.forces(p, mass, e, box, targets=tgt, ties=t) for t in ("raw", "flip")}
+        assert _row_err(want["flip"], want["raw"]).min() > 100 * TIE_TOL
+        err = _row_err(_forces(engine, _posm(p, mass), 0, N_F, e, box)[tgt], want[ties])
+        print(f"production route witness {path}: {ties} image, max error {err.max():.2e}")
+        assert np.all(err < TIE_TOL), path
     pos, idx = production
     n = pos.shape[0]
     posm = _posm(pos, np.ones(n, np.float32))
-    assert np.float32(0.01) == np.float32(np.float32(1e-4) * np.float32(100.0))
-    assert _force_instance(n, _tiles(n), 0.01, 100.0) == "FIXED_R4"
-    _with_env(monkeypatch, {})
-    dflt = _forces(engine, posm, 0, n, 0.01, 100.0)
-    _with_env(monkeypatch, FIXED_ENV)
-    fixed = _forces(engine, posm, 0, n, 0.01, 100.0)
-    _with_env(monkeypatch, FLOAT_ENV)
-    flt = _forces(engine, posm, 0, n, 0.01, 100.0)
-    assert np.array_equal(dflt, fixed) and not np.array_equal(dflt, flt)
-    want = direct_np.forces(pos, None, 0.01, 100.0, targets=idx)
-    e_fixed, e_float = rel_l2(fixed[idx], want), rel_l2(flt[idx], want)
-    print(f"production FIXED_R4 {e_fixed:.2e} FLOAT_R4 {e_float:.2e}")
-    assert e_fixed < TOL and e_float < TOL
-    below = float(np.nextafter(np.float32(0.01), np.float32(0)))
-    assert _force_instance(n, _tiles(n), below, 100.0) == "FLOAT_R4"
-    _with_env(monkeypatch, {})
-    b_dflt = _forces(engine, posm, 0, n, below, 100.0)
-    _with_env(monkeypatch, FLOAT_ENV)
-    assert np.array_equal(b_dflt, _forces(engine, posm, 0, n, below, 100.0))
+    for e, path in ((eps, "FIXED_R4"), (below, "FLOAT_R4")):
+        assert _force_instance(n, _tiles(n), e, box) == path
+        err = rel_l2(_forces(engine, posm, 0, n, e, box)[idx], direct_np.forces(pos, None, e, box, targets=idx))
+        print(f"production {path} eps {e:.9g}: {err:.2e}")
+        assert err < TOL
 
 
-def test_production_float_r4_small_eps(engine, monkeypatch, production):
+def test_production_float_r4_small_eps(engine, production):
     pos, idx = production
     n = pos.shape[0]
     m = _mass(n, False, 3)
-    _with_env(monkeypatch, {})
     assert _force_instance(n, _tiles(n), 1e-3, 100.0) == "FLOAT_R4"
     a = _forces(engine, _posm(pos, m), 0, n, 1e-3, 100.0)
     err = rel_l2(a[idx], direct_np.forces(pos, m, 1e-3, 100.0, targets=idx))
@@ -258,6 +261,11 @@ def _centred(pos, box):
     return np.where(pos >= box / 2, pos - np.float32(box), pos).astype(np.float32)
 
 
+def _row_err(a, want):
+    """Relative error of each row."""
+    return np.linalg.norm(a - want, axis=1) / np.linalg.norm(want, axis=1)
+
+
 def _planted_ties(n, box, seed, n_pairs=32, heavy=1000.0):
     """A tie-free cloud plus n_pairs light targets, each exactly half a box (on x) from one heavy partner and from
     nothing else.  Returns pos, mass, target indices."""
@@ -275,25 +283,25 @@ def _planted_ties(n, box, seed, n_pairs=32, heavy=1000.0):
 
 
 @pytest.mark.parametrize("box", [64.0, 100.0, 1000.0])
-def test_half_box_ties_take_one_of_the_two_images(engine, oracle, monkeypatch, box):
+def test_half_box_ties_take_one_of_the_two_images(engine, oracle, box):
     """A tie resolves to one of the two images on both periodic paths, in frame and in the origin-centred frame; in
     frame at box 64 and 100 it keeps the raw sign on both (fixed point: in-frame encoding; FP32: fl(1/box) box / 2
-    <= 1/2 there)."""
+    <= 1/2 there).  Fixed point at eps = max(0.05, fl(1e-4f * box)), FP32 one float below that bound."""
     n = N_F
     pos, mass, tgt = _planted_ties(n, box, int(box))
     partners = direct_np.tie_partners(pos, box, tgt)
     assert all(list(p) == [t + 1] for p, t in zip(partners, tgt))
+    paths = (("fixed", float(max(np.float32(0.05), _fixed_eps_bound(box))), "FIXED_R4"),
+             ("float", _float_eps(box), "FLOAT_R4"))
     for frame in ("in", "centred"):
         p = pos if frame == "in" else _centred(pos, box)
-        raw = direct_np.forces(p, mass, 0.05, box, targets=tgt, ties="raw")
-        flip = direct_np.forces(p, mass, 0.05, box, targets=tgt, ties="flip")
-        gap = np.linalg.norm(raw - flip, axis=1) / np.linalg.norm(raw, axis=1)
-        assert gap.min() > 100 * TIE_TOL
-        for path, env in (("fixed", FIXED_ENV), ("float", FLOAT_ENV)):
-            _with_env(monkeypatch, env)
-            a = _forces(engine, _posm(p, mass), 0, n, 0.05, box)[tgt].astype(np.float64)
-            e_raw = np.linalg.norm(a - raw, axis=1) / np.linalg.norm(raw, axis=1)
-            e_flip = np.linalg.norm(a - flip, axis=1) / np.linalg.norm(flip, axis=1)
+        for path, eps, instance in paths:
+            assert _force_instance(n, _tiles(n), eps, box) == instance
+            raw = direct_np.forces(p, mass, eps, box, targets=tgt, ties="raw")
+            flip = direct_np.forces(p, mass, eps, box, targets=tgt, ties="flip")
+            assert _row_err(flip, raw).min() > 100 * TIE_TOL
+            a = _forces(engine, _posm(p, mass), 0, n, eps, box)[tgt]
+            e_raw, e_flip = _row_err(a, raw), _row_err(a, flip)
             assert np.all(np.minimum(e_raw, e_flip) < TIE_TOL), (frame, path)
             if frame == "in" and box in (64.0, 100.0):
                 assert np.all(e_raw < TIE_TOL), (frame, path)
@@ -301,20 +309,21 @@ def test_half_box_ties_take_one_of_the_two_images(engine, oracle, monkeypatch, b
                   f"max error {np.minimum(e_raw, e_flip).max():.2e}")
 
 
-def test_frame_and_period_invariance_bitwise(engine, monkeypatch):
+def test_frame_and_period_invariance_bitwise(engine):
     """Tie-free dyadic input at box 64: FP32 separations and the fixed-point encoding (taken modulo 2^32) are exact,
-    so shifting any particle by whole periods, or writing the origin-centred frame, changes no bit."""
+    so shifting any particle by whole periods, or writing the origin-centred frame, changes no bit.  Fixed point at
+    eps 0.05, FP32 one float below fl(1e-4f * 64)."""
     box, n = 64.0, N_F
     pos = _tie_free_cloud(n, box, 7)
     mass = _mass(n, False, 8)
     k = np.random.default_rng(9).integers(-3, 4, (n, 3)).astype(np.float32)
     shifted = (pos + k * np.float32(box)).astype(np.float32)
     assert np.array_equal(shifted - k * np.float32(box), pos)
-    for env in (FIXED_ENV, FLOAT_ENV):
-        _with_env(monkeypatch, env)
-        a0 = _forces(engine, _posm(pos, mass), 0, n, 0.05, box)
+    for eps, instance in ((0.05, "FIXED_R4"), (_float_eps(box), "FLOAT_R4")):
+        assert _force_instance(n, _tiles(n), eps, box) == instance
+        a0 = _forces(engine, _posm(pos, mass), 0, n, eps, box)
         for q in (shifted, _centred(pos, box)):
-            assert np.array_equal(_forces(engine, _posm(q, mass), 0, n, 0.05, box), a0), env
+            assert np.array_equal(_forces(engine, _posm(q, mass), 0, n, eps, box), a0), instance
 
 
 # ---- 5. masses -------------------------------------------------------------------------------------------------------
@@ -343,8 +352,7 @@ def _mass_case(kind, n):
 @pytest.mark.parametrize("box", [0.0, 100.0], ids=["open_r8", "fixed_r4"])
 @pytest.mark.parametrize("kind", ["differs_first", "differs_last", "differs_in_last_tile", "negative_equal",
                                   "signed_zero_total", "ratio_1e4"])
-def test_masses_vs_float64(engine, oracle, monkeypatch, kind, box):
-    _with_env(monkeypatch, {})
+def test_masses_vs_float64(engine, oracle, kind, box):
     n, nt = N_MASS, 8192
     assert _force_instance(nt, _tiles(n), 0.05, box) == ("OPEN_R8" if box == 0 else "FIXED_R4")
     pos, m = _cloud(n, box, 11), _mass_case(kind, N_MASS)
@@ -358,9 +366,8 @@ def test_masses_vs_float64(engine, oracle, monkeypatch, kind, box):
 
 
 @pytest.mark.parametrize("box", [0.0, 100.0], ids=["open_r8", "fixed_r4"])
-def test_zero_masses_give_exact_zero(engine, monkeypatch, box):
+def test_zero_masses_give_exact_zero(engine, box):
     """All zero, and +0.0 mixed with -0.0 (equal under ==, so the equal-mass instance runs with m0 = +-0)."""
-    _with_env(monkeypatch, {})
     n = N_MASS
     pos = _cloud(n, box, 12)
     signs = np.where(np.random.default_rng(2).random(n) < 0.5, np.float32(0.0), np.float32(-0.0)).astype(np.float32)
@@ -371,8 +378,8 @@ def test_zero_masses_give_exact_zero(engine, monkeypatch, box):
 
 # ---- 6. coordinates --------------------------------------------------------------------------------------------------
 
-@pytest.mark.parametrize("env", [{}, FLOAT_ENV], ids=["fixed_r4", "float_r4"])
-def test_periodic_coordinate_edges(engine, oracle, monkeypatch, env):
+@pytest.mark.parametrize("instance", ["FIXED_R4", "FLOAT_R4"], ids=["fixed_r4", "float_r4_eps_below_bound"])
+def test_periodic_coordinate_edges(engine, oracle, instance):
     """Coincident pairs (r^2 = eps^2 on the fixed path), particles at 0, -0, box and the floats just below box, and
     particles several boxes out of frame.
 
@@ -380,9 +387,11 @@ def test_periodic_coordinate_edges(engine, oracle, monkeypatch, env):
     below box on every axis, 7.6e-6 and 1.5e-5 from it: pairs far closer than eps.  The FP32 path gets their
     separations exactly; the fixed-point path quantises each x and y to box / 2^32 (up to 2 units per separation
     with the upper-half shift), so there a pair's force m d / eps^3 may be off by m 2 box 2^-32 / eps^3 per
-    component: 1e-3 of these targets' forces, the documented price of that path (DESIGN 3.1), bounded here."""
-    _with_env(monkeypatch, env)
-    box, n, eps = 100.0, N_F, 0.05
+    component: 1e-3 of these targets' forces at eps 0.05, the documented price of that path (DESIGN 3.1), bounded
+    here.  The FP32 path runs one float below fl(1e-4f * box) and is held to the same bound."""
+    box, n = 100.0, N_F
+    eps = 0.05 if instance == "FIXED_R4" else _float_eps(box)
+    assert _force_instance(n, _tiles(n), eps, box) == instance
     pos = _cloud(n, box, 13)
     pos[10:20] = pos[0:10]
     below = np.nextafter(np.float32(box), np.float32(0))
@@ -398,15 +407,14 @@ def test_periodic_coordinate_edges(engine, oracle, monkeypatch, env):
     want = direct_np.forces(pos, m, eps, box, targets=idx)
     assert np.isfinite(a).all()
     close = np.isin(idx, np.arange(45, 50))
-    err = rel_l2(a[idx], want) if env else rel_l2(a[idx[~close]], want[~close])
+    err = rel_l2(a[idx], want) if instance == "FLOAT_R4" else rel_l2(a[idx[~close]], want[~close])
     near = np.abs(a[idx[close]] - want[close]).max()
-    bound = 4 * float(m.max()) * 2 * (box / 2 ** 32) / float(np.float32(eps)) ** 3      # 4 close partners each
-    print(f"coordinates {'float' if env else 'fixed'}: {err:.2e}, rows 45-49 off by {near:.2e} (bound {bound:.2e})")
+    bound = 4 * float(m.max()) * 2 * (box / 2 ** 32) / float(np.float32(0.05)) ** 3     # 4 close partners each
+    print(f"coordinates {instance}: {err:.2e}, rows 45-49 off by {near:.2e} (bound {bound:.2e})")
     assert err < TOL and near <= bound
 
 
-def test_open_offset_1e4(engine, oracle, monkeypatch):
-    _with_env(monkeypatch, {})
+def test_open_offset_1e4(engine, oracle):
     n = NS_HI
     pos = (_cloud(n, 0.0, 16) + np.float32(1e4)).astype(np.float32)
     m = _mass(n, False, 17)
@@ -420,18 +428,18 @@ def test_open_offset_1e4(engine, oracle, monkeypatch):
 @pytest.mark.parametrize("path", ["open", "float", "fixed"])
 @pytest.mark.parametrize("axis", [0, 1, 2], ids=["x", "y", "z"])
 @pytest.mark.parametrize("bad", [np.nan, np.inf, -np.inf], ids=["nan", "inf", "-inf"])
-def test_non_finite_coordinate_poisons(engine, monkeypatch, path, axis, bad):
+def test_non_finite_coordinate_poisons(engine, path, axis, bad):
     """One non-finite coordinate makes every force NaN (periodic: all three components; open: at least the
     component of the bad axis, where an infinite separation meets a zero 1/r^3), the particle's own row included.
     The fixed-point conversion of x and y saturates on +-inf: the guard must catch infinities as well as NaN."""
-    _with_env(monkeypatch, FLOAT_ENV if path == "float" else {})
     n, box = 32768, (0.0 if path == "open" else 100.0)
-    assert _force_instance(n, _tiles(n), 0.05, box, force_float=path == "float") == \
-        {"open": "OPEN_R8", "float": "FLOAT_R4", "fixed": "FIXED_R4"}[path]
+    eps = _float_eps(box) if path == "float" else 0.05
+    assert _force_instance(n, _tiles(n), eps, box) == {"open": "OPEN_R8", "float": "FLOAT_R4",
+                                                        "fixed": "FIXED_R4"}[path]
     pos = _cloud(n, 100.0, 18)
     k = n // 2
     pos[k, axis] = bad
-    a = _forces(engine, _posm(pos, np.ones(n, np.float32)), 0, n, 0.05, box)
+    a = _forces(engine, _posm(pos, np.ones(n, np.float32)), 0, n, eps, box)
     rows = np.isnan(a).any(1) if path == "open" else np.isnan(a).all(1)
     assert rows.sum() >= n - 1 and rows[k]
 
@@ -448,9 +456,8 @@ POT_CASES = [
 
 
 @pytest.mark.parametrize("case", POT_CASES, ids=[f"{c[0]}_{c[1]}_{'unit' if c[3] else 'general'}" for c in POT_CASES])
-def test_potential_instance_vs_float64(engine, monkeypatch, case):
+def test_potential_instance_vs_float64(engine, case):
     name, n, box, unit = case
-    _with_env(monkeypatch, {})
     pos, m = _cloud(n, box, n), _mass(n, unit, 19)
     posm = _posm(pos, m)
     phi = _potential(engine, posm, 0, n, 0.05, box)
@@ -492,14 +499,15 @@ def _part_tiles():
 
 
 @pytest.mark.parametrize("unit", [True, False], ids=["unit", "general"])
-@pytest.mark.parametrize("env", [{}, FLOAT_ENV], ids=["fixed_r4", "float_r4"])
-def test_parts_periodic(engine, oracle, monkeypatch, env, unit):
-    _with_env(monkeypatch, env)
+@pytest.mark.parametrize("instance", ["FIXED_R4", "FLOAT_R4"], ids=["fixed_r4", "float_r4"])
+def test_parts_periodic(engine, oracle, instance, unit):
     n, box = PART_CUTS[-1], 100.0
+    eps = 0.05 if instance == "FIXED_R4" else _float_eps(box)
+    assert _force_instance(n, _part_tiles(), eps, box) == instance
     pos, m = _cloud(n, box, 23), _mass(n, unit, 24)
     posm = _posm(pos, m)
     whole = torch.empty((n, 3), dtype=torch.float32, device="cuda")
-    engine.direct_forces_dev(posm, whole, 0, n, eps=0.05, box=box)
+    engine.direct_forces_dev(posm, whole, 0, n, eps=eps, box=box)
     parts, lens = [], []
     for a, b in zip(PART_CUTS[:-1], PART_CUTS[1:]):
         t = torch.empty(max(engine.tiles_bytes(b - a), 16) // 4, dtype=torch.float32, device="cuda")
@@ -508,14 +516,14 @@ def test_parts_periodic(engine, oracle, monkeypatch, env, unit):
         parts.append(t)
         lens.append(b - a)
     idx = _sample(0, n, 512)
-    want = direct_np.forces(pos, m, 0.05, box, targets=idx)
+    want = direct_np.forces(pos, m, eps, box, targets=idx)
     for equal_flag in ([True, False] if unit else [False]):
         out = torch.empty((n, 3), dtype=torch.float32, device="cuda")
-        engine.direct_forces_parts_dev(parts, lens, posm, n, out, eps=0.05, box=box, all_masses_equal=equal_flag)
+        engine.direct_forces_parts_dev(parts, lens, posm, n, out, eps=eps, box=box, all_masses_equal=equal_flag)
         torch.cuda.synchronize()
         o, w = out.cpu().numpy(), whole.cpu().numpy()
         e_whole, e_64 = rel_l2(o, w), rel_l2(o[idx], want)
-        print(f"parts {env or 'fixed'} {'unit' if unit else 'general'} flag={equal_flag}: {e_whole:.2e} {e_64:.2e}")
+        print(f"parts {instance} {'unit' if unit else 'general'} flag={equal_flag}: {e_whole:.2e} {e_64:.2e}")
         assert e_whole < 2e-6 and e_64 < TOL
 
 
@@ -532,7 +540,7 @@ def test_every_instance_is_reached():
         forces.add((_force_instance(8192, _tiles(N_MASS), 0.05, box), False))
     for unit in (True, False):                              # parts
         forces.add((_force_instance(N_F + 777, _part_tiles(), 0.05, 100.0), unit))
-        forces.add((_force_instance(N_F + 777, _part_tiles(), 0.05, 100.0, force_float=True), unit))
+        forces.add((_force_instance(N_F + 777, _part_tiles(), _float_eps(100.0), 100.0), unit))
     want = {(f, u) for f in ("OPEN_R2", "OPEN_R8", "FLOAT_R2", "FLOAT_R4", "FIXED_R4") for u in (True, False)}
     assert want <= forces, sorted(want - forces)
     pots = {(_potential_instance(n, _tiles(n), box), unit) for _, n, box, unit in POT_CASES}
