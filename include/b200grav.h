@@ -162,7 +162,8 @@ int b200_power_spectrum_dev(b200_ctx* ctx, const void* posm4, size_t n, int grid
  * filter the W^-2 deconvolution makes the pair force noisy (100-200 % r.m.s. at 2-8 cells).  Recommended:
  * r_split = 1.25 h.  The PM force plus the short-range remainder sum m d / r^3 [erfc(r / 2 r_s) + r / (r_s sqrt(pi))
  * exp(-r^2 / 4 r_s^2)] (minimum image) then matches an Ewald sum to 0.02 / 0.2 / 0.8 / 1.0 / 0.6 / 0.3 % r.m.s. at
- * r = 0.5 / 1 / 2 / 4 / 8 / 12 h; used alone, the PM force is smooth below a few cells, the mesh's resolution.
+ * r = 0.5 / 1 / 2 / 4 / 8 / 12 h (b200_tree_walk_short_dev adds that remainder, cut off, from the fixed-physics
+ * tree); used alone, the PM force is smooth below a few cells, the mesh's resolution.
  * The mass deposit accumulates in int64 fixed point: the meshes, and so the result for a target, are bitwise the
  * same whatever the storage order of the sources and whichever target range is asked for.  Sharded use: every rank
  * passes the full all-gathered array (b200_allgather_sources_dev) and its own target range (b200_shard_range); the
@@ -239,6 +240,24 @@ int b200_tree_build_fixed_dev(b200_ctx* ctx, const void* posm4, size_t n, int le
  * sum as theta -> 0; no Ewald sum.  0 = open
  * boundary (default).  The reference-faithful tree is never periodic (the CPU TreeForceComputer is not). */
 int b200_tree_set_periodic(b200_ctx* ctx, float box);
+/* TreePM short range: adds to acc3 (float[3*n_targets], device) the short-range periodic acceleration of the
+ * targets posm4[i0 .. i0+n_targets) from every particle of the last b200_tree_build_fixed_dev tree, in a periodic
+ * box of edge `box` (any frame: only separations are used).  With the long range of b200_pm_forces_dev(..., grid, box, r_split, ...) written into acc3 first,
+ * acc3 holds the TreePM force.  G = 1.  For target i and source j, d = minimum image of x_j - x_i, r = |d|:
+ *   a_i += m_j g(r) d / (r^2 + eps^2)^(3/2)  for r < r_cut only,
+ *   g(r) = erfc(r / 2 r_s) + r / (r_s sqrt(pi)) exp(-r^2 / 4 r_s^2)   (unsoftened r; the self pair adds 0).
+ * The tree approximates it with the fixed walk's opening test (size / |d_c| < theta, d_c the minimum image of the
+ * centre of mass; a cell that reaches across the half-box distance is never a monopole).  A cell with
+ * |d_c| - sqrt(3) size >= r_cut holds no source within r_cut and is skipped; an accepted cell adds
+ * M g(|d_c|) d_c / (|d_c|^2 + eps^2)^(3/2).  theta = 0 gives the exact truncated sum.  GADGET-2 cuts at
+ * r_cut = 4.5 r_s, where truncation changes the force by 1e-4 to 1e-3 of its norm.  Reads and changes no
+ * b200_tree_set_periodic state.  With counting on (b200_tree_set_counting), counters[2] counts the source pairs
+ * inside r_cut, and stats[3] every leaf pair evaluated.  A tree that overflowed fills acc3 with NaN.
+ * B200_ERR_STATE without a fixed-physics tree (the reference-faithful tree included); B200_ERR_INVALID unless
+ * box > 0, r_split > 0 and 0 < r_cut < box / 2 (beyond, a second image could be within reach), and for a NULL
+ * acc3 or i0 + n_targets > n; n_targets = 0 is a no-op. */
+int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
+                             float r_cut, void* acc3, void* stream);
 /* Energy diagnostic from the fixed-physics tree (after b200_tree_build_fixed_dev): the walk accumulating
  * phi_i = sum m / sqrt(|d|^2 + eps^2) -- M / r for an accepted cell -- so that compute_energy
  * (src/physics/lambda_cdm_kernels.cu:338-408) costs O(N log N) in a tree run instead of O(N^2).

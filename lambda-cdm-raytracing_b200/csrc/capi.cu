@@ -508,6 +508,13 @@ int b200_tree_energy_dev(b200_ctx* ctx, size_t i0, size_t n_targets, const void*
     return B200_OK;
 }
 
+int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
+                             float r_cut, void* acc3, void* stream) {
+    if (!ctx) return B200_ERR_INVALID;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return tree_walk_short(ctx, i0, n_targets, theta, box, r_split, r_cut, acc3, pick_stream(ctx, stream));
+}
+
 int b200_tree_set_periodic(b200_ctx* ctx, float box) {
     if (!ctx) return B200_ERR_INVALID;
     return tree_set_periodic(ctx, box);

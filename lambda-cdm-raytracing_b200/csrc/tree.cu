@@ -36,6 +36,7 @@
 #include "shard.cuh"
 #include "sort.cuh"
 #include "tree.cuh"
+#include "treepm.cuh"
 
 namespace b200 {
 
@@ -1109,6 +1110,12 @@ __device__ __forceinline__ bool accept_cell_d(float size, float dx, float dy, fl
     return __fdiv_rn(size, __fsqrt_rn(d2)) < theta;
 }
 
+__device__ __forceinline__ float sqrt_fast(float x) {    // one MUFU.SQRT; 0 at 0
+    float r;
+    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
+
 __device__ __forceinline__ unsigned long long w_pk(float lo, float hi) {
     unsigned long long r;
     asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
@@ -1175,12 +1182,23 @@ __device__ __forceinline__ unsigned ends_first(unsigned cta, unsigned n_ctas) {
 // known (after the vote) measured no gain, and speculative requests (the skip target, or id + 1, before the vote)
 // cost time -- every broadcast 256-bit load writes 1 KB into the register file, and in this kernel that return path
 // (l1tex lsu writeback, 128 B per clock and SM) is 76 % busy, as busy as the issue slots: a wrong guess is not free.
-template <bool COUNT, bool PERIODIC, bool POT>
-__global__ void __launch_bounds__(128, 9)
+// SHORT (with PERIODIC, without POT): the short-range half of TreePM (b200_tree_walk_short_dev).  Every pair and
+// accepted cell is weighted by g(r) = erfc(r / 2 r_s) + r / (r_s sqrt(pi)) exp(-r^2 / 4 r_s^2) of its unsoftened
+// minimum-image distance (inv2rs = 1 / (2 r_s)); pairs at r >= r_cut weigh 0 (r^2 >= rcut2).  A cell whose centre
+// of mass is at least r_cut + sqrt(3) edge away is cut: accepted with weight 0, its subtree skipped -- every
+// particle of the cell lies within sqrt(3) edge of its centre of mass, and the torus distance obeys the triangle
+// inequality, so no particle of a cut cell is within r_cut of the target, whether or not the cell straddles the
+// half-box distance.  The result is added to acc3.  COUNT: the pair interactions (counter 2) are the pairs inside
+// r_cut; the pair-row slots (counter 3) still count every leaf pair issued.  The walk fits the 56 registers of 9
+// resident CTAs per SM without spilling; its counting instance spills there and gets 8 (64 registers).
+template <bool COUNT, bool PERIODIC, bool POT, bool SHORT = false>
+__global__ void __launch_bounds__(128, SHORT && COUNT ? 8 : 9)
 walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order, int i0, int n_targets,
                  const float4* __restrict__ nodes,
                  const ulonglong2* __restrict__ leaf_pairs, float theta, float theta2, float eps2, float box,
-                 float* __restrict__ acc3, TreeGlobals* __restrict__ g, int by_slot) {
+                 float* __restrict__ acc3, TreeGlobals* __restrict__ g, int by_slot, float inv2rs, float rcut,
+                 float rcut2) {
+    static_assert(!SHORT || (PERIODIC && !POT), "the short-range walk is periodic and has no potential");
     typedef unsigned long long u64;
     const int t = ends_first(blockIdx.x, gridDim.x) * blockDim.x + threadIdx.x;
     const bool valid = t < n_targets;
@@ -1223,6 +1241,23 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                 dy = w_fma2(w_add2(w_fma2(dy, inv_box2, magic2), nmagic2), nbox2, dy);
                 dz = w_fma2(w_add2(w_fma2(dz, inv_box2, magic2), nmagic2), nbox2, dz);
             }
+            if constexpr (SHORT) {
+                // g of the unsoftened distance, 0 at r >= r_cut; an out lane still has rinv = 0 (eps^2 = +inf)
+                u64 d2 = w_mul2(dx, dx);
+                d2 = w_fma2(dy, dy, d2);
+                d2 = w_fma2(dz, dz, d2);
+                float d2a, d2b, r2a, r2b;
+                w_unpk(d2, d2a, d2b);
+                w_unpk(w_add2(d2, e2_2), r2a, r2b);
+                const bool ina = d2a < rcut2, inb = d2b < rcut2;
+                const float ga = ina ? treepm_short_g(sqrt_fast(d2a) * inv2rs) : 0.0f;
+                const float gb = inb ? treepm_short_g(sqrt_fast(d2b) * inv2rs) : 0.0f;
+                const u64 rinv = w_pk(rsqrt_fast(r2a), rsqrt_fast(r2b));
+                if (COUNT) { c_slots += 2; if (on_lane) c_pp += (unsigned)ina + (unsigned)inb; }
+                const u64 f = w_mul2(w_mul2(w_mul2(rinv, rinv), rinv), w_mul2(b.y, w_pk(ga, gb)));
+                ax2 = w_fma2(f, dx, ax2); ay2 = w_fma2(f, dy, ay2); az2 = w_fma2(f, dz, az2);
+                return;
+            }
             u64 r2 = w_fma2(dx, dx, e2_2);
             r2 = w_fma2(dy, dy, r2);
             r2 = w_fma2(dz, dz, r2);
@@ -1237,7 +1272,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             const u64 f = w_mul2(w_mul2(w_mul2(rinv, rinv), rinv), b.y);  // m / r^3
             ax2 = w_fma2(f, dx, ax2); ay2 = w_fma2(f, dy, ay2); az2 = w_fma2(f, dz, az2);
         };
-        if (COUNT && on_lane) c_pp += cnt;
+        if (COUNT && !SHORT && on_lane) c_pp += cnt;
         const ulonglong2* src = pairs + 2 * (size_t)q;
         const int np = (cnt + 1) >> 1;
         int k2 = 0;
@@ -1298,7 +1333,21 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                     sure = true; accept = false;
                 }
             }
+            [[maybe_unused]] bool cut = false;
+            if constexpr (SHORT) {       // no particle of the cell within r_cut: accepted with weight 0
+                const float reach = fmaf(1.7320509f, mf.z, rcut);           // sqrt(3) rounded up
+                cut = d2 >= reach * reach;
+                if (cut) { sure = true; accept = true; }
+            }
             auto monopole = [&](bool take) {                                 // :280-290; 1/r = 0 for a lane that is out
+                if constexpr (SHORT) {
+                    const float rinv = (take && !cut) ? rsqrt_fast(d2 + eps2) : 0.0f;
+                    const float f = c.w * treepm_short_g(sqrt_fast(d2) * inv2rs) * rinv * rinv * rinv;
+                    ax = fmaf(f, dx, ax); ay = fmaf(f, dy, ay); az = fmaf(f, dz, az);
+                    if (COUNT) c_pc += take && !cut;
+                    if (take) wake = skip;
+                    return;
+                }
                 const float rinv = take ? rsqrt_fast(d2 + eps2) : 0.0f;
                 if constexpr (POT) {
                     ax = fmaf(c.w, rinv, ax);
@@ -1354,6 +1403,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             w_unpk(ay2, lo, hi); ay += lo + hi;
             w_unpk(az2, lo, hi); az += lo + hi;
             const size_t o = (size_t)(by_slot ? t : i - i0) * 3;
+            if constexpr (SHORT) { ax += acc3[o + 0]; ay += acc3[o + 1]; az += acc3[o + 2]; }
             acc3[o + 0] = ax; acc3[o + 1] = ay; acc3[o + 2] = az;
         }
     }
@@ -1998,7 +2048,7 @@ static void launch_fixed_walk(const TreeState* T, const int* order, size_t i0, s
     auto kernel = T->periodic_box > 0.f ? walk_warp_kernel<COUNT, true, POT> : walk_warp_kernel<COUNT, false, POT>;
     kernel<<<grid, 128, 0, st>>>(T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(),
                                  T->leaf_pos.as<ulonglong2>(), theta, theta2, T->eps * T->eps, T->periodic_box, out,
-                                 T->globals.as<TreeGlobals>(), by_slot);
+                                 T->globals.as<TreeGlobals>(), by_slot, 0.f, 0.f, 0.f);
 }
 
 // The faithful tree's walk (two targets per lane), of this context's tree or (FOREST) of the published forest.
@@ -2067,6 +2117,34 @@ int tree_walk(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, void* acc
 int tree_walk_list(b200_ctx* ctx, const int* list, size_t n_list, float theta, void* acc3, cudaStream_t st) {
     if (n_list && !list) return B200_ERR_INVALID;
     return tree_walk_impl(ctx, list, 0, n_list, theta, acc3, st);
+}
+
+// The short-range TreePM walk (walk_warp_kernel, SHORT) of the targets [i0, i0 + n_targets) of the fixed-physics
+// tree, in the periodic box `box` whatever tree_set_periodic holds: added to acc3.
+int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split, float r_cut,
+                    void* acc3, cudaStream_t st) {
+    TreeState* T = ctx->tree;
+    if (!T || !T->built || !T->fixed) return B200_ERR_STATE;
+    // r_cut < box / 2: the minimum image is the only image of a source within reach
+    if (!(box > 0.f) || !(r_split > 0.f) || !(r_cut > 0.f) || !(r_cut < 0.5f * box)) return B200_ERR_INVALID;
+    if (n_targets == 0) return B200_OK;
+    if (!acc3 || i0 + n_targets > T->n) return B200_ERR_INVALID;
+    B200_TRY(tree_target_order(ctx, T, i0, n_targets, st));
+    if (T->counting) {
+        zero_counters_kernel<<<1, 1, 0, st>>>(T->globals.as<TreeGlobals>());
+        ctx->launches += 1;
+    }
+    if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev0, st));
+    const unsigned grid = (unsigned)((n_targets + 127) / 128);
+    const float theta2 = theta > 0.f ? theta * theta : 0.f;
+    auto kernel = T->counting ? walk_warp_kernel<true, true, false, true> : walk_warp_kernel<false, true, false, true>;
+    kernel<<<grid, 128, 0, st>>>(T->posm, T->order.as<int>(), (int)i0, (int)n_targets, T->nodes.as<float4>(),
+                                 T->leaf_pos.as<ulonglong2>(), theta, theta2, T->eps * T->eps, box, (float*)acc3,
+                                 T->globals.as<TreeGlobals>(), 0, 0.5f / r_split, r_cut, r_cut * r_cut);
+    if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev1, st));
+    B200_CUDA(cudaGetLastError());
+    ctx->launches += 1;
+    return B200_OK;
 }
 
 // ---- forest of part builds -------------------------------------------------------------------

@@ -13,6 +13,9 @@ int tree_forest_root(b200_ctx* ctx, float out[8]);
 // targets given as an explicit list of particle slots; acc3 in list order.  Like tree_walk, it walks the
 // published forest when the context holds a part build
 int tree_walk_list(b200_ctx* ctx, const int* list, size_t n_list, float theta, void* acc3, cudaStream_t st);
+// short-range TreePM walk of the fixed-physics tree in a periodic box, added to acc3
+int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split, float r_cut,
+                    void* acc3, cudaStream_t st);
 int tree_set_counting(b200_ctx* ctx, int enabled);
 int tree_set_periodic(b200_ctx* ctx, float box);
 int tree_potential(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, void* phi, cudaStream_t st);

@@ -28,7 +28,7 @@ EXPORTS = [
     "b200_device_alloc", "b200_device_free", "b200_memcpy_h2d", "b200_memcpy_d2h", "b200_unpack_pos3_dev", "b200_ipc_export", "b200_ipc_open", "b200_ipc_close",
     "b200_shard_range", "b200_shard_unique_id", "b200_shard_init", "b200_shard_finalize", "b200_shard_info",
     "b200_allgather_sources_dev", "b200_allreduce_sum_f64", "b200_direct_potential_dev", "b200_energy_dev",
-    "b200_ic_params_default", "b200_zeldovich_ics_dev", "b200_force_error_dev", "b200_power_spectrum_dev", "b200_tree_build_fixed_dev", "b200_tree_forces_fixed_host", "b200_tree_set_periodic", "b200_spatial_order_dev", "b200_tree_build_host", "b200_tree_walk_host", "b200_tree_potential_dev", "b200_tree_energy_dev",
+    "b200_ic_params_default", "b200_zeldovich_ics_dev", "b200_force_error_dev", "b200_power_spectrum_dev", "b200_tree_build_fixed_dev", "b200_tree_forces_fixed_host", "b200_tree_set_periodic", "b200_tree_walk_short_dev", "b200_spatial_order_dev", "b200_tree_build_host", "b200_tree_walk_host", "b200_tree_potential_dev", "b200_tree_energy_dev",
     "b200_fp32_peak_probe", "b200_last_kernel_ms", "b200_set_timing", "b200_launch_count",
     "b200_pm_forces_dev", "b200_pm_forces_host", "b200_pm_phase_ms",
 ]
@@ -75,6 +75,7 @@ def load_library(path=None):
     L.b200_tree_build_fixed_dev.argtypes = [vp, vp, sz, i32, i32, f32, vp]
     L.b200_tree_forces_fixed_host.argtypes = [vp, vp, vp, vp, sz, f32, i32, i32, f32]
     L.b200_tree_set_periodic.argtypes = [vp, f32]
+    L.b200_tree_walk_short_dev.argtypes = [vp, sz, sz, f32, f32, f32, f32, vp, vp]
     L.b200_spatial_order_dev.argtypes = [vp, vp, sz, f32, vp, vp]
     L.b200_tree_build_host.argtypes = [vp, vp, vp, sz, f32, i32, i32]
     L.b200_tree_walk_host.argtypes = [vp, vp, sz, f32]
@@ -269,6 +270,23 @@ class Engine:
     def tree_walk_dev(self, acc, i0, n_targets, theta=0.5, stream=None):
         self._check(self.L.b200_tree_walk_dev(self._h, i0, n_targets, theta, _ptr(acc), _stream(stream)))
         return acc
+
+    def tree_walk_short_dev(self, acc, i0, n_targets, theta, box, r_split, r_cut, stream=None):
+        """Adds the TreePM short-range acceleration (cut off at r_cut) of targets [i0, i0+n_targets) of the last
+        fixed-physics tree to acc (device float[n_targets, 3])."""
+        self._check(self.L.b200_tree_walk_short_dev(self._h, i0, n_targets, theta, box, r_split, r_cut, _ptr(acc),
+                                                    _stream(stream)))
+        return acc
+
+    def treepm_forces_dev(self, posm, acc, i0, n_targets, grid, box, r_split=None, r_cut_factor=4.5, theta=0.5,
+                          leaf_cap=8, max_depth=20, eps=0.01, stream=None):
+        """Periodic TreePM acceleration of targets posm[i0 : i0+n_targets) from all of posm (device): a
+        fixed-physics tree of every source, the PM long range (written into acc), then the short-range walk
+        cut off at r_cut_factor * r_split (added).  r_split=None: 1.25 box / grid."""
+        rs = 1.25 * box / grid if r_split is None else r_split
+        self.tree_build_fixed_dev(posm, posm.shape[0], leaf_cap, max_depth, eps, stream)
+        self.pm_forces_dev(posm, acc, i0, n_targets, grid, box, rs, stream=stream)
+        return self.tree_walk_short_dev(acc, i0, n_targets, theta, box, rs, r_cut_factor * rs, stream)
 
     def tree_forces_host(self, pos, mass, theta=0.5, leaf_cap=8, max_depth=20, box=100.0, out=None):
         pos = np.ascontiguousarray(pos, np.float32)
@@ -520,8 +538,9 @@ class LambdaCDMSimulation:
     physics::LambdaCDMSimulation (include/physics/lambda_cdm.hpp:22-75;
     step order src/physics/lambda_cdm_impl.cu:167-213), driving the C ABI.
 
-    force: "direct", "tree" or "pm" (periodic particle mesh on a pm_grid^3 mesh, Gaussian split radius r_split,
-    None = 1.25 box / pm_grid).  The first half-kick of the first step uses the
+    force: "direct", "tree", "pm" (periodic particle mesh on a pm_grid^3 mesh, Gaussian split radius r_split,
+    None = 1.25 box / pm_grid) or "treepm" (that PM long range plus the short-range walk of the fixed-physics
+    tree at theta, softening eps, cut off at 4.5 r_split).  The first half-kick of the first step uses the
     forces at the initial positions (the reference reads uninitialised memory
     there; SURVEY 8c)."""
 
@@ -555,6 +574,9 @@ class LambdaCDMSimulation:
             self.e.direct_forces_dev(self.posm, self.acc, self.i0, self.nl, self.eps, 0.0)
         elif self.force == "pm":
             self.e.pm_forces_dev(self.posm, self.acc, self.i0, self.nl, self.pm_grid, self.box, self.r_split)
+        elif self.force == "treepm":
+            self.e.treepm_forces_dev(self.posm, self.acc, self.i0, self.nl, self.pm_grid, self.box, self.r_split,
+                                     theta=self.theta, leaf_cap=self.leaf_cap, max_depth=self.max_depth, eps=self.eps)
         else:
             self.e.tree_build_dev(self.posm, self.n, self.box, self.leaf_cap, self.max_depth)
             self.e.tree_walk_dev(self.acc, self.i0, self.nl, self.theta)
