@@ -10,6 +10,7 @@
 // is HBM-bound: 20 B per element per pass, coalesced 128-bit loads, tiles of
 // 4096 keys so a 16 M sort is 4096 CTAs (~28 per SM).
 #include "common.cuh"
+#include "scan.cuh"
 #include "sort.cuh"
 
 namespace b200 {
@@ -113,41 +114,8 @@ rs_hist_kernel(const uint32_t* __restrict__ keys, long long n, int shift, int n_
 // and the digit total.
 __global__ void __launch_bounds__(1024)
 rs_scan_kernel(uint32_t* __restrict__ hist, int n_tiles, uint32_t* __restrict__ totals) {
-    __shared__ uint32_t warp_sums[32];
-    __shared__ uint32_t carry_s, chunk_total;
-    uint32_t* row = hist + (size_t)blockIdx.x * n_tiles;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    for (int base = 0; base < n_tiles; base += 1024) {
-        const int i = base + threadIdx.x;
-        const uint32_t v = (i < n_tiles) ? row[i] : 0u;
-        uint32_t x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) warp_sums[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            const uint32_t w = warp_sums[lane];
-            uint32_t xs = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                uint32_t y = __shfl_up_sync(0xffffffffu, xs, o);
-                if (lane >= o) xs += y;
-            }
-            warp_sums[lane] = xs - w;       // exclusive prefix of the warp sums
-            if (lane == 31) chunk_total = xs;
-        }
-        __syncthreads();
-        if (i < n_tiles) row[i] = carry_s + warp_sums[warp] + (x - v);
-        __syncthreads();
-        if (threadIdx.x == 0) carry_s += chunk_total;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) totals[blockIdx.x] = carry_s;
+    const uint32_t total = cta_exclusive_scan<1>(hist + (size_t)blockIdx.x * n_tiles, n_tiles, 1);
+    if (threadIdx.x == 0) totals[blockIdx.x] = total;
 }
 
 __global__ void __launch_bounds__(RS_THREADS)
@@ -164,19 +132,8 @@ rs_scatter_kernel(const uint32_t* __restrict__ keys_in, const int32_t* __restric
 
     for (int k = threadIdx.x; k < RS_WARPS * RADIX; k += RS_THREADS) (&warp_cnt[0][0])[k] = 0;
     // global base of each digit = exclusive scan of totals (256 values, one per thread)
-    {
-        uint32_t v = totals[threadIdx.x], x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        uint32_t wbase = 0;
-        for (int w = 0; w < warp; ++w) wbase += wsum[w];
-        digit_base[threadIdx.x] = wbase + x - v + hist[(size_t)threadIdx.x * n_tiles + tile];
-    }
+    digit_base[threadIdx.x] =
+        block_exclusive_prefix(hist[(size_t)threadIdx.x * n_tiles + tile], totals[threadIdx.x], wsum);
     __syncthreads();
 
     uint32_t key[RS_ITEMS];

@@ -33,6 +33,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "scan.cuh"
 #include "shard.cuh"
 #include "sort.cuh"
 #include "tree.cuh"
@@ -257,18 +258,6 @@ __device__ __forceinline__ u64 node_value(int count, int cap, bool may_split, in
     return split ? ((1ull << 40) | (u64)keep) : (u64)count;
 }
 
-__device__ __forceinline__ u64 block_reduce_u64(u64 v, u64* sh /* >= 8 */) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(FULL, v, o);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __syncthreads();
-    if (lane == 0) sh[warp] = v;
-    __syncthreads();
-    u64 t = 0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += sh[w];
-    return t;
-}
-
 __global__ void __launch_bounds__(256)
 node_reduce_kernel(const TreeGlobals* __restrict__ g, int level, int cap, int keep, int max_depth,
                    const int* __restrict__ ncount, u64* __restrict__ tile_sum) {
@@ -284,7 +273,7 @@ node_reduce_kernel(const TreeGlobals* __restrict__ g, int level, int cap, int ke
             int k = tile * NODE_TILE + threadIdx.x * 8 + j;
             if (k < n_nodes) v += node_value(ncount[L.node_begin + k], cap, may_split, keep);
         }
-        u64 t = block_reduce_u64(v, sh);
+        const u64 t = block_sum<8>(v, sh);
         if (threadIdx.x == 0) tile_sum[tile] = t;
     }
 }
@@ -292,44 +281,10 @@ node_reduce_kernel(const TreeGlobals* __restrict__ g, int level, int cap, int ke
 // single CTA: exclusive scan of the tile sums; publishes the extents of the next level
 __global__ void __launch_bounds__(1024)
 node_scan_kernel(TreeGlobals* __restrict__ g, int level, u64* __restrict__ tile_sum, int max_nodes) {
-    __shared__ u64 wsum[32];
-    __shared__ u64 carry_s, chunk_s;
     const LevelInfo L = g->lv[level];
     const int n_nodes = L.node_end - L.node_begin;
-    const int n_tiles = (n_nodes + NODE_TILE - 1) / NODE_TILE;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    for (int base = 0; base < n_tiles; base += 1024) {
-        const int i = base + threadIdx.x;
-        const u64 v = (i < n_tiles) ? tile_sum[i] : 0ull;
-        u64 x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u64 y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            const u64 w = wsum[lane];
-            u64 xs = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                u64 y = __shfl_up_sync(FULL, xs, o);
-                if (lane >= o) xs += y;
-            }
-            wsum[lane] = xs - w;
-            if (lane == 31) chunk_s = xs;
-        }
-        __syncthreads();
-        if (i < n_tiles) tile_sum[i] = carry_s + wsum[warp] + (x - v);
-        __syncthreads();
-        if (threadIdx.x == 0) carry_s += chunk_s;
-        __syncthreads();
-    }
+    const u64 tot = cta_exclusive_scan<1>(tile_sum, (n_nodes + NODE_TILE - 1) / NODE_TILE, 1);
     if (threadIdx.x == 0) {
-        const u64 tot = carry_s;
         const int n_split = (int)(tot >> 40);
         const int stored = (int)(tot & ((1ull << 40) - 1));
         g->lv[level].n_split = n_split;
@@ -354,7 +309,6 @@ node_apply_kernel(const TreeGlobals* __restrict__ g, int level, int cap, int kee
     const int n_nodes = L.node_end - L.node_begin;
     const int n_tiles = (n_nodes + NODE_TILE - 1) / NODE_TILE;
     const bool may_split = level < max_depth;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         u64 v[8], tsum = 0;
 #pragma unroll
@@ -363,17 +317,7 @@ node_apply_kernel(const TreeGlobals* __restrict__ g, int level, int cap, int kee
             v[j] = (k < n_nodes) ? node_value(ncount[L.node_begin + k], cap, may_split, keep) : 0ull;
             tsum += v[j];
         }
-        u64 x = tsum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u64 y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        __syncthreads();
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        u64 pre = tile_sum[tile] + (x - tsum);
-        for (int w = 0; w < warp; ++w) pre += wsum[w];
+        u64 pre = block_exclusive_prefix(tile_sum[tile], tsum, wsum);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             int k = tile * NODE_TILE + threadIdx.x * 8 + j;
@@ -499,56 +443,12 @@ entry_digit_kernel(const TreeGlobals* __restrict__ g, int level, int keep, unsig
 // entry count is the sum of the 8 channel totals (reset by node_scan_kernel, added here).
 __global__ void __launch_bounds__(1024)
 tile_scan_kernel(TreeGlobals* __restrict__ g, int level, unsigned* __restrict__ tile_hist) {
-    __shared__ unsigned wsum[32];
-    __shared__ unsigned carry_s, chunk_s;
-    constexpr int PER = 8;
-    const LevelInfo L = g->lv[level];
-    const int n_tiles = (L.n_entries + ENT_TILE - 1) / ENT_TILE;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, d = blockIdx.x;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    for (int base = 0; base < n_tiles; base += 1024 * PER) {
-        unsigned v[PER], sum = 0;
-#pragma unroll
-        for (int j = 0; j < PER; ++j) {
-            const int t = base + threadIdx.x * PER + j;
-            v[j] = (t < n_tiles) ? tile_hist[(size_t)t * 8 + d] : 0u;
-            sum += v[j];
-        }
-        unsigned x = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            const unsigned w = wsum[lane];
-            unsigned xs = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned y = __shfl_up_sync(FULL, xs, o);
-                if (lane >= o) xs += y;
-            }
-            wsum[lane] = xs - w;
-            if (lane == 31) chunk_s = xs;
-        }
-        __syncthreads();
-        unsigned pre = carry_s + wsum[warp] + (x - sum);
-#pragma unroll
-        for (int j = 0; j < PER; ++j) {
-            const int t = base + threadIdx.x * PER + j;
-            if (t < n_tiles) tile_hist[(size_t)t * 8 + d] = pre;
-            pre += v[j];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) carry_s += chunk_s;
-        __syncthreads();
-    }
+    const int n_tiles = (g->lv[level].n_entries + ENT_TILE - 1) / ENT_TILE;
+    const int d = blockIdx.x;
+    const unsigned total = cta_exclusive_scan<8>(tile_hist + d, n_tiles, 8);
     if (threadIdx.x == 0) {
-        g->totals[d] = carry_s;
-        atomicAdd(&g->lv[level + 1].n_entries, (int)carry_s);
+        g->totals[d] = total;
+        atomicAdd(&g->lv[level + 1].n_entries, (int)total);
     }
 }
 
@@ -891,56 +791,15 @@ leaf_reduce_kernel(const TreeGlobals* __restrict__ g, int max_depth, const int4*
             const int k = tile * NODE_TILE + j * 256 + threadIdx.x;
             if (k < nn) v += scan_value<MODE>(k, meta, lscan);
         }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(FULL, v, o);
-        __syncthreads();
-        if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int t = 0;
-            for (int w = 0; w < 8; ++w) t += sh[w];
-            tile_sum[tile] = t;
-        }
+        const int t = block_sum<8>(v, sh);
+        if (threadIdx.x == 0) tile_sum[tile] = t;
     }
 }
 template <int MODE>
 __global__ void __launch_bounds__(1024)
 leaf_scan_kernel(const TreeGlobals* __restrict__ g, int max_depth, int* __restrict__ tile_sum) {
-    __shared__ int wsum[32];
-    __shared__ int carry_s, chunk_s;
     const int nn = scan_items<MODE>(tree_node_count(g, max_depth));
-    const int n_tiles = (nn + NODE_TILE - 1) / NODE_TILE;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    for (int base = 0; base < n_tiles; base += 1024) {
-        const int i = base + threadIdx.x;
-        const int v = (i < n_tiles) ? tile_sum[i] : 0;
-        int x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            const int w = wsum[lane];
-            int xs = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int y = __shfl_up_sync(FULL, xs, o);
-                if (lane >= o) xs += y;
-            }
-            wsum[lane] = xs - w;
-            if (lane == 31) chunk_s = xs;
-        }
-        __syncthreads();
-        if (i < n_tiles) tile_sum[i] = carry_s + wsum[warp] + (x - v);
-        __syncthreads();
-        if (threadIdx.x == 0) carry_s += chunk_s;
-        __syncthreads();
-    }
+    cta_exclusive_scan<1>(tile_sum, (nn + NODE_TILE - 1) / NODE_TILE, 1);
 }
 // out[k] = sum of the values of items < k (k = 0..items); one tile of 2048 items per CTA pass,
 // thread t owns items [8t, 8t+8) of the tile so the in-tile scan is a thread-serial + warp + CTA scan
@@ -952,7 +811,6 @@ leaf_apply_kernel(const TreeGlobals* __restrict__ g, int max_depth, const int4* 
     const int nn = scan_items<MODE>(tree_node_count(g, max_depth));
     if (nn == 0 && blockIdx.x == 0 && threadIdx.x == 0) lscan[0] = 0;
     const int n_tiles = (nn + NODE_TILE - 1) / NODE_TILE;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         int v[8], tsum = 0;
 #pragma unroll
@@ -961,17 +819,7 @@ leaf_apply_kernel(const TreeGlobals* __restrict__ g, int max_depth, const int4* 
             v[j] = (k < nn) ? scan_value<MODE>(k, meta, lscan_in) : 0;
             tsum += v[j];
         }
-        int x = tsum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int y = __shfl_up_sync(FULL, x, o);
-            if (lane >= o) x += y;
-        }
-        __syncthreads();
-        if (lane == 31) wsum[warp] = x;
-        __syncthreads();
-        int pre = tile_sum[tile] + (x - tsum);
-        for (int w = 0; w < warp; ++w) pre += wsum[w];
+        int pre = block_exclusive_prefix(tile_sum[tile], tsum, wsum);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             const int k = tile * NODE_TILE + threadIdx.x * 8 + j;
@@ -1172,6 +1020,28 @@ __device__ __forceinline__ void ld256(const ulonglong2* p, ulonglong2& a, ulongl
 __device__ __forceinline__ unsigned ends_first(unsigned cta, unsigned n_ctas) {
     const unsigned tail = (n_ctas + 15u) >> 4;
     return cta < tail ? n_ctas - tail + cta : cta - tail;
+}
+
+// Counting walks: adds the warp's sums of the six counters to the walk's totals in TreeGlobals::counters.
+__device__ __forceinline__ void flush_walk_counters(TreeGlobals* g, u64 c_vis, u64 c_pc, u64 c_pp, u64 c_slots,
+                                                    u64 c_nl, u64 c_na) {
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        c_vis += __shfl_down_sync(FULL, c_vis, s);
+        c_pc += __shfl_down_sync(FULL, c_pc, s);
+        c_pp += __shfl_down_sync(FULL, c_pp, s);
+        c_slots += __shfl_down_sync(FULL, c_slots, s);
+        c_nl += __shfl_down_sync(FULL, c_nl, s);
+        c_na += __shfl_down_sync(FULL, c_na, s);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        atomicAdd(&g->counters[0], c_vis);
+        atomicAdd(&g->counters[1], c_pc);
+        atomicAdd(&g->counters[2], c_pp);
+        atomicAdd(&g->counters[3], c_slots);
+        atomicAdd(&g->counters[4], c_nl);
+        atomicAdd(&g->counters[5], c_na);
+    }
 }
 
 // One target per lane: the "fixed physics" walk -- leaf sources carry their real mass in .w and there is no
@@ -1407,25 +1277,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             acc3[o + 0] = ax; acc3[o + 1] = ay; acc3[o + 2] = az;
         }
     }
-    if (COUNT) {
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) {
-            c_vis += __shfl_down_sync(FULL, c_vis, s);
-            c_pc += __shfl_down_sync(FULL, c_pc, s);
-            c_pp += __shfl_down_sync(FULL, c_pp, s);
-            c_slots += __shfl_down_sync(FULL, c_slots, s);
-            c_nl += __shfl_down_sync(FULL, c_nl, s);
-            c_na += __shfl_down_sync(FULL, c_na, s);
-        }
-        if ((threadIdx.x & 31) == 0) {
-            atomicAdd(&g->counters[0], c_vis);
-            atomicAdd(&g->counters[1], c_pc);
-            atomicAdd(&g->counters[2], c_pp);
-            atomicAdd(&g->counters[3], c_slots);
-            atomicAdd(&g->counters[4], c_nl);
-            atomicAdd(&g->counters[5], c_na);
-        }
-    }
+    if (COUNT) flush_walk_counters(g, c_vis, c_pc, c_pp, c_slots, c_nl, c_na);
 }
 
 // Two targets per lane: a warp owns 64 Hilbert-adjacent targets -- lane l holds targets l (A) and 32 + l (B) of the
@@ -1657,25 +1509,7 @@ walk_warp2_kernel(const float4* __restrict__ posm, const int* __restrict__ order
         w_unpk(by2, lo, hi); acc3[o + 1] = cyB + (lo + hi);
         w_unpk(bz2, lo, hi); acc3[o + 2] = czB + (lo + hi);
     }
-    if (COUNT) {
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) {
-            c_vis += __shfl_down_sync(FULL, c_vis, s);
-            c_pc += __shfl_down_sync(FULL, c_pc, s);
-            c_pp += __shfl_down_sync(FULL, c_pp, s);
-            c_slots += __shfl_down_sync(FULL, c_slots, s);
-            c_nl += __shfl_down_sync(FULL, c_nl, s);
-            c_na += __shfl_down_sync(FULL, c_na, s);
-        }
-        if (lane == 0) {
-            atomicAdd(&g->counters[0], c_vis);
-            atomicAdd(&g->counters[1], c_pc);
-            atomicAdd(&g->counters[2], c_pp);
-            atomicAdd(&g->counters[3], c_slots);
-            atomicAdd(&g->counters[4], c_nl);
-            atomicAdd(&g->counters[5], c_na);
-        }
-    }
+    if (COUNT) flush_walk_counters(g, c_vis, c_pc, c_pp, c_slots, c_nl, c_na);
 }
 
 // order[] of a target range holds range-local indices after the sort: shift to global
