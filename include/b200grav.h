@@ -258,6 +258,29 @@ int b200_tree_set_periodic(b200_ctx* ctx, float box);
  * acc3 or i0 + n_targets > n; n_targets = 0 is a no-op. */
 int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
                              float r_cut, void* acc3, void* stream);
+/* TreePM short-range POTENTIAL: ADDS to phi (float[n_targets], device) of the targets posm4[i0 .. i0+n_targets)
+ *   sum_j m_j erfc(r / 2 r_s) / sqrt(r^2 + eps^2) - m_i / (sqrt(pi) r_s) - 4 pi r_s^2 M / box^3
+ * over the sources of the last b200_tree_build_fixed_dev tree with 0 < r < r_cut (r the unsoftened minimum-image
+ * distance, as the force; the particle itself -- and an exact duplicate -- adds 0), M = the tree's total mass.
+ * The second term removes the target's own long-range self term, which the PM potential (b200_pm_forces_dev's
+ * phi, of the same r_split) holds; the third is the short-range potential of the uniform background, whose long
+ * range the PM mesh removes with its k = 0 mode.  With that PM potential in phi first, phi becomes the periodic potential in the Ewald convention -- positive,
+ * uniform background subtracted, the particle's own direct term excluded and its periodic images included.
+ * The walk, its cell cut-off and its opening test are those of b200_tree_walk_short_dev; an accepted cell adds
+ * M erfc(|d_c| / 2 r_s) / sqrt(|d_c|^2 + eps^2).  theta = 0 gives the exact truncated sum.  Errors: those of
+ * b200_tree_walk_short_dev (phi in place of acc3), and B200_ERR_UNSUPPORTED for theta > 1/sqrt(3) (a target must
+ * not accept a cell that contains itself).  Counting is ignored.  A tree that overflowed writes NaN. */
+int b200_tree_potential_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
+                                  float r_cut, void* phi, void* stream);
+/* TreePM energies of the targets posm4[i0 .. i0+n_targets), after b200_tree_build_fixed_dev(posm4, n_sources, ...)
+ * of the same array (else B200_ERR_STATE): the PM potential of b200_pm_forces_dev (grid, box, r_split; its
+ * acceleration goes to a context scratch buffer) plus b200_tree_potential_short_dev (theta, r_cut), i.e. the Ewald
+ * potential; kinetic = sum 1/2 m v^2 of vel3 (float[3*n_targets], device), potential = -1/2 sum m phi, two HOST
+ * doubles; blocking.  Argument errors are those of the two calls.  For the comoving energies of a cosmological
+ * run pass vel3 = the momenta p and divide: K = kinetic / a^2, W = potential / a. */
+int b200_treepm_energy_dev(b200_ctx* ctx, const void* posm4, size_t n_sources, size_t i0, size_t n_targets,
+                           const void* vel3, int grid, float box, float r_split, float r_cut, float theta,
+                           double* kinetic, double* potential, void* stream);
 /* Energy diagnostic from the fixed-physics tree (after b200_tree_build_fixed_dev): the walk accumulating
  * phi_i = sum m / sqrt(|d|^2 + eps^2) -- M / r for an accepted cell -- so that compute_energy
  * (src/physics/lambda_cdm_kernels.cu:338-408) costs O(N log N) in a tree run instead of O(N^2).
@@ -365,6 +388,16 @@ int b200_leapfrog_host(b200_ctx* ctx, float* pos3, float* vel3, const float* acc
 double b200_hubble_a(double a, double omega_m, double omega_k, double omega_lambda, double h);
 double b200_scale_factor_step(double a, double dt, double omega_m, double omega_k,
                               double omega_lambda, double h);
+/* Comoving leapfrog factors of a KDK step from a0 to a1 (H0 = 1, E(a)^2 = Om a^-3 + Ok a^-2 + OL):
+ *   drift = int_a0^a1 da / (a^3 E(a)),   kick = int_a0^a1 da / (a^2 E(a)).
+ * With the canonical momentum p = a^2 dx/dt and the comoving peculiar acceleration g (G = 1, particle masses
+ * 3 Om L^3 / (8 pi N)), dx/da = p / (a^3 E) and dp/da = g / (a^2 E); a step is: kick by K(a0, am), drift by
+ * D(a0, a1), forces at a1, kick by K(am, a1), am = sqrt(a0 a1) -- b200_leapfrog_dev with a = 1, dt_kick = K,
+ * dt_drift = D.  Double precision, relative error <= 1e-12 (composite Gauss-Legendre in ln a).  a0 == a1 gives
+ * 0.  B200_ERR_INVALID for a0 <= 0, a1 < a0, a non-finite argument, a NULL output, or E^2 <= 0 anywhere on
+ * [a0, a1].  Host scalar: no context, no GPU. */
+int b200_comoving_kdk_factors(double a0, double a1, double omega_m, double omega_k, double omega_lambda,
+                              double* drift, double* kick);
 
 /* ---- initial conditions (SURVEY 8f N3) ------------------------------------------
  * Zel'dovich particles on the device.  Everything the reference's

@@ -78,6 +78,7 @@ int b200_ctx_destroy(b200_ctx* ctx) {
     pm_destroy(ctx);
     ctx->src_tiles.release(); ctx->partials.release(); ctx->mass_flag.release(); ctx->zero_flag.release();
     ctx->energy_part.release(); ctx->energy_phi.release(); ctx->energy_out.release();
+    ctx->energy_acc.release();
     ctx->ic_wk.release(); ctx->ic_tmp.release(); ctx->ic_psi.release(); ctx->ic_stats.release();
     ctx->h_pos3.release(); ctx->h_vel3.release(); ctx->h_mass.release(); ctx->h_posm4.release(); ctx->h_acc3.release();
     ctx->h_tree_posm4.release();
@@ -515,6 +516,40 @@ int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float t
     return tree_walk_short(ctx, i0, n_targets, theta, box, r_split, r_cut, acc3, pick_stream(ctx, stream));
 }
 
+int b200_tree_potential_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
+                                  float r_cut, void* phi, void* stream) {
+    if (!ctx) return B200_ERR_INVALID;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return tree_potential_short(ctx, i0, n_targets, theta, box, r_split, r_cut, phi, pick_stream(ctx, stream));
+}
+
+// PM potential (its acceleration goes to energy_acc), then the short-range potential added to it: the Ewald potential.
+int b200_treepm_energy_dev(b200_ctx* ctx, const void* posm4, size_t n_sources, size_t i0, size_t n_targets,
+                           const void* vel3, int grid, float box, float r_split, float r_cut, float theta,
+                           double* kinetic, double* potential, void* stream) {
+    if (!ctx || !kinetic || !potential) return B200_ERR_INVALID;
+    *kinetic = *potential = 0.0;
+    if (n_targets == 0) return B200_OK;
+    if (!posm4 || !vel3) return B200_ERR_INVALID;
+    if (tree_posm(ctx) != posm4) return B200_ERR_STATE;      // the fixed tree must be of these sources
+    B200_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = pick_stream(ctx, stream);
+    B200_TRY(ctx->energy_phi.reserve(n_targets * sizeof(float)));
+    B200_TRY(ctx->energy_acc.reserve(n_targets * 3 * sizeof(float)));
+    B200_TRY(ctx->energy_out.reserve(2 * sizeof(double)));
+    B200_TRY(b200_pm_forces_dev(ctx, posm4, n_sources, i0, n_targets, grid, box, r_split, ctx->energy_acc.p,
+                                ctx->energy_phi.p, st));
+    B200_TRY(tree_potential_short(ctx, i0, n_targets, theta, box, r_split, r_cut, ctx->energy_phi.p, st));
+    B200_TRY(energy_reduce(ctx, (const float4*)posm4 + i0, vel3, ctx->energy_phi.p, n_targets,
+                           ctx->energy_out.as<double>(), st));
+    double h[2];
+    B200_CUDA(cudaMemcpyAsync(h, ctx->energy_out.p, sizeof h, cudaMemcpyDeviceToHost, st));
+    B200_CUDA(cudaStreamSynchronize(st));
+    *kinetic = h[0];
+    *potential = h[1];
+    return B200_OK;
+}
+
 int b200_tree_set_periodic(b200_ctx* ctx, float box) {
     if (!ctx) return B200_ERR_INVALID;
     return tree_set_periodic(ctx, box);
@@ -590,6 +625,41 @@ double b200_hubble_a(double a, double omega_m, double omega_k, double omega_lamb
     const double aa = 1.0 / (1.0 + z);
     const double e2 = omega_m * pow(aa, -3) + omega_k * pow(aa, -2) + omega_lambda;
     return 100.0 * h * sqrt(e2);
+}
+
+// Comoving KDK factors, H0 = 1: drift = int da / (a^3 E), kick = int da / (a^2 E), E^2 = Om a^-3 + Ok a^-2 + OL.
+// Composite 10-point Gauss-Legendre in ln a (the integrands a^-2 / E and a^-1 / E are smooth in ln a) on panels no
+// wider than 1/8: the quadrature error is far below double rounding, which bounds the result at ~1e-15 relative.
+int b200_comoving_kdk_factors(double a0, double a1, double omega_m, double omega_k, double omega_lambda,
+                              double* drift, double* kick) {
+    if (!drift || !kick || !(a0 > 0.0) || !(a1 >= a0) || !isfinite(a1)) return B200_ERR_INVALID;
+    if (!isfinite(omega_m) || !isfinite(omega_k) || !isfinite(omega_lambda)) return B200_ERR_INVALID;
+    auto e2 = [&](double a) { return omega_m / (a * a * a) + omega_k / (a * a) + omega_lambda; };
+    // E^2 > 0 on [a0, a1]: at both ends and at its one interior extremum a* = -3 Om / (2 Ok), if there is one
+    if (!(e2(a0) > 0.0) || !(e2(a1) > 0.0)) return B200_ERR_INVALID;
+    if (omega_k != 0.0) {
+        const double as = -1.5 * omega_m / omega_k;
+        if (as > a0 && as < a1 && !(e2(as) > 0.0)) return B200_ERR_INVALID;
+    }
+    static const double X[5] = {0.14887433898163122, 0.4333953941292472, 0.6794095682990244, 0.8650633666889845,
+                                0.9739065285171717};
+    static const double W[5] = {0.2955242247147528, 0.2692667193099965, 0.219086362515982, 0.1494513491505804,
+                                0.06667134430868814};
+    const double u0 = log(a0), width = log(a1) - u0;
+    const int panels = (int)ceil(width * 8.0);
+    double sd = 0.0, sk = 0.0;
+    for (int p = 0; p < panels; ++p) {
+        const double h = 0.5 * width / panels, mid = u0 + (2 * p + 1) * h;
+        for (int q = 0; q < 10; ++q) {
+            const double a = exp(mid + (q < 5 ? -X[q] : X[q - 5]) * h);
+            const double w = W[q % 5] * h / (a * sqrt(e2(a)));        // d ln a / E, times 1/a (kick) or 1/a^2 (drift)
+            sk += w;
+            sd += w / a;
+        }
+    }
+    *drift = sd;
+    *kick = sk;
+    return B200_OK;
 }
 
 // src/physics/lambda_cdm_impl.cu:261-269: a += a * H(a) * dt (H in km/s/Mpc, as the reference).

@@ -68,6 +68,7 @@ struct b200_ctx {
     DevBuf zero_flag;       // int that always reads 0 (equal-mass promise of the parts API)
     DevBuf mass_flag;       // int: number of sources whose mass differs from the first
     DevBuf energy_part, energy_phi, energy_out;   // energy diagnostic scratch
+    DevBuf energy_acc;      // the PM acceleration b200_treepm_energy_dev computes with the potential and discards
     DevBuf ic_wk, ic_tmp, ic_psi, ic_stats;       // initial-conditions scratch (released after each call)
     // host-entry staging
     DevBuf h_pos3, h_vel3, h_mass, h_posm4, h_acc3;

@@ -1052,7 +1052,7 @@ __device__ __forceinline__ void flush_walk_counters(TreeGlobals* g, u64 c_vis, u
 // known (after the vote) measured no gain, and speculative requests (the skip target, or id + 1, before the vote)
 // cost time -- every broadcast 256-bit load writes 1 KB into the register file, and in this kernel that return path
 // (l1tex lsu writeback, 128 B per clock and SM) is 76 % busy, as busy as the issue slots: a wrong guess is not free.
-// SHORT (with PERIODIC, without POT): the short-range half of TreePM (b200_tree_walk_short_dev).  Every pair and
+// SHORT (with PERIODIC): the short-range half of TreePM (b200_tree_walk_short_dev).  Every pair and
 // accepted cell is weighted by g(r) = erfc(r / 2 r_s) + r / (r_s sqrt(pi)) exp(-r^2 / 4 r_s^2) of its unsoftened
 // minimum-image distance (inv2rs = 1 / (2 r_s)); pairs at r >= r_cut weigh 0 (r^2 >= rcut2).  A cell whose centre
 // of mass is at least r_cut + sqrt(3) edge away is cut: accepted with weight 0, its subtree skipped -- every
@@ -1061,6 +1061,13 @@ __device__ __forceinline__ void flush_walk_counters(TreeGlobals* g, u64 c_vis, u
 // half-box distance.  The result is added to acc3.  COUNT: the pair interactions (counter 2) are the pairs inside
 // r_cut; the pair-row slots (counter 3) still count every leaf pair issued.  The walk fits the 56 registers of 9
 // resident CTAs per SM without spilling; its counting instance spills there and gets 8 (64 registers).
+// SHORT and POT: the short-range potential (b200_tree_potential_short_dev), same cut-off and cell cut, a pair or an
+// accepted cell adding m erfc(r / 2 r_s) / sqrt(r^2 + eps^2).  Pairs at r = 0 add 0: the particle itself is skipped
+// rather than added as m / eps and subtracted, which would round the whole sum at the ulp of m / eps.  The result,
+// minus the target's own long-range self term m / (sqrt(pi) r_s) that the PM potential holds and minus the
+// short-range potential 4 pi r_s^2 M / box^3 of the uniform background (M = the root's mass; the PM potential has
+// only its long range), is added to acc3[i - i0]: the PM potential plus this is the Ewald potential.  No counting
+// instance.
 template <bool COUNT, bool PERIODIC, bool POT, bool SHORT = false>
 __global__ void __launch_bounds__(128, SHORT && COUNT ? 8 : 9)
 walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order, int i0, int n_targets,
@@ -1068,7 +1075,7 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                  const ulonglong2* __restrict__ leaf_pairs, float theta, float theta2, float eps2, float box,
                  float* __restrict__ acc3, TreeGlobals* __restrict__ g, int by_slot, float inv2rs, float rcut,
                  float rcut2) {
-    static_assert(!SHORT || (PERIODIC && !POT), "the short-range walk is periodic and has no potential");
+    static_assert(!SHORT || PERIODIC, "the short-range walk is periodic");
     typedef unsigned long long u64;
     const int t = ends_first(blockIdx.x, gridDim.x) * blockDim.x + threadIdx.x;
     const bool valid = t < n_targets;
@@ -1119,6 +1126,13 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
                 float d2a, d2b, r2a, r2b;
                 w_unpk(d2, d2a, d2b);
                 w_unpk(w_add2(d2, e2_2), r2a, r2b);
+                if constexpr (POT) {       // erfc of the unsoftened distance over the softened one; r = 0 adds 0
+                    const float ea = d2a < rcut2 && d2a > 0.0f ? treepm_short_erfc(sqrt_fast(d2a) * inv2rs) : 0.0f;
+                    const float eb = d2b < rcut2 && d2b > 0.0f ? treepm_short_erfc(sqrt_fast(d2b) * inv2rs) : 0.0f;
+                    const u64 rinv = w_pk(rsqrt_fast(r2a), rsqrt_fast(r2b));
+                    ax2 = w_fma2(rinv, w_mul2(b.y, w_pk(ea, eb)), ax2);
+                    return;
+                }
                 const bool ina = d2a < rcut2, inb = d2b < rcut2;
                 const float ga = ina ? treepm_short_g(sqrt_fast(d2a) * inv2rs) : 0.0f;
                 const float gb = inb ? treepm_short_g(sqrt_fast(d2b) * inv2rs) : 0.0f;
@@ -1212,8 +1226,12 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
             auto monopole = [&](bool take) {                                 // :280-290; 1/r = 0 for a lane that is out
                 if constexpr (SHORT) {
                     const float rinv = (take && !cut) ? rsqrt_fast(d2 + eps2) : 0.0f;
-                    const float f = c.w * treepm_short_g(sqrt_fast(d2) * inv2rs) * rinv * rinv * rinv;
-                    ax = fmaf(f, dx, ax); ay = fmaf(f, dy, ay); az = fmaf(f, dz, az);
+                    if constexpr (POT) {
+                        ax = fmaf(c.w * treepm_short_erfc(sqrt_fast(d2) * inv2rs), rinv, ax);
+                    } else {
+                        const float f = c.w * treepm_short_g(sqrt_fast(d2) * inv2rs) * rinv * rinv * rinv;
+                        ax = fmaf(f, dx, ax); ay = fmaf(f, dy, ay); az = fmaf(f, dz, az);
+                    }
                     if (COUNT) c_pc += take && !cut;
                     if (take) wake = skip;
                     return;
@@ -1267,7 +1285,12 @@ walk_warp_kernel(const float4* __restrict__ posm, const int* __restrict__ order,
     if (valid) {
         float lo, hi;
         w_unpk(ax2, lo, hi); ax += lo + hi;
-        if constexpr (POT) {
+        if constexpr (SHORT && POT) {
+            // minus m / (sqrt(pi) r_s) (2 / sqrt(pi) = 1.128...) and the background's 4 pi r_s^2 M / box^3, M = the
+            // root's mass
+            const float bg = 3.14159265f * c.w / (inv2rs * inv2rs * box * box * box);
+            acc3[i - i0] += fmaf(-p.w, 1.128379167f * inv2rs, ax) - bg;
+        } else if constexpr (POT) {
             acc3[i - i0] = ax - p.w * rsqrt_fast(eps2);                  // minus the i == i term of the pair loop
         } else {
             w_unpk(ay2, lo, hi); ay += lo + hi;
@@ -1976,6 +1999,26 @@ int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, flo
                                  T->leaf_pos.as<ulonglong2>(), theta, theta2, T->eps * T->eps, box, (float*)acc3,
                                  T->globals.as<TreeGlobals>(), 0, 0.5f / r_split, r_cut, r_cut * r_cut);
     if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev1, st));
+    B200_CUDA(cudaGetLastError());
+    ctx->launches += 1;
+    return B200_OK;
+}
+
+// The short-range TreePM potential (walk_warp_kernel, SHORT and POT) of the same targets, added to phi: the checks
+// of tree_walk_short plus the theta bound of tree_potential.
+int tree_potential_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
+                         float r_cut, void* phi, cudaStream_t st) {
+    TreeState* T = ctx->tree;
+    if (!T || !T->built || !T->fixed) return B200_ERR_STATE;
+    if (!(box > 0.f) || !(r_split > 0.f) || !(r_cut > 0.f) || !(r_cut < 0.5f * box)) return B200_ERR_INVALID;
+    if (!(theta <= 0.57735f)) return B200_ERR_UNSUPPORTED;  // a target must never accept a cell containing itself
+    if (n_targets == 0) return B200_OK;
+    if (!phi || i0 + n_targets > T->n) return B200_ERR_INVALID;
+    B200_TRY(tree_target_order(ctx, T, i0, n_targets, st));
+    walk_warp_kernel<false, true, true, true><<<(unsigned)((n_targets + 127) / 128), 128, 0, st>>>(
+        T->posm, T->order.as<int>(), (int)i0, (int)n_targets, T->nodes.as<float4>(), T->leaf_pos.as<ulonglong2>(),
+        theta, theta > 0.f ? theta * theta : 0.f, T->eps * T->eps, box, (float*)phi, T->globals.as<TreeGlobals>(), 0,
+        0.5f / r_split, r_cut, r_cut * r_cut);
     B200_CUDA(cudaGetLastError());
     ctx->launches += 1;
     return B200_OK;

@@ -31,6 +31,7 @@ EXPORTS = [
     "b200_ic_params_default", "b200_zeldovich_ics_dev", "b200_force_error_dev", "b200_power_spectrum_dev", "b200_tree_build_fixed_dev", "b200_tree_forces_fixed_host", "b200_tree_set_periodic", "b200_tree_walk_short_dev", "b200_spatial_order_dev", "b200_tree_build_host", "b200_tree_walk_host", "b200_tree_potential_dev", "b200_tree_energy_dev",
     "b200_fp32_peak_probe", "b200_last_kernel_ms", "b200_set_timing", "b200_launch_count",
     "b200_pm_forces_dev", "b200_pm_forces_host", "b200_pm_phase_ms",
+    "b200_comoving_kdk_factors", "b200_tree_potential_short_dev", "b200_treepm_energy_dev",
 ]
 
 
@@ -129,6 +130,10 @@ def load_library(path=None):
     L.b200_pm_forces_dev.argtypes = [vp, vp, sz, sz, sz, i32, f32, f32, vp, vp, vp]
     L.b200_pm_forces_host.argtypes = [vp, vp, vp, vp, sz, i32, f32, f32]
     L.b200_pm_phase_ms.argtypes = [vp, vp]
+    L.b200_comoving_kdk_factors.argtypes = [f64] * 5 + [C.POINTER(f64)] * 2
+    L.b200_tree_potential_short_dev.argtypes = [vp, sz, sz, f32, f32, f32, f32, vp, vp]
+    L.b200_treepm_energy_dev.argtypes = [vp, vp, sz, sz, sz, vp, i32, f32, f32, f32, f32, C.POINTER(f64),
+                                         C.POINTER(f64), vp]
     L.b200_fp32_peak_probe.argtypes = [vp, i32, i32, C.POINTER(f64), C.POINTER(f32)]
     L.b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
     L.b200_set_timing.argtypes = [vp, i32]
@@ -288,6 +293,25 @@ class Engine:
         self.pm_forces_dev(posm, acc, i0, n_targets, grid, box, rs, stream=stream)
         return self.tree_walk_short_dev(acc, i0, n_targets, theta, box, rs, r_cut_factor * rs, stream)
 
+    def tree_potential_short_dev(self, phi, i0, n_targets, theta, box, r_split, r_cut, stream=None):
+        """Adds the TreePM short-range potential minus the PM self term (b200_tree_potential_short_dev) of targets
+        [i0, i0+n_targets) of the last fixed-physics tree to phi (device float[n_targets])."""
+        self._check(self.L.b200_tree_potential_short_dev(self._h, i0, n_targets, theta, box, r_split, r_cut,
+                                                         _ptr(phi), _stream(stream)))
+        return phi
+
+    def treepm_energy_dev(self, posm, vel, i0, n_targets, grid, box, r_split=None, r_cut=None, theta=0.5,
+                          stream=None):
+        """(sum 1/2 m v^2, -1/2 sum m phi) of targets posm[i0 : i0+n_targets), phi the TreePM (Ewald-convention)
+        potential; the fixed-physics tree of posm must be built.  r_split=None: 1.25 box / grid; r_cut=None:
+        4.5 r_split."""
+        rs = 1.25 * box / grid if r_split is None else r_split
+        rc = 4.5 * rs if r_cut is None else r_cut
+        ke, pe = C.c_double(), C.c_double()
+        self._check(self.L.b200_treepm_energy_dev(self._h, _ptr(posm), posm.shape[0], i0, n_targets, _ptr(vel), grid,
+                                                  box, rs, rc, theta, C.byref(ke), C.byref(pe), _stream(stream)))
+        return ke.value, pe.value
+
     def tree_forces_host(self, pos, mass, theta=0.5, leaf_cap=8, max_depth=20, box=100.0, out=None):
         pos = np.ascontiguousarray(pos, np.float32)
         mass = np.ascontiguousarray(mass, np.float32)
@@ -387,6 +411,10 @@ class Engine:
 
     def scale_factor_step(self, a, dt, om=0.31, ok=0.0, ol=0.69, h=0.67):
         return float(self.L.b200_scale_factor_step(a, dt, om, ok, ol, h))
+
+    def comoving_kdk_factors(self, a0, a1, om=0.31, ok=0.0, ol=0.69):
+        """(drift, kick) = (int da / (a^3 E), int da / (a^2 E)) from a0 to a1, H0 = 1."""
+        return comoving_kdk_factors(self.L, a0, a1, om, ok, ol)
 
     def pack_posm_dev(self, pos3, mass, n, posm, stream=None):
         self._check(self.L.b200_pack_posm_dev(self._h, _ptr(pos3), _ptr(mass), n, _ptr(posm), _stream(stream)))
@@ -606,6 +634,114 @@ class LambdaCDMSimulation:
 
     def velocities(self):
         return self.vel.cpu().numpy()
+
+
+def comoving_kdk_factors(lib, a0, a1, om=0.31, ok=0.0, ol=0.69):
+    """b200_comoving_kdk_factors through a loaded library (a host scalar: no context, no GPU)."""
+    d, k = C.c_double(), C.c_double()
+    rc = lib.b200_comoving_kdk_factors(a0, a1, om, ok, ol, C.byref(d), C.byref(k))
+    if rc != 0:
+        raise B200Error(f"b200grav status {rc}: {lib.b200_error_string(rc).decode()}")
+    return d.value, k.value
+
+
+def comoving_zeldovich_dev(engine, **params):
+    """Zel'dovich particles (Engine.zeldovich_ics_dev, params as there) in the units of ComovingSimulation:
+    returns (pos, mom, mass, a0) as device tensors and a float -- positions in [0, box), masses 3 Om box^3 / (8 pi N)
+    (mean density Om rho_crit with G = H0 = 1), momenta p = a v / (100 h) (v = a H f D psi in km/s with
+    H = 100 h E, so v / (100 h) is the peculiar velocity in box units times H0)."""
+    import torch
+    p = ICParams()
+    engine.L.b200_ic_params_default(C.byref(p))
+    for k, v in params.items():
+        setattr(p, k, v)
+    n = p.grid ** 3
+    dev = torch.device("cuda", engine.device)
+    posm = torch.empty((n, 4), dtype=torch.float32, device=dev)
+    vel = torch.empty((n, 3), dtype=torch.float32, device=dev)
+    engine.zeldovich_ics_dev(posm, vel, **params)
+    a0 = 1.0 / (1.0 + p.z_initial)
+    mass = torch.full((n,), 3.0 * p.omega_m * float(p.box) ** 3 / (8.0 * np.pi * n), dtype=torch.float32, device=dev)
+    return posm[:, :3].contiguous(), vel * (a0 / (100.0 * p.h)), mass, a0
+
+
+class ComovingSimulation:
+    """Comoving KDK integration of a periodic LambdaCDM box with the PM or TreePM force (DESIGN 3.13).
+
+    Units: comoving lengths in the box's unit, time in 1 / H0 (H0 = 1), G = 1; masses 3 Om L^3 / (8 pi N) give the
+    mean density Om rho_crit, and the engine's periodic acceleration g is then the comoving peculiar acceleration.
+    State: positions x in [0, box), canonical momenta p = a^2 dx/dt (peculiar velocity p / a).  Equations of
+    motion dx/da = p / (a^3 E), dp/da = g / (a^2 E), E^2 = Om a^-3 + Ok a^-2 + OL.  step(a1) from a0: half-kick
+    K(a0, am), drift D(a0, a1), forces at a1, half-kick K(am, a1), am = sqrt(a0 a1), with the exact factors of
+    b200_comoving_kdk_factors.  force: "treepm" (PM on a pm_grid^3 mesh plus the short-range walk at theta,
+    softening eps, cut off at 4.5 r_split) or "pm"; r_split=None: 1.25 box / pm_grid."""
+
+    def __init__(self, engine, pos, mom, mass, box, a0, force="treepm", pm_grid=128, r_split=None, theta=0.5,
+                 eps=0.01, leaf_cap=8, max_depth=20, cosmo=(0.31, 0.0, 0.69)):
+        import torch
+        if force not in ("treepm", "pm"):
+            raise ValueError(f"force must be 'treepm' or 'pm', not {force!r}")
+        self.e = engine
+        dev = torch.device("cuda", engine.device)
+        f32 = lambda x: torch.as_tensor(x, dtype=torch.float32, device=dev)
+        self.posm = torch.cat([f32(pos).reshape(-1, 3), f32(mass).reshape(-1, 1)], 1).contiguous()
+        self.mom = f32(mom).reshape(-1, 3).clone()
+        self.n = self.posm.shape[0]
+        self.acc = torch.zeros((self.n, 3), dtype=torch.float32, device=dev)
+        self.box, self.force, self.theta, self.eps = float(box), force, float(theta), float(eps)
+        self.pm_grid, self.leaf_cap, self.max_depth = int(pm_grid), leaf_cap, max_depth
+        self.r_split = 1.25 * self.box / self.pm_grid if r_split is None else float(r_split)
+        self.cosmo = tuple(float(c) for c in cosmo)
+        self.a = float(a0)
+        self.steps = 0
+        self.have_forces = False
+
+    @property
+    def scale_factor(self):
+        return self.a
+
+    def compute_forces(self):
+        if self.force == "pm":
+            self.e.pm_forces_dev(self.posm, self.acc, 0, self.n, self.pm_grid, self.box, self.r_split)
+        else:
+            self.e.treepm_forces_dev(self.posm, self.acc, 0, self.n, self.pm_grid, self.box, self.r_split,
+                                     theta=self.theta, leaf_cap=self.leaf_cap, max_depth=self.max_depth, eps=self.eps)
+        self.have_forces = True
+
+    def step(self, a_next):
+        a0, a1 = self.a, float(a_next)
+        am = np.sqrt(a0 * a1)
+        drift, _ = self.e.comoving_kdk_factors(a0, a1, *self.cosmo)
+        _, k0 = self.e.comoving_kdk_factors(a0, am, *self.cosmo)
+        _, k1 = self.e.comoving_kdk_factors(am, a1, *self.cosmo)
+        if not self.have_forces:
+            self.compute_forces()
+        # b200_leapfrog_dev at a = 1 (1/a^2 = 1 exactly) with dt_kick = K and dt_drift = D is the comoving kick and
+        # drift: p += g K, x += p D, x wrapped into [0, box)
+        self.e.leapfrog_dev(self.posm, self.mom, self.acc, self.n, 1, np.float32(k0), 1.0, np.float32(drift),
+                            self.box)
+        self.compute_forces()
+        self.e.leapfrog_dev(self.posm, self.mom, self.acc, self.n, 1, np.float32(k1), 1.0, 0.0, self.box)
+        self.a = a1
+        self.steps += 1
+
+    def energies(self):
+        """(K, W) at the current scale factor (force="treepm" only): K = sum 1/2 m p^2 / a^2 and
+        W = -1/2 sum m phi / a, phi the periodic potential in the Ewald convention.  The Layzer-Irvine equation
+        d[a (K + W)] = -K da holds for them."""
+        if self.force != "treepm":
+            raise ValueError("energies() needs force='treepm'")
+        if not self.have_forces:
+            self.compute_forces()       # builds the fixed-physics tree of the current positions
+        ke, pe = self.e.treepm_energy_dev(self.posm, self.mom, 0, self.n, self.pm_grid, self.box, self.r_split,
+                                          4.5 * self.r_split, self.theta)
+        return ke / (self.a * self.a), pe / self.a
+
+    def positions(self):
+        return self.posm[:, :3].cpu().numpy()
+
+    def momenta(self):
+        return self.mom.cpu().numpy()
 
 
 # ---------------------------------------------------------------------------
