@@ -258,6 +258,18 @@ int b200_tree_set_periodic(b200_ctx* ctx, float box);
  * acc3 or i0 + n_targets > n; n_targets = 0 is a no-op. */
 int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
                              float r_cut, void* acc3, void* stream);
+/* Short range of the particles active at sync point k of the block time steps (b200_block_kick_dev, DESIGN 3.14).
+ * With L = max_bins - 1, particle i is active when k is a multiple of 2^(L - bins_u8[i]) (a stored bin above L
+ * counts as L; every particle is active at k = 0 and k = 2^L).  Their rows of acc_short3 (float[3n], device) are
+ * set to the short-range acceleration of b200_tree_walk_short_dev (the same walk, bit for bit); the rows of
+ * inactive particles are not touched.  *n_active (HOST) = the number of active particles; for 0 < k < 2^L the
+ * call synchronises the stream to read it.  The tree must be the last b200_tree_build_fixed_dev of exactly n sources (else B200_ERR_STATE, as
+ * without a fixed-physics tree); B200_ERR_INVALID for max_bins outside 1..16, k outside 0..2^L, a NULL bins_u8,
+ * acc_short3 or n_active, and the box / r_split / r_cut rules of b200_tree_walk_short_dev.  Counting and timing
+ * as there. */
+int b200_tree_walk_short_active_dev(b200_ctx* ctx, const void* bins_u8, size_t n, int k, int max_bins, float theta,
+                                    float box, float r_split, float r_cut, void* acc_short3, size_t* n_active,
+                                    void* stream);
 /* TreePM short-range POTENTIAL: ADDS to phi (float[n_targets], device) of the targets posm4[i0 .. i0+n_targets)
  *   sum_j m_j erfc(r / 2 r_s) / sqrt(r^2 + eps^2) - m_i / (sqrt(pi) r_s) - 4 pi r_s^2 M / box^3
  * over the sources of the last b200_tree_build_fixed_dev tree with 0 < r < r_cut (r the unsoftened minimum-image
@@ -398,6 +410,33 @@ double b200_scale_factor_step(double a, double dt, double omega_m, double omega_
  * [a0, a1].  Host scalar: no context, no GPU. */
 int b200_comoving_kdk_factors(double a0, double a1, double omega_m, double omega_k, double omega_lambda,
                               double* drift, double* kick);
+/* Block (hierarchical) time steps of the comoving KDK, DESIGN 3.14: one sync point k of a PM step from a0 to a1,
+ * Delta = ln(a1 / a0), divided into S = 2^L sub-steps (L = max_bins - 1) uniform in ln a.  Particle i steps in bin
+ * bins_u8[i] (uint8[n], device): 2^(L - b) sub-steps; its step ends, and the next begins, where k is a multiple
+ * of that.  Every kick is b200_leapfrog_dev's kick at a = 1.  factors_dev (float, device): the opening kicks
+ * Ko[b][j] at (2^b - 1) + j and the closing kicks Kc[b][j] at (2^max_bins - 1) + (2^b - 1) + j, b <= L,
+ * j < 2^b, the float casts of b200_comoving_kdk_factors over the halves of step j of bin b; Ko[0][0] and Kc[0][0]
+ * are also the long-range kicks.  One pass over posm4 (masses), mom3, acc3 (the total acceleration), acc_long3,
+ * acc_short3 (float[3n]) and the bins, in this order per particle:
+ *   k > 0, step of bin b ends: k = S: acc = fl(acc_long + acc_short), then bin 0 kicks with acc Kc[0][0], other
+ *     bins with acc_long Kc[0][0] and then acc_short Kc[b][S / w_b - 1]; 0 < k < S: acc_short Kc[b][k / w_b - 1],
+ *     then the bin becomes max(b*, L - ctz(k)) (a longer step only where it starts on its own grid);
+ *   k = 0: the bin becomes b* of the stored acc, then bin 0 kicks with acc Ko[0][0], other bins with
+ *     acc_long Ko[0][0] and then acc_short Ko[b][0];  0 < k < S, rebinned above: acc_short Ko[b][k / w_b].
+ * b* = the smallest b < L with float(dlna^2 / 4^b) |g| <= crit, else L (also for a non-finite |g|), with |g| =
+ * sqrt((gx^2 + gy^2) + gz^2) rounded per operation and g = acc at k = 0, fl(acc_long + acc_short) at 0 < k < S:
+ * the criterion dln a <= sqrt(2 eta eps a^3 E^2 / |g|) with crit = float(2 eta eps a_k^3 E(a_k)^2).  Then, with
+ * drift != 0 (k < S), every particle drifts as in b200_leapfrog_dev: x += p drift, wrapped into [0, box) when
+ * box > 0.  The drift runs to the next sync point k' at which a step ends, D(a_k, a_k'), so that idle sub-steps
+ * are skipped whole; k' depends on the bins this pass writes unless max_bins = 1 (k' = S), so a caller that does
+ * not know it passes drift = 0, reads the histogram and drifts with b200_leapfrog_dev (n_kicks = 0): the same
+ * float operations.  hist_u32_dev (uint32[16], device) is set to the count of particles per bin after the pass.
+ * acc3 is read at k = 0 and written at k = S only.  B200_ERR_INVALID for max_bins outside 1..16, k outside
+ * 0..2^L, crit < 0 or NaN, dlna < 0 or not finite, drift not finite or != 0 at k = S, a NULL buffer, posm4 / mom3
+ * / acc3 / acc_long3 / acc_short3 not 16-byte aligned.  n = 0 only clears the histogram. */
+int b200_block_kick_dev(b200_ctx* ctx, void* posm4, void* mom3, void* acc3, const void* acc_long3,
+                        const void* acc_short3, void* bins_u8, size_t n, int k, int max_bins, const void* factors_dev,
+                        float crit, double dlna, void* hist_u32_dev, float drift, float box, void* stream);
 
 /* ---- initial conditions (SURVEY 8f N3) ------------------------------------------
  * Zel'dovich particles on the device.  Everything the reference's

@@ -516,6 +516,15 @@ int b200_tree_walk_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float t
     return tree_walk_short(ctx, i0, n_targets, theta, box, r_split, r_cut, acc3, pick_stream(ctx, stream));
 }
 
+int b200_tree_walk_short_active_dev(b200_ctx* ctx, const void* bins_u8, size_t n, int k, int max_bins, float theta,
+                                    float box, float r_split, float r_cut, void* acc_short3, size_t* n_active,
+                                    void* stream) {
+    if (!ctx) return B200_ERR_INVALID;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return tree_walk_short_active(ctx, bins_u8, n, k, max_bins, theta, box, r_split, r_cut, acc_short3, n_active,
+                                  pick_stream(ctx, stream));
+}
+
 int b200_tree_potential_short_dev(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
                                   float r_cut, void* phi, void* stream) {
     if (!ctx) return B200_ERR_INVALID;
@@ -587,6 +596,15 @@ int b200_leapfrog_dev(b200_ctx* ctx, void* posm4, void* vel3, const void* acc3, 
     B200_CUDA(cudaSetDevice(ctx->device));
     return leapfrog(ctx, posm4, vel3, acc3, n, n_kicks, dt_kick, a, dt_drift, box,
                     pick_stream(ctx, stream));
+}
+
+int b200_block_kick_dev(b200_ctx* ctx, void* posm4, void* mom3, void* acc3, const void* acc_long3,
+                        const void* acc_short3, void* bins_u8, size_t n, int k, int max_bins, const void* factors_dev,
+                        float crit, double dlna, void* hist_u32_dev, float drift, float box, void* stream) {
+    if (!ctx) return B200_ERR_INVALID;
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return block_kick(ctx, posm4, mom3, acc3, acc_long3, acc_short3, bins_u8, n, k, max_bins, factors_dev, crit, dlna,
+                      hist_u32_dev, drift, box, pick_stream(ctx, stream));
 }
 
 int b200_leapfrog_host(b200_ctx* ctx, float* pos3, float* vel3, const float* acc3, const float* mass,

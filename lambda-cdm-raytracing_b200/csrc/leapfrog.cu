@@ -19,6 +19,7 @@
 //     x  = fmodf((x + v*dt) + box, box)            (:322-329)
 #include "common.cuh"
 #include "leapfrog.cuh"
+#include "blockstep.cuh"
 
 namespace b200 {
 namespace {
@@ -143,6 +144,133 @@ leapfrog_kernel(float4* __restrict__ posm, float4* __restrict__ vel4, const floa
     }
 }
 
+// ---- hierarchical time steps: the sync-point pass (DESIGN 3.14) ----------------------------------------------------
+// Bin thresholds of the time-step criterion: t[b] = float(dlna^2 / 4^b) for b <= L (host-computed, double first).
+struct BinThresholds { float t[BLOCK_MAX_BINS]; };
+
+// The smallest b < L with t[b] |g| <= crit, else L (a non-finite |g| fails every test); |g| with one rounding per
+// operation in a fixed order, so that numpy restates it bit for bit.
+__device__ __forceinline__ int desired_bin(float gx, float gy, float gz, const BinThresholds& thr, float crit, int L) {
+    const float g = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(gx, gx), __fmul_rn(gy, gy)), __fmul_rn(gz, gz)));
+    for (int b = 0; b < L; ++b)
+        if (__fmul_rn(thr.t[b], g) <= crit) return b;
+    return L;
+}
+
+constexpr int BK_THREADS = 128;
+constexpr int BK_PER = 2;
+constexpr int BK_TILE = BK_THREADS * BK_PER;           // 256 particles, 192 float4 words per 3-float array; 2048
+                                                       // threads per SM (at 8 CTAs of 512 particles, 1024, the
+                                                       // pass took twice leapfrog_kernel's time per byte)
+constexpr int BK_WORDS = 3 * BK_TILE / 4;
+
+// Floats [0, nf) of a tile's 3-float rows between global and shared memory: whole 16-byte words as vectors (lane l
+// of a warp moves bytes [16 l, 16 l + 16) of a 512-byte run), the one word that the ragged end of n cuts, by floats.
+__device__ __forceinline__ void bk_load(float* __restrict__ s, const float* __restrict__ g, int nf) {
+    for (int w = threadIdx.x; w < BK_WORDS; w += BK_THREADS) {
+        if (4 * w + 4 <= nf) reinterpret_cast<float4*>(s)[w] = reinterpret_cast<const float4*>(g)[w];
+        else for (int q = 4 * w; q < nf && q < 4 * w + 4; ++q) s[q] = g[q];
+    }
+}
+__device__ __forceinline__ void bk_store(float* __restrict__ g, const float* __restrict__ s, int nf) {
+    for (int w = threadIdx.x; w < BK_WORDS; w += BK_THREADS) {
+        if (4 * w + 4 <= nf) reinterpret_cast<float4*>(g)[w] = reinterpret_cast<const float4*>(s)[w];
+        else for (int q = 4 * w; q < nf && q < 4 * w + 4; ++q) g[q] = s[q];
+    }
+}
+
+__device__ __forceinline__ void kick3(float* v, const float* a, float m, float minv, float dt) {
+    v[0] = kick1(v[0], a[0], m, minv, dt, 1.0f);
+    v[1] = kick1(v[1], a[1], m, minv, dt, 1.0f);
+    v[2] = kick1(v[2], a[2], m, minv, dt, 1.0f);
+}
+
+// Sync point k of a PM step of S = 2^L sub-steps: closing kicks, rebinning, opening kicks, bin histogram, and with
+// drift != 0 the drift of every particle.  fac holds the opening kicks Ko[b][j] at (2^b - 1) + j and the closing
+// kicks Kc[b][j] 2^(L+1) - 1 further; Ko[0][0] and Kc[0][0] are also the long-range kicks.  mom, and at k = S acc,
+// are written back for the whole tile.
+__global__ void __launch_bounds__(BK_THREADS, 16)
+block_kick_kernel(float4* __restrict__ posm, float* __restrict__ mom3, float* __restrict__ acc3,
+                  const float* __restrict__ long3, const float* __restrict__ short3, unsigned char* __restrict__ bins,
+                  long long n, int k, int L, const float* __restrict__ fac, float crit, BinThresholds thr,
+                  unsigned* __restrict__ hist, float drift, float box) {
+    __shared__ __align__(16) float sv[3 * BK_TILE], sa[3 * BK_TILE], sl[3 * BK_TILE], ss[3 * BK_TILE];
+    __shared__ unsigned sh_hist[BLOCK_MAX_BINS];
+    const int S = 1 << L;
+    const float* Ko = fac;
+    const float* Kc = fac + ((2 << L) - 1);
+    if (threadIdx.x < BLOCK_MAX_BINS) sh_hist[threadIdx.x] = 0;
+    const long long n_tiles = (n + BK_TILE - 1) / BK_TILE;
+    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        const long long base = tile * BK_TILE;
+        const int m = (int)(n - base < BK_TILE ? n - base : BK_TILE);
+        bk_load(sv, mom3 + 3 * base, 3 * m);
+        if (k > 0 || L > 0) {                               // one bin: at k = 0 every particle kicks with acc
+            bk_load(sl, long3 + 3 * base, 3 * m);
+            bk_load(ss, short3 + 3 * base, 3 * m);
+        }
+        if (k == 0) bk_load(sa, acc3 + 3 * base, 3 * m);
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < BK_PER; ++j) {
+            const int q = j * BK_THREADS + threadIdx.x;
+            if (q >= m) continue;
+            float* v = sv + 3 * q;
+            float* a = sa + 3 * q;
+            const float* gl = sl + 3 * q;
+            const float* gs = ss + 3 * q;
+            float4 p = posm[base + q];
+            const float mass = p.w, minv = __fdiv_rn(1.0f, mass);
+            int b = block_bin(bins[base + q], L);
+            bool open = false;
+            if (k == 0) {                                   // every step starts: rebin from the stored total
+                b = desired_bin(a[0], a[1], a[2], thr, crit, L);
+                open = true;
+            } else if (block_active(b, k, L)) {             // the step of bin b ends at k
+                const float kc = Kc[(1 << b) - 1 + (k >> (L - b)) - 1];
+                if (k == S) {
+                    a[0] = __fadd_rn(gl[0], gs[0]); a[1] = __fadd_rn(gl[1], gs[1]); a[2] = __fadd_rn(gl[2], gs[2]);
+                    if (b == 0) {
+                        kick3(v, a, mass, minv, kc);
+                    } else {
+                        kick3(v, gl, mass, minv, Kc[0]);
+                        kick3(v, gs, mass, minv, kc);
+                    }
+                } else {
+                    kick3(v, gs, mass, minv, kc);
+                    const int lo = L - (__ffs(k) - 1);       // the longest step that starts on its own grid at k
+                    const int want = desired_bin(__fadd_rn(gl[0], gs[0]), __fadd_rn(gl[1], gs[1]),
+                                                 __fadd_rn(gl[2], gs[2]), thr, crit, L);
+                    b = want > lo ? want : lo;
+                    open = true;
+                }
+            }
+            if (open) {                                     // k < S: the (new) step of bin b starts at k
+                const float ko = Ko[(1 << b) - 1 + (k >> (L - b))];
+                if (k == 0 && b == 0) {
+                    kick3(v, a, mass, minv, ko);
+                } else {
+                    if (k == 0) kick3(v, gl, mass, minv, Ko[0]);
+                    kick3(v, gs, mass, minv, ko);
+                }
+            }
+            if (drift != 0.f) {
+                p.x = drift1(p.x, v[0], drift, box);
+                p.y = drift1(p.y, v[1], drift, box);
+                p.z = drift1(p.z, v[2], drift, box);
+                posm[base + q] = p;
+            }
+            bins[base + q] = (unsigned char)b;
+            atomicAdd(&sh_hist[b], 1u);
+        }
+        __syncthreads();
+        bk_store(mom3 + 3 * base, sv, 3 * m);
+        if (k == S) bk_store(acc3 + 3 * base, sa, 3 * m);
+        __syncthreads();                                    // sv / sa are refilled by the next tile
+    }
+    if (threadIdx.x < BLOCK_MAX_BINS && sh_hist[threadIdx.x]) atomicAdd(&hist[threadIdx.x], sh_hist[threadIdx.x]);
+}
+
 __global__ void pack_posm_kernel(const float* __restrict__ pos3, const float* __restrict__ mass,
                                  long long n, float4* __restrict__ posm) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -226,6 +354,33 @@ int leapfrog(b200_ctx* ctx, void* posm4, void* vel3, const void* acc3, size_t n,
         ctx->launches += 1;
     }
     B200_CUDA(cudaGetLastError());
+    return B200_OK;
+}
+
+int block_kick(b200_ctx* ctx, void* posm4, void* mom3, void* acc3, const void* acc_long3, const void* acc_short3,
+               void* bins_u8, size_t n, int k, int max_bins, const void* factors, float crit, double dlna,
+               void* hist_u32, float drift, float box, cudaStream_t st) {
+    if (max_bins < 1 || max_bins > BLOCK_MAX_BINS) return B200_ERR_INVALID;
+    const int L = max_bins - 1;
+    if (k < 0 || k > (1 << L)) return B200_ERR_INVALID;
+    if (!isfinite(drift) || (k == (1 << L) && drift != 0.f)) return B200_ERR_INVALID;
+    if (!(crit >= 0.f) || !(dlna >= 0.0) || !isfinite(dlna)) return B200_ERR_INVALID;
+    if (!posm4 || !mom3 || !acc3 || !acc_long3 || !acc_short3 || !bins_u8 || !factors || !hist_u32)
+        return B200_ERR_INVALID;
+    if (((uintptr_t)posm4 | (uintptr_t)mom3 | (uintptr_t)acc3 | (uintptr_t)acc_long3 | (uintptr_t)acc_short3) & 15)
+        return B200_ERR_INVALID;
+    if (((uintptr_t)factors | (uintptr_t)hist_u32) & 3) return B200_ERR_INVALID;
+    B200_CUDA(cudaMemsetAsync(hist_u32, 0, BLOCK_MAX_BINS * sizeof(unsigned), st));
+    if (n == 0) return B200_OK;
+    BinThresholds thr = {};
+    for (int b = 0; b <= L; ++b) thr.t[b] = (float)(dlna * dlna / ldexp(1.0, 2 * b));
+    const long long tiles = ((long long)n + BK_TILE - 1) / BK_TILE;
+    const long long cap = (long long)ctx->sm_count * 16;   // 16 CTAs per SM (12 KB of shared memory, 32 registers)
+    block_kick_kernel<<<(unsigned)(tiles < cap ? tiles : cap), BK_THREADS, 0, st>>>(
+        (float4*)posm4, (float*)mom3, (float*)acc3, (const float*)acc_long3, (const float*)acc_short3,
+        (unsigned char*)bins_u8, (long long)n, k, L, (const float*)factors, crit, thr, (unsigned*)hist_u32, drift, box);
+    B200_CUDA(cudaGetLastError());
+    ctx->launches += 1;
     return B200_OK;
 }
 

@@ -33,6 +33,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "blockstep.cuh"
 #include "scan.cuh"
 #include "shard.cuh"
 #include "sort.cuh"
@@ -85,6 +86,7 @@ struct TreeState {
     DevBuf tile_hist, tile_warp_prefix, node_tile_sum;
     DevBuf split_node, split_where, split_local, split_cstart;
     DevBuf keys, keys_sorted, perm, sort_scratch, order;
+    DevBuf active_list, active_tiles;   // block time steps: the active targets of a sync point, in target order
     size_t order_i0 = 0, order_n = 0;
     bool order_valid = false;
     int order_age = 0;            // builds since the target order was computed
@@ -152,7 +154,7 @@ struct TreeState {
                          &ent_idx[1], &ent_node[0], &ent_node[1], &digit, &part_idx, &nodes, &leaf_pos, &lscan, &pscan, &sub, &leaf_tile_sum, &slot_node, &slot_digit,
                          &globals, &tile_hist, &tile_warp_prefix, &node_tile_sum, &split_node,
                          &split_where, &split_local, &split_cstart, &keys, &keys_sorted, &perm,
-                         &sort_scratch, &order};
+                         &sort_scratch, &order, &active_list, &active_tiles};
         for (DevBuf* b : all) b->release();
     }
 };
@@ -1544,6 +1546,59 @@ __global__ void zero_counters_kernel(TreeGlobals* g) {
     for (int c = 0; c < 6; ++c) g->counters[c] = 0;
 }
 
+// Compaction of the target order to the particles active at sync point k of the block time steps (DESIGN 3.14):
+// tiles of ACT_TILE entries, 8 consecutive per thread; count, single-CTA scan of the tile counts (the total lands in
+// tile_sum[n_tiles]), then the stable write of the active entries, whose acc_short rows are zeroed on the way.
+constexpr int ACT_TILE = 2048;
+
+__global__ void __launch_bounds__(256)
+active_count_kernel(const int* __restrict__ order, const unsigned char* __restrict__ bins, int n, int k, int L,
+                    unsigned* __restrict__ tile_sum) {
+    __shared__ unsigned sh[8];
+    const int n_tiles = (n + ACT_TILE - 1) / ACT_TILE;
+    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        unsigned c = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int t = tile * ACT_TILE + threadIdx.x * 8 + j;
+            if (t < n) c += block_active(block_bin(bins[order[t]], L), k, L) ? 1u : 0u;
+        }
+        const unsigned s = block_sum<8>(c, sh);
+        if (threadIdx.x == 0) tile_sum[tile] = s;
+    }
+}
+
+__global__ void __launch_bounds__(1024)
+active_scan_kernel(unsigned* __restrict__ tile_sum, int n_tiles) {
+    const unsigned tot = cta_exclusive_scan<1>(tile_sum, n_tiles, 1);
+    if (threadIdx.x == 0) tile_sum[n_tiles] = tot;
+}
+
+__global__ void __launch_bounds__(256)
+active_apply_kernel(const int* __restrict__ order, const unsigned char* __restrict__ bins, int n, int k, int L,
+                    const unsigned* __restrict__ tile_sum, int* __restrict__ list, float* __restrict__ acc3) {
+    __shared__ unsigned sh[8];
+    const int n_tiles = (n + ACT_TILE - 1) / ACT_TILE;
+    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        int idx[8];
+        unsigned c = 0, on = 0;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int t = tile * ACT_TILE + threadIdx.x * 8 + j;
+            idx[j] = t < n ? order[t] : 0;
+            if (t < n && block_active(block_bin(bins[idx[j]], L), k, L)) { on |= 1u << j; ++c; }
+        }
+        unsigned pos = block_exclusive_prefix(tile_sum[tile], c, sh);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            if (!(on >> j & 1u)) continue;
+            list[pos++] = idx[j];
+            float* r = acc3 + 3 * (size_t)idx[j];
+            r[0] = r[1] = r[2] = 0.f;
+        }
+    }
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------- host side ---
@@ -1978,6 +2033,9 @@ int tree_walk_list(b200_ctx* ctx, const int* list, size_t n_list, float theta, v
 
 // The short-range TreePM walk (walk_warp_kernel, SHORT) of the targets [i0, i0 + n_targets) of the fixed-physics
 // tree, in the periodic box `box` whatever tree_set_periodic holds: added to acc3.
+static int launch_short_walk(b200_ctx* ctx, TreeState* T, const int* order, size_t i0, size_t n_targets, float theta,
+                             float box, float r_split, float r_cut, void* acc3, cudaStream_t st);
+
 int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split, float r_cut,
                     void* acc3, cudaStream_t st) {
     TreeState* T = ctx->tree;
@@ -1987,6 +2045,13 @@ int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, flo
     if (n_targets == 0) return B200_OK;
     if (!acc3 || i0 + n_targets > T->n) return B200_ERR_INVALID;
     B200_TRY(tree_target_order(ctx, T, i0, n_targets, st));
+    return launch_short_walk(ctx, T, T->order.as<int>(), i0, n_targets, theta, box, r_split, r_cut, acc3, st);
+}
+
+// walk_warp_kernel<SHORT> of the targets order[0 .. n_targets) (particle indices), added to acc3[index - i0]; a
+// plain function rather than a template, so that the instances stay where they were in the module
+static int launch_short_walk(b200_ctx* ctx, TreeState* T, const int* order, size_t i0, size_t n_targets, float theta,
+                             float box, float r_split, float r_cut, void* acc3, cudaStream_t st) {
     if (T->counting) {
         zero_counters_kernel<<<1, 1, 0, st>>>(T->globals.as<TreeGlobals>());
         ctx->launches += 1;
@@ -1995,13 +2060,52 @@ int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, flo
     const unsigned grid = (unsigned)((n_targets + 127) / 128);
     const float theta2 = theta > 0.f ? theta * theta : 0.f;
     auto kernel = T->counting ? walk_warp_kernel<true, true, false, true> : walk_warp_kernel<false, true, false, true>;
-    kernel<<<grid, 128, 0, st>>>(T->posm, T->order.as<int>(), (int)i0, (int)n_targets, T->nodes.as<float4>(),
+    kernel<<<grid, 128, 0, st>>>(T->posm, order, (int)i0, (int)n_targets, T->nodes.as<float4>(),
                                  T->leaf_pos.as<ulonglong2>(), theta, theta2, T->eps * T->eps, box, (float*)acc3,
                                  T->globals.as<TreeGlobals>(), 0, 0.5f / r_split, r_cut, r_cut * r_cut);
     if (ctx->timing) B200_CUDA(cudaEventRecord(ctx->ev1, st));
     B200_CUDA(cudaGetLastError());
     ctx->launches += 1;
     return B200_OK;
+}
+
+// The short-range walk of the particles of [0, n) active at sync point k of the block time steps: the Hilbert order
+// of [0, n) compacted to them (its warps stay spatially coherent), their acc_short rows zeroed, then the walk adds
+// into them.  The count comes back to the host for the launch size.
+int tree_walk_short_active(b200_ctx* ctx, const void* bins_u8, size_t n, int k, int max_bins, float theta, float box,
+                           float r_split, float r_cut, void* acc_short3, size_t* n_active, cudaStream_t st) {
+    if (!n_active) return B200_ERR_INVALID;
+    *n_active = 0;
+    TreeState* T = ctx->tree;
+    if (!T || !T->built || !T->fixed || T->n != n) return B200_ERR_STATE;
+    if (!(box > 0.f) || !(r_split > 0.f) || !(r_cut > 0.f) || !(r_cut < 0.5f * box)) return B200_ERR_INVALID;
+    if (max_bins < 1 || max_bins > BLOCK_MAX_BINS) return B200_ERR_INVALID;
+    const int L = max_bins - 1;
+    if (k < 0 || k > (1 << L) || !bins_u8 || !acc_short3) return B200_ERR_INVALID;
+    B200_TRY(tree_target_order(ctx, T, 0, n, st));
+    if (k == 0 || k == (1 << L)) {                      // every step ends: the whole Hilbert order, no count to read
+        B200_CUDA(cudaMemsetAsync(acc_short3, 0, n * 3 * sizeof(float), st));
+        *n_active = n;
+        return launch_short_walk(ctx, T, T->order.as<int>(), 0, n, theta, box, r_split, r_cut, acc_short3, st);
+    }
+    const int n_tiles = (int)((n + ACT_TILE - 1) / ACT_TILE);
+    B200_TRY(T->active_list.reserve(n * sizeof(int)));
+    B200_TRY(T->active_tiles.reserve((n_tiles + 1) * sizeof(unsigned)));
+    const unsigned grid = (unsigned)(n_tiles < ctx->sm_count * 4 ? n_tiles : ctx->sm_count * 4);
+    const unsigned char* bins = (const unsigned char*)bins_u8;
+    unsigned* tiles = T->active_tiles.as<unsigned>();
+    active_count_kernel<<<grid, 256, 0, st>>>(T->order.as<int>(), bins, (int)n, k, L, tiles);
+    active_scan_kernel<<<1, 1024, 0, st>>>(tiles, n_tiles);
+    active_apply_kernel<<<grid, 256, 0, st>>>(T->order.as<int>(), bins, (int)n, k, L, tiles,
+                                              T->active_list.as<int>(), (float*)acc_short3);
+    ctx->launches += 3;
+    unsigned count = 0;
+    B200_CUDA(cudaMemcpyAsync(&count, tiles + n_tiles, sizeof count, cudaMemcpyDeviceToHost, st));
+    B200_CUDA(cudaStreamSynchronize(st));
+    B200_CUDA(cudaGetLastError());
+    *n_active = count;
+    if (count == 0) return B200_OK;
+    return launch_short_walk(ctx, T, T->active_list.as<int>(), 0, count, theta, box, r_split, r_cut, acc_short3, st);
 }
 
 // The short-range TreePM potential (walk_warp_kernel, SHORT and POT) of the same targets, added to phi: the checks

@@ -16,6 +16,9 @@ int tree_walk_list(b200_ctx* ctx, const int* list, size_t n_list, float theta, v
 // short-range TreePM walk of the fixed-physics tree in a periodic box, added to acc3
 int tree_walk_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split, float r_cut,
                     void* acc3, cudaStream_t st);
+// the short-range walk of the particles of [0, n) active at sync point k of the block time steps, into zeroed rows
+int tree_walk_short_active(b200_ctx* ctx, const void* bins_u8, size_t n, int k, int max_bins, float theta, float box,
+                           float r_split, float r_cut, void* acc_short3, size_t* n_active, cudaStream_t st);
 // short-range TreePM potential (erfc(r / 2 r_s) / r, minus the PM self term), added to phi; theta <= 1/sqrt(3)
 int tree_potential_short(b200_ctx* ctx, size_t i0, size_t n_targets, float theta, float box, float r_split,
                          float r_cut, void* phi, cudaStream_t st);

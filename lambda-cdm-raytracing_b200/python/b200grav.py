@@ -32,6 +32,7 @@ EXPORTS = [
     "b200_fp32_peak_probe", "b200_last_kernel_ms", "b200_set_timing", "b200_launch_count",
     "b200_pm_forces_dev", "b200_pm_forces_host", "b200_pm_phase_ms",
     "b200_comoving_kdk_factors", "b200_tree_potential_short_dev", "b200_treepm_energy_dev",
+    "b200_block_kick_dev", "b200_tree_walk_short_active_dev",
 ]
 
 
@@ -134,6 +135,8 @@ def load_library(path=None):
     L.b200_tree_potential_short_dev.argtypes = [vp, sz, sz, f32, f32, f32, f32, vp, vp]
     L.b200_treepm_energy_dev.argtypes = [vp, vp, sz, sz, sz, vp, i32, f32, f32, f32, f32, C.POINTER(f64),
                                          C.POINTER(f64), vp]
+    L.b200_block_kick_dev.argtypes = [vp] * 7 + [sz, i32, i32, vp, f32, f64, vp, f32, f32, vp]
+    L.b200_tree_walk_short_active_dev.argtypes = [vp, vp, sz, i32, i32, f32, f32, f32, f32, vp, C.POINTER(sz), vp]
     L.b200_fp32_peak_probe.argtypes = [vp, i32, i32, C.POINTER(f64), C.POINTER(f32)]
     L.b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
     L.b200_set_timing.argtypes = [vp, i32]
@@ -293,6 +296,15 @@ class Engine:
         self.pm_forces_dev(posm, acc, i0, n_targets, grid, box, rs, stream=stream)
         return self.tree_walk_short_dev(acc, i0, n_targets, theta, box, rs, r_cut_factor * rs, stream)
 
+    def tree_walk_short_active_dev(self, bins, n, k, max_bins, theta, box, r_split, r_cut, acc_short, stream=None):
+        """Sets the acc_short rows (device float[n, 3]) of the particles active at sync point k of the block time
+        steps (bins: device uint8[n]) to their short-range acceleration from the last fixed-physics tree of n sources;
+        returns the number of active particles (synchronises)."""
+        na = C.c_size_t()
+        self._check(self.L.b200_tree_walk_short_active_dev(self._h, _ptr(bins), n, k, max_bins, theta, box, r_split,
+                                                           r_cut, _ptr(acc_short), C.byref(na), _stream(stream)))
+        return na.value
+
     def tree_potential_short_dev(self, phi, i0, n_targets, theta, box, r_split, r_cut, stream=None):
         """Adds the TreePM short-range potential minus the PM self term (b200_tree_potential_short_dev) of targets
         [i0, i0+n_targets) of the last fixed-physics tree to phi (device float[n_targets])."""
@@ -405,6 +417,15 @@ class Engine:
         m = None if mass is None else np.ascontiguousarray(mass, np.float32)
         self._check(self.L.b200_leapfrog_host(self._h, _ptr(pos), _ptr(vel), _ptr(np.ascontiguousarray(acc, np.float32)),
                                               _ptr(m), n, n_kicks, dt_kick, a, dt_drift, box))
+
+    def block_kick_dev(self, posm, mom, acc, acc_long, acc_short, bins, n, k, max_bins, factors, crit, dlna, hist,
+                       drift=0.0, box=0.0, stream=None):
+        """Sync point k of the block time steps (b200_block_kick_dev): kicks and rebins the particles whose step ends
+        or starts at k, then drifts every particle by drift (0: none); hist (device uint32 / int32[16]) receives
+        the bin counts."""
+        self._check(self.L.b200_block_kick_dev(self._h, _ptr(posm), _ptr(mom), _ptr(acc), _ptr(acc_long),
+                                               _ptr(acc_short), _ptr(bins), n, k, max_bins, _ptr(factors), crit, dlna,
+                                               _ptr(hist), drift, box, _stream(stream)))
 
     def hubble_a(self, a, om=0.31, ok=0.0, ol=0.69, h=0.67):
         return float(self.L.b200_hubble_a(a, om, ok, ol, h))
@@ -645,6 +666,37 @@ def comoving_kdk_factors(lib, a0, a1, om=0.31, ok=0.0, ol=0.69):
     return d.value, k.value
 
 
+def block_factor_table(lib, a0, a1, max_bins, cosmo=(0.31, 0.0, 0.69)):
+    """Factors of one PM step from a0 to a1 with block time steps (DESIGN 3.14), doubles from
+    b200_comoving_kdk_factors; no context, no GPU.  Returns (kicks, nodes): nodes[k] = a0 exp(k Delta / S),
+    k = 0..S, Delta = ln(a1 / a0), S = 2^(max_bins - 1), the ends exactly a0 and a1; kicks[(2^b - 1) + j] =
+    K(a_s, m) (opening) and kicks[(2^max_bins - 1) + (2^b - 1) + j] = K(m, a_e) (closing) for step j of bin b, from
+    a_s = nodes[j w_b] to a_e = nodes[(j + 1) w_b], w_b = 2^(max_bins - 1 - b), m = sqrt(a_s a_e).
+    float32(kicks) is the factor table of b200_block_kick_dev."""
+    if not 1 <= max_bins <= 16:
+        raise ValueError(f"max_bins must be in 1..16, not {max_bins}")
+    L = max_bins - 1
+    S = 1 << L
+    d = np.log(a1 / a0)
+    nodes = np.array([a0] + [a0 * np.exp(k * d / S) for k in range(1, S)] + [a1], np.float64)
+    nb = (1 << max_bins) - 1
+    kicks = np.empty(2 * nb, np.float64)
+    for b in range(max_bins):
+        w = S >> b
+        for j in range(1 << b):
+            s, e = nodes[j * w], nodes[(j + 1) * w]
+            m = np.sqrt(s * e)
+            kicks[(1 << b) - 1 + j] = comoving_kdk_factors(lib, s, m, *cosmo)[1]
+            kicks[nb + (1 << b) - 1 + j] = comoving_kdk_factors(lib, m, e, *cosmo)[1]
+    return kicks, nodes
+
+
+def next_sync_point(k, counts, max_bins):
+    """The first sync point after k at which the step of some occupied bin (counts[b] > 0) ends."""
+    L = max_bins - 1
+    return min((((k >> (L - b)) + 1) << (L - b)) for b in range(max_bins) if counts[b] > 0)
+
+
 def comoving_zeldovich_dev(engine, **params):
     """Zel'dovich particles (Engine.zeldovich_ics_dev, params as there) in the units of ComovingSimulation:
     returns (pos, mom, mass, a0) as device tensors and a float -- positions in [0, box), masses 3 Om box^3 / (8 pi N)
@@ -666,7 +718,7 @@ def comoving_zeldovich_dev(engine, **params):
 
 
 class ComovingSimulation:
-    """Comoving KDK integration of a periodic LambdaCDM box with the PM or TreePM force (DESIGN 3.13).
+    """Comoving KDK integration of a periodic LambdaCDM box with the PM or TreePM force (DESIGN 3.13, 3.14).
 
     Units: comoving lengths in the box's unit, time in 1 / H0 (H0 = 1), G = 1; masses 3 Om L^3 / (8 pi N) give the
     mean density Om rho_crit, and the engine's periodic acceleration g is then the comoving peculiar acceleration.
@@ -674,13 +726,28 @@ class ComovingSimulation:
     motion dx/da = p / (a^3 E), dp/da = g / (a^2 E), E^2 = Om a^-3 + Ok a^-2 + OL.  step(a1) from a0: half-kick
     K(a0, am), drift D(a0, a1), forces at a1, half-kick K(am, a1), am = sqrt(a0 a1), with the exact factors of
     b200_comoving_kdk_factors.  force: "treepm" (PM on a pm_grid^3 mesh plus the short-range walk at theta,
-    softening eps, cut off at 4.5 r_split) or "pm"; r_split=None: 1.25 box / pm_grid."""
+    softening eps, cut off at 4.5 r_split) or "pm"; r_split=None: 1.25 box / pm_grid.
+
+    max_bins > 1 (force="treepm" only): block time steps.  step(a1) is one PM step: the long-range force is kicked
+    as above, the short-range force on power-of-two subdivisions of the step (bin b: 2^(max_bins - 1 - b) of the
+    2^(max_bins - 1) sub-steps, uniform in ln a), each particle's bin chosen by the criterion
+    dln a <= sqrt(2 eta eps a^3 E^2 / |g|) and only the particles whose step ends walked at a sync point.  With
+    max_bins = 1, or with every particle in bin 0, a step is the global KDK above, bit for bit.  After step()
+    every particle is synchronised.  acc holds the total acceleration, acc_long and acc_short its two parts, bins
+    the bins (device uint8); bin_counts is the bin histogram after the last sync point and short_targets the number
+    of short-range target evaluations so far."""
 
     def __init__(self, engine, pos, mom, mass, box, a0, force="treepm", pm_grid=128, r_split=None, theta=0.5,
-                 eps=0.01, leaf_cap=8, max_depth=20, cosmo=(0.31, 0.0, 0.69)):
+                 eps=0.01, leaf_cap=8, max_depth=20, cosmo=(0.31, 0.0, 0.69), max_bins=1, eta=0.025):
         import torch
         if force not in ("treepm", "pm"):
             raise ValueError(f"force must be 'treepm' or 'pm', not {force!r}")
+        if not (isinstance(max_bins, (int, np.integer)) and 1 <= max_bins <= 16):
+            raise ValueError(f"max_bins must be an integer in 1..16, not {max_bins!r}")
+        if force == "pm" and max_bins > 1:
+            raise ValueError("block time steps (max_bins > 1) subdivide the short range: they need force='treepm'")
+        if not eta > 0:
+            raise ValueError(f"eta must be > 0, not {eta!r}")
         self.e = engine
         dev = torch.device("cuda", engine.device)
         f32 = lambda x: torch.as_tensor(x, dtype=torch.float32, device=dev)
@@ -688,10 +755,16 @@ class ComovingSimulation:
         self.mom = f32(mom).reshape(-1, 3).clone()
         self.n = self.posm.shape[0]
         self.acc = torch.zeros((self.n, 3), dtype=torch.float32, device=dev)
+        self.acc_long = torch.zeros_like(self.acc)
+        self.acc_short = torch.zeros_like(self.acc)
+        self.bins = torch.zeros(self.n, dtype=torch.uint8, device=dev)
+        self._hist = torch.zeros(16, dtype=torch.int32, device=dev)      # uint32 counts, < 2^31 particles
+        self.short_targets = 0
         self.box, self.force, self.theta, self.eps = float(box), force, float(theta), float(eps)
         self.pm_grid, self.leaf_cap, self.max_depth = int(pm_grid), leaf_cap, max_depth
         self.r_split = 1.25 * self.box / self.pm_grid if r_split is None else float(r_split)
         self.cosmo = tuple(float(c) for c in cosmo)
+        self.max_bins, self.eta = int(max_bins), float(eta)
         self.a = float(a0)
         self.steps = 0
         self.have_forces = False
@@ -700,28 +773,69 @@ class ComovingSimulation:
     def scale_factor(self):
         return self.a
 
+    @property
+    def bin_counts(self):
+        """Particles per bin after the last sync point (int64[16], host; synchronises)."""
+        return self._hist.cpu().numpy().view(np.uint32).astype(np.int64)
+
     def compute_forces(self):
-        if self.force == "pm":
-            self.e.pm_forces_dev(self.posm, self.acc, 0, self.n, self.pm_grid, self.box, self.r_split)
-        else:
-            self.e.treepm_forces_dev(self.posm, self.acc, 0, self.n, self.pm_grid, self.box, self.r_split,
-                                     theta=self.theta, leaf_cap=self.leaf_cap, max_depth=self.max_depth, eps=self.eps)
+        """acc_long, acc_short and their sum acc at the current positions, for every particle."""
+        self.e.pm_forces_dev(self.posm, self.acc_long, 0, self.n, self.pm_grid, self.box, self.r_split)
+        self.acc_short.zero_()
+        if self.force == "treepm":
+            self.e.tree_build_fixed_dev(self.posm, self.n, self.leaf_cap, self.max_depth, self.eps)
+            self.e.tree_walk_short_dev(self.acc_short, 0, self.n, self.theta, self.box, self.r_split,
+                                       4.5 * self.r_split)
+            self.short_targets += self.n
+        self.acc.copy_(self.acc_long).add_(self.acc_short)              # fl(acc_long + acc_short), as the pass at k = S
         self.have_forces = True
 
+    def _sync_forces(self, k, S):
+        """Forces at sync point k > 0: the tree of the current positions, PM at k = S, the active short walk."""
+        if self.force == "pm":
+            self.e.pm_forces_dev(self.posm, self.acc_long, 0, self.n, self.pm_grid, self.box, self.r_split)
+            return
+        self.e.tree_build_fixed_dev(self.posm, self.n, self.leaf_cap, self.max_depth, self.eps)
+        if k == S:
+            self.e.pm_forces_dev(self.posm, self.acc_long, 0, self.n, self.pm_grid, self.box, self.r_split)
+        self.short_targets += self.e.tree_walk_short_active_dev(self.bins, self.n, k, self.max_bins, self.theta,
+                                                                self.box, self.r_split, 4.5 * self.r_split,
+                                                                self.acc_short)
+
+    def _pass(self, k, a_k, factors, dlna, drift=0.0):
+        om, ok, ol = self.cosmo
+        crit = np.float32(2.0 * self.eta * self.eps * a_k ** 3 * (om / a_k ** 3 + ok / a_k ** 2 + ol))
+        self.e.block_kick_dev(self.posm, self.mom, self.acc, self.acc_long, self.acc_short, self.bins, self.n, k,
+                              self.max_bins, factors, crit, dlna, self._hist, np.float32(drift), self.box)
+
     def step(self, a_next):
+        import torch
         a0, a1 = self.a, float(a_next)
-        am = np.sqrt(a0 * a1)
-        drift, _ = self.e.comoving_kdk_factors(a0, a1, *self.cosmo)
-        _, k0 = self.e.comoving_kdk_factors(a0, am, *self.cosmo)
-        _, k1 = self.e.comoving_kdk_factors(am, a1, *self.cosmo)
+        L = self.max_bins - 1
+        S = 1 << L
+        kicks, nodes = block_factor_table(self.e.L, a0, a1, self.max_bins, self.cosmo)
+        # through pinned memory, so that the copy does not wait for the previous step's work to finish
+        factors = torch.from_numpy(kicks.astype(np.float32)).pin_memory().to(self.acc.device, non_blocking=True)
+        dlna = float(np.log(a1 / a0))
         if not self.have_forces:
             self.compute_forces()
-        # b200_leapfrog_dev at a = 1 (1/a^2 = 1 exactly) with dt_kick = K and dt_drift = D is the comoving kick and
-        # drift: p += g K, x += p D, x wrapped into [0, box)
-        self.e.leapfrog_dev(self.posm, self.mom, self.acc, self.n, 1, np.float32(k0), 1.0, np.float32(drift),
-                            self.box)
-        self.compute_forces()
-        self.e.leapfrog_dev(self.posm, self.mom, self.acc, self.n, 1, np.float32(k1), 1.0, 0.0, self.box)
+        k = 0
+        if S == 1:                      # the next sync point is the end: the pass drifts too, D(a0, a1)
+            self._pass(0, a0, factors, dlna, self.e.comoving_kdk_factors(a0, a1, *self.cosmo)[0])
+        else:
+            self._pass(0, a0, factors, dlna)
+        while k < S:
+            if S > 1:
+                # the drift to the next sync point at which a step ends, D(a_k, a_k1), once the pass has set the bins:
+                # b200_leapfrog_dev at a = 1 with no kick, x += p D wrapped into [0, box); idle sub-steps are skipped
+                k1 = next_sync_point(k, self.bin_counts, self.max_bins)
+                drift, _ = self.e.comoving_kdk_factors(nodes[k], nodes[k1], *self.cosmo)
+                self.e.leapfrog_dev(self.posm, self.mom, self.acc, self.n, 0, 0.0, 1.0, np.float32(drift), self.box)
+            else:
+                k1 = S
+            k = k1
+            self._sync_forces(k, S)
+            self._pass(k, nodes[k], factors, dlna)
         self.a = a1
         self.steps += 1
 
